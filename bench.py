@@ -3,12 +3,15 @@
 
     python bench.py [--gpus N --steps K --warmup W]            # this repo's engine on N B200s (torchrun for N > 1)
     python bench.py --impl reference [--steps K --warmup W]    # the reference algorithm on the host CPU (oracle port)
+    python bench.py --dump-outputs DIR ...                     # also write the last timed step's results to DIR/*.npy
 
 One "step" = one attack_text_leaf call on one batch of synthetic captions: 2*k*B*rho candidates expanded, tokenized,
 encoded by the text tower and scored (SURVEY.md 8d). Prints ONE JSON line on rank 0.
   value : device-resident throughput (captions and draws already in HBM, CUDA events around the kernels)
   e2e   : the same through leaf_b200.attack_text_leaf with host strings (H2D of captions/draws and D2H of the
           winners inside the timed region)
+The inputs (tower weights, captions, draws, anchors) are seeded and computed without this repo's kernels, so two builds
+run with the same arguments can be compared output for output with --dump-outputs.
 """
 import argparse
 import json
@@ -49,7 +52,31 @@ def parse():
     ap.add_argument("--no-library-baseline", action="store_true", help="skip the stock-PyTorch-on-the-same-GPU leg (N = 1 only)")
     ap.add_argument("--no-dense77", action="store_true", help="skip the worst-case (every row truncated to 77 tokens) leg")
     ap.add_argument("--no-global-batch", action="store_true", help="skip the strong-scaling legs with a collective on the path (N > 1 only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed on rank 0 "
+                    "(winning position and character index per caption, winner features) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT_BYTES, seed=0):
+    """Writes `arrays` (name -> array, one row per caption) as path/<name>.npy, floats as float32 / float64 and integers as
+    float64 (exact). When they hold more than `limit` bytes, the same seeded sample of rows is written for every array, with
+    the sampled row indices as path/rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v.nbytes for v in arrays.values()) // max(n, 1) + 8
+    if n * row_bytes > limit:
+        rows = np.sort(np.random.RandomState(seed).choice(n, size=limit // row_bytes, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def peaks():
@@ -251,6 +278,7 @@ def run_ours(a):
     from leaf_b200 import attack_text_leaf
     from leaf_b200.attack import V_DEFAULT
     from leaf_b200.tower import LeafTextTower
+    from oracle import leaf_oracle as O
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -266,13 +294,22 @@ def run_ours(a):
     eng = tower.leaf_engine
     caps = synth.make_captions(B, seed=100 + rank, kind=a.captions)
     frozen_sd = synth.perturbed_copy(tower.open_clip_state_dict(), seed=1, std=1e-3)
-    frozen = LeafTextTower(frozen_sd, heads=cfg.heads, quick_gelu=cfg.quick_gelu, device=dev)
-    anchor = frozen.encode_text(frozen.tokenizer(caps)).clone()
+    otok = O.OracleTokenizer()
+
+    def frozen_anchor(cs):
+        """E_frozen(x) by the fp32 oracle tower on this GPU, not by this repo's kernels: the anchors are the same whichever
+        build is measured."""
+        tok = otok(cs).to(dev)
+        with torch.no_grad():
+            return torch.cat([O.encode_text_device(frozen_sd, tok[s:s + 256], cfg.heads, quick_gelu=cfg.quick_gelu)
+                              for s in range(0, len(cs), 256)])
+
+    anchor = frozen_anchor(caps)
     dense_caps = synth.make_captions(B, seed=100 + rank, kind="dense-77")
-    dense_anchor = frozen.encode_text(frozen.tokenizer(dense_caps)).clone()
+    dense_anchor = frozen_anchor(dense_caps)
     gcaps = synth.make_captions(B, seed=100, kind=a.captions)               # ONE global batch, identical on every rank
-    ganchor = frozen.encode_text(frozen.tokenizer(gcaps)).clone()
-    del frozen, frozen_sd
+    ganchor = frozen_anchor(gcaps)
+    del frozen_sd
     torch.cuda.empty_cache()
     eng.reserve(B * n + B)
     Vt = np.asarray(V_DEFAULT, dtype=np.int32)
@@ -289,7 +326,8 @@ def run_ours(a):
     space = torch.full((B * n,), 32, dtype=torch.int32, device=dev)
 
     def device_step(pos_d, chr_d, record=None, cset=None):
-        """The hot path with inputs resident in HBM (k = 1 form: no host round trip between the phases)."""
+        """The hot path with inputs resident in HBM (k = 1 form: no host round trip between the phases). Returns the
+        winning position index [B], the winning character index [B] and the winner's features [B, E]."""
         caps_d, off_d, anc = typical_set if cset is None else cset
         tok, ln, base = eng.expand_tokenize(caps_d, off_d, B, n, pos=pos_d, chr_=space)
         f = eng.encode_tokens(tok, ln, False, base, (B * n, n), trim=True)
@@ -300,7 +338,8 @@ def run_ours(a):
         f = eng.encode_tokens(tok, ln, False, base, (B * n, n), trim=True)
         if record is not None:
             record.append((ln[:B * n], eng.last_rows()))
-        return eng.score(f, anc, B, n, "l2")
+        best2, best_feat, _ = eng.score(f, anc, B, n, "l2")
+        return best1, best2, best_feat
 
     def barrier():
         if world > 1:
@@ -321,10 +360,12 @@ def run_ours(a):
             flush.fill_(i)                                  # L2 flush between timed iterations (outside the events)
             ev[i][0].record()
             for _ in range(k):
-                device_step(*all_draws[a.warmup + i])
+                last = device_step(*all_draws[a.warmup + i])
             ev[i][1].record()
         torch.cuda.synchronize()
         launches = eng.launch_count()
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, dict(zip(("best_position", "best_character", "best_features"), (t.cpu().numpy() for t in last))))
         barrier()
         dev_ms = sum(s.elapsed_time(e) for s, e in ev)
         # ---- end to end through the public API (host strings in, winners out) ----

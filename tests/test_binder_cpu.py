@@ -47,14 +47,15 @@ def test_open_clip_module_detection():
 
 
 def test_real_open_clip_models_are_recognised():
-    """The reference's own model classes (open_clip.create_model through oracle/ref_shims), where /root/reference exists (this
-    container; the GPU box does not have it): CLIP with nn.GELU and with QuickGELU, heads, eps, layout, and the DDP-style holder."""
+    """The reference's own model classes (open_clip.create_model through oracle/ref_shims) from a LIONS-EPFL/LEAF checkout named
+    by LEAF_REFERENCE (not part of this repository, so skipped without it): CLIP with nn.GELU and with QuickGELU, heads, eps,
+    layout, and the DDP-style holder. tests/test_gpu_dropin.py's OpenClipNamedTower stands in for these classes elsewhere."""
     import os
     import subprocess
     import sys
-    ref = os.environ.get("LEAF_REFERENCE", "/root/reference")
-    if not os.path.isdir(os.path.join(ref, "src", "open_clip")):
-        pytest.skip("reference tree not present")
+    ref = os.environ.get("LEAF_REFERENCE", "")
+    if not ref or not os.path.isdir(os.path.join(ref, "src", "open_clip")):
+        pytest.skip("set LEAF_REFERENCE to a LIONS-EPFL/LEAF checkout to run this test")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     code = r'''
 import sys, torch
