@@ -181,7 +181,8 @@ int leaf_topk(leaf_handle_t h, const float* score_a, const float* score_b, int32
  * weight-gradient contractions on the host: pass rows_hint = sum(len) and max_len_hint >= max(len) when the host knows them
  * (checked on the device: a wrong hint traps) and nothing synchronises; with 0 / 0 the stream is synchronised once to learn them; leaf_backward consumes dfeat [N,E] fp32 and ACCUMULATES (+=) the parameter
  * gradients into the fp32 device buffers named by `grads` (same struct and layouts as leaf_bind_weights; a NULL
- * pointer marks a frozen parameter). bf16 operands, fp32 accumulation, fp32 LayerNorm/softmax/activation math.
+ * pointer marks a frozen parameter). bf16 operands, fp32 accumulation, fp32 LayerNorm/softmax/activation math. By default
+ * some gradients are atomic sums and not bit-reproducible run to run; leaf_set_deterministic(h, 1) makes all of them so.
  * ONE forward, ONE backward: the engine keeps a single activation store. Every leaf_forward_train gets a generation
  * number (> 0, written to *generation_out when that is not NULL); leaf_backward(generation != 0) fails with
  * LEAF_ERR_STATE when the store holds a different forward (a second encode_text ran before this output's backward -
@@ -206,6 +207,19 @@ int leaf_set_backward_hook(leaf_handle_t h, leaf_backward_hook_t fn, void* user)
 /* Cap the persistent GEMM grids at n_sms SMs (0 = the whole device) so that a collective's CTAs find SMs of their own while
  * it runs next to the backward. */
 int leaf_set_sm_budget(leaf_handle_t h, int32_t n_sms);
+/* Deterministic mode (off by default; PyTorch's torch.use_deterministic_algorithms(True) turns it on through
+ * leaf_b200.LeafEngine). The forward is deterministic in either mode. Off, leaf_backward sums several gradients with fp32
+ * atomics in arrival order and they are not bit-reproducible run to run: the split-K weight gradients (out-proj, QKV, HF q/k/v,
+ * the [E,W] projection, any weight gradient with fewer output tiles than CTA pairs), the fc1 / fc2 / out-proj / in-projection
+ * biases, the LayerNorm gains and biases, the token and positional embeddings; leaf_sumsq adds its block sums with atomics too.
+ * On, every one of these is a fixed-order reduction: each gradient leaf_backward writes and the value leaf_sumsq adds are
+ * functions of the inputs alone, bit for bit - whatever the run, leaf_set_sm_budget, LEAF_PDL or the order in which blocks
+ * finish. The two modes sum in different orders, so they agree to rounding, not to the bit. Turning it on allocates its
+ * workspace (a few tens of MB; synchronises the device) for the current leaf_train_reserve size, and leaf_train_reserve
+ * sizes it from then on. The deterministic reductions of one handle share that workspace and their arrival counters: in this
+ * mode its leaf_backward and leaf_sumsq calls must be stream-ordered (one stream, or ordered by events); two of them running
+ * at the same time on different streams would corrupt each other's sums. */
+int leaf_set_deterministic(leaf_handle_t h, int32_t on);
 
 /* AdamW (torch.optim.AdamW semantics, decoupled weight decay) over the tower's parameters held in ONE flat fp32 buffer
  * (train_AT_text_only.py:326-341: the gain / bias / LayerNorm group with weight_decay 0 is laid out first, elements

@@ -51,6 +51,7 @@ SIGNATURES = {
     "leaf_backward": (c_int, [c_void_p, c_i64, c_void_p, c_int, ctypes.POINTER(LeafWeightPtrs), c_void_p]),
     "leaf_set_backward_hook": (c_int, [c_void_p, c_void_p, c_void_p]),
     "leaf_set_sm_budget": (c_int, [c_void_p, c_int]),
+    "leaf_set_deterministic": (c_int, [c_void_p, c_int]),
     "leaf_adamw": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_i64, ctypes.c_float, ctypes.c_float,
                            ctypes.c_float, ctypes.c_float, ctypes.c_float, c_int, ctypes.c_float, c_void_p]),
     "leaf_sumsq": (c_int, [c_void_p, c_void_p, c_i64, c_void_p, c_void_p]),

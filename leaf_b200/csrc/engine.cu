@@ -9,6 +9,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <map>
 #include <string>
 #include <tuple>
@@ -70,6 +71,12 @@ struct TrainWs {
   float *x_out = nullptr, *dx = nullptr, *dtmp = nullptr, *scratch = nullptr;
   __nv_bfloat16 *pooled = nullptr, *d16 = nullptr, *dx16 = nullptr;
   float* ln_stats = nullptr;         // (mean, rstd) per row, from the LayerNorm backward's row kernel to its column kernel
+  // deterministic mode only (leaf_set_deterministic): partial sums of the fixed-order reductions, their arrival counters (zero
+  // between launches) and the embedding backward's row sort (row_tok | order | key, rows_cap each)
+  float* det_ws = nullptr;
+  int* det_cnt = nullptr;
+  int* det_idx = nullptr;
+  size_t det_ws_floats = 0, det_cnt_ints = 0;
   int *tok = nullptr, *cu = nullptr, *eos_row = nullptr, *total_rows = nullptr, *pfx = nullptr, *own_len = nullptr;
   int4* meta = nullptr;
   std::vector<void*> allocs;
@@ -116,6 +123,9 @@ struct leaf_engine {
   bool prune_last = true;             // final layer: out-proj + MLP on the pooled rows only
   int gemm_sm_budget = 0;             // > 0: the persistent GEMM grids use at most this many SMs (leaf_set_sm_budget)
   int pdl = 1;                        // launch the per-layer chain with programmatic dependent launch (LEAF_PDL=0 turns it off)
+  bool deterministic = false;         // leaf_set_deterministic: fixed-order reductions in leaf_backward / leaf_sumsq
+  float* det_sum_ws = nullptr;        // leaf_sumsq's per-block sums and arrival counter in deterministic mode
+  int* det_sum_cnt = nullptr;
   int att_impl = 1;                   // 1 = register-fed attention_kernel (default: faster in situ), 2 = cp.async ring attention2_kernel (LEAF_ATTENTION_IMPL=2)
   int *cu = nullptr, *eos_row = nullptr, *total_rows = nullptr, *pfx = nullptr, *own_len = nullptr, *dup_of = nullptr, *need = nullptr;
   int4* meta = nullptr;
@@ -220,27 +230,48 @@ static int launch_gemm(leaf_engine* e, const __nv_bfloat16* A, long a_rows, cons
   p.res = res;
   p.C2 = C2;
   p.split_k = 1;
+  p.ws = nullptr;
+  p.cnt = nullptr;
   p.tx_bytes = static_cast<uint32_t>(a_box + b_box) * GEMM_BK * 2 * 2;       // both CTAs of the pair
   p.M = M; p.m_dev = m_dev; p.N = N; p.K = K; p.bias = bias; p.C = C; p.ldc = ldc; p.act = act; p.delta = delta;
   const int m_tiles = (M + GEMM2_BM - 1) / GEMM2_BM, n_tiles = (N + GEMM_BN - 1) / GEMM_BN;
   long tiles = static_cast<long>(m_tiles) * n_tiles;
   const int pairs_cap = ((e->gemm_sm_budget > 0 && e->gemm_sm_budget < e->sm_count) ? e->gemm_sm_budget : e->sm_count) / 2;
-  if (allow_split_k && epi == EPI_F32_RESIDUAL && !bias && !delta && !res && !m_dev && tiles < pairs_cap) {
+  // Deterministic mode: fc1's bias gradient and the split-K partial sums are added in a fixed order (gemm_sm100.cuh,
+  // EPI_*_DET), and the split factor is chosen for the whole device, so that an SM budget cannot change the summation order.
+  const bool det = e->deterministic && ((epi == EPI_BF16_ACTBWD && C2) || allow_split_k);
+  const int split_pairs = det ? e->sm_count / 2 : pairs_cap;
+  if (det) {
+    if (!e->tw.det_ws) return fail(LEAF_ERR_STATE, "deterministic mode without its workspace (leaf_train_reserve)");
+    p.ws = e->tw.det_ws;
+    p.cnt = e->tw.det_cnt;
+    if (epi == EPI_BF16_ACTBWD) {
+      if (static_cast<size_t>((M + 31) / 32) * N > e->tw.det_ws_floats || static_cast<size_t>(n_tiles) * 4 > e->tw.det_cnt_ints)
+        return fail(LEAF_ERR_STATE, "deterministic workspace too small for a %dx%d bias reduction", M, N);
+      epi = EPI_BF16_ACTBWD_DET;
+    }
+  }
+  if (allow_split_k && epi == EPI_F32_RESIDUAL && !bias && !delta && !res && !m_dev && tiles < split_pairs) {
     // C += A.B with few output tiles and a long contraction (the weight gradients: 16-64 tiles, K = packed rows): divide the
     // k-blocks over several work units so that the launch fills the 74 CTA pairs; cost model = waves x (k-blocks per part +
     // 3 for the epilogue and the pipeline ramp). Partial sums are added with red.global.add.v4.f32.
     const int kblocks = (K + GEMM_BK - 1) / GEMM_BK;
-    long best = ((tiles + pairs_cap - 1) / pairs_cap) * (kblocks + 3);
+    long best = ((tiles + split_pairs - 1) / split_pairs) * (kblocks + 3);
     for (int s = 2; s <= 8 && s <= kblocks; ++s) {
       const int kpb = (kblocks + s - 1) / s;
       const int s_eff = (kblocks + kpb - 1) / kpb;              // every part non-empty
-      const long cost = ((tiles * s_eff + pairs_cap - 1) / pairs_cap) * (kpb + 3);
+      if (det && tiles * s_eff > 2L * split_pairs) continue;    // the partial tiles' workspace holds two waves of units
+      const long cost = ((tiles * s_eff + split_pairs - 1) / split_pairs) * (kpb + 3);
       if (cost < best) { best = cost; p.split_k = s_eff; }
     }
+    if (det && p.split_k > 1 && (static_cast<size_t>(tiles) * p.split_k * GEMM2_BM * GEMM_BN > e->tw.det_ws_floats ||
+                                 static_cast<size_t>(tiles) * 2 * EPI_WARPS > e->tw.det_cnt_ints))
+      return fail(LEAF_ERR_STATE, "deterministic workspace too small for a %dx%d split-K product", M, N);
     tiles *= p.split_k;
-    if (p.split_k > 1) epi = EPI_F32_SPLITK;
+    if (p.split_k > 1) epi = det ? EPI_F32_SPLITK_DET : EPI_F32_SPLITK;
   }
-  TimedSpan span(e, (epi == EPI_F32_SPLITK) ? 4 + EPI_F32_RESIDUAL : (epi == EPI_BF16_ACTBWD) ? 4 + EPI_F32 : (epi == EPI_F32_RESIDUAL && K > N) ? 8 : (epi == EPI_BF16 && K == N) ? 9 : 4 + epi, st);
+  TimedSpan span(e, (epi == EPI_F32_SPLITK || epi == EPI_F32_SPLITK_DET) ? 4 + EPI_F32_RESIDUAL :
+                    (epi == EPI_BF16_ACTBWD || epi == EPI_BF16_ACTBWD_DET) ? 4 + EPI_F32 : (epi == EPI_F32_RESIDUAL && K > N) ? 8 : (epi == EPI_BF16 && K == N) ? 9 : 4 + epi, st);
   const int pairs = static_cast<int>(tiles < pairs_cap ? tiles : pairs_cap);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(2 * pairs);
@@ -261,6 +292,8 @@ static int launch_gemm(leaf_engine* e, const __nv_bfloat16* A, long a_rows, cons
     case EPI_F32: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32>, ta, tb, p)); break;
     case EPI_F32_SPLITK: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32_SPLITK>, ta, tb, p)); break;
     case EPI_BF16_ACTBWD: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD>, ta, tb, p)); break;
+    case EPI_F32_SPLITK_DET: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32_SPLITK_DET>, ta, tb, p)); break;
+    case EPI_BF16_ACTBWD_DET: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD_DET>, ta, tb, p)); break;
     default: return fail(LEAF_ERR_INVALID, "unknown epilogue %d", epi);
   }
   e->launches++;
@@ -299,12 +332,16 @@ extern "C" int leaf_create(const leaf_cfg_t* cfg, leaf_handle_t* out) {
   CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32_SPLITK>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32_SPLITK_DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD_DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(embed_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LEAF_VOCAB * 4));
   CK(cudaFuncSetAttribute(topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   CK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   if (const char* ai = getenv("LEAF_ATTENTION_IMPL")) e->att_impl = atoi(ai) == 2 ? 2 : 1;
   if (const char* pd = getenv("LEAF_PDL")) e->pdl = atoi(pd) != 0;
-  CK(cudaFuncSetAttribute(attention_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
+  CK(cudaFuncSetAttribute(attention_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
+  CK(cudaFuncSetAttribute(attention_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
   *out = e;
   return LEAF_OK;
 }
@@ -340,6 +377,8 @@ extern "C" int leaf_destroy(leaf_handle_t e) {
   free_weights(e);
   for (void* p : e->table_allocs) cudaFree(p);
   cudaFree(e->cn_count);
+  cudaFree(e->det_sum_ws);
+  cudaFree(e->det_sum_cnt);
   for (auto& sp : e->spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
   for (auto ev : e->event_pool) cudaEventDestroy(ev);
   delete e;
@@ -709,7 +748,7 @@ extern "C" int leaf_test_attention(leaf_handle_t e, const void* qkv, const int32
 extern "C" int leaf_test_attention_bwd(leaf_handle_t e, const void* qkv, const void* o, const float* dout, const int32_t* meta,
                                        int32_t N, int32_t T, void* dqkv, void* stream) {
   if (!e || !qkv || !o || !dout || !meta || !dqkv || N <= 0 || T <= 0 || T > LEAF_CTX) return fail(LEAF_ERR_INVALID, "bad argument");
-  attention_bwd_kernel<<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(T), static_cast<cudaStream_t>(stream)>>>(
+  attention_bwd_kernel<false><<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(T), static_cast<cudaStream_t>(stream)>>>(
       static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(o), dout, reinterpret_cast<const int4*>(meta),
       e->cfg.width, T, static_cast<__nv_bfloat16*>(dqkv));
   e->launches++;
@@ -790,6 +829,32 @@ static void free_train(leaf_engine* e) {
   e->tmaps.clear();
 }
 
+// Workspace of the deterministic backward for the reserved training shape (a no-op when it exists or nothing is reserved).
+// Largest user of each buffer: the split-K partial tiles (two waves of work units at the device's pair count), fc1's bias
+// (one row of column sums per 32 packed rows), the LayerNorm bands (at most 2 x SMs / column blocks + 1), the attention
+// bias partials (one per sequence and warp).
+static int reserve_deterministic(leaf_engine* e) {
+  TrainWs& t = e->tw;
+  if (t.det_ws || t.max_seqs == 0) return LEAF_OK;
+  const size_t W = e->cfg.width, rows = static_cast<size_t>(t.rows_cap), pairs = static_cast<size_t>(e->sm_count / 2);
+  const size_t cbx = (W + 255) / 256;
+  size_t f = 2 * pairs * GEMM2_BM * GEMM_BN;
+  f = std::max(f, (rows + 31) / 32 * 4 * W);
+  f = std::max(f, (2 * static_cast<size_t>(e->sm_count) + cbx) * 3 * 256);
+  f = std::max(f, static_cast<size_t>(t.max_seqs) * ATTB_WARPS * 3 * W);
+  size_t c = std::max(pairs * 2 * EPI_WARPS, (4 * W + GEMM_BN - 1) / GEMM_BN * 4);
+  c = std::max(c, std::max(cbx, static_cast<size_t>(e->cfg.heads)));
+  int rc;
+  if ((rc = tw_alloc(t, &t.det_ws, f))) return rc;
+  if ((rc = tw_alloc(t, &t.det_cnt, c))) return rc;
+  if ((rc = tw_alloc(t, &t.det_idx, 3 * rows))) return rc;
+  CK(cudaMemset(t.det_cnt, 0, c * 4));
+  CK(cudaDeviceSynchronize());
+  t.det_ws_floats = f;
+  t.det_cnt_ints = c;
+  return LEAF_OK;
+}
+
 extern "C" int leaf_train_reserve(leaf_handle_t e, int32_t max_seqs) {
   if (!e || max_seqs <= 0) return fail(LEAF_ERR_INVALID, "max_seqs");
   if (!e->bound) return fail(LEAF_ERR_STATE, "weights not bound");
@@ -829,7 +894,7 @@ extern "C" int leaf_train_reserve(leaf_handle_t e, int32_t max_seqs) {
   if ((rc = tw_alloc(t, &t.meta, static_cast<size_t>(max_seqs)))) return rc;
   t.max_seqs = max_seqs;
   t.rows_cap = static_cast<long>(rows);
-  return LEAF_OK;
+  return e->deterministic ? reserve_deterministic(e) : LEAF_OK;
 }
 
 static int launch_ew(leaf_engine* e, size_t n) {      // grid for the grid-stride element-wise kernels
@@ -918,7 +983,15 @@ static int launch_layernorm_bwd(leaf_engine* e, const float* dy, const float* x,
   int bands = (2 * e->sm_count + cbx - 1) / cbx;
   if (bands > (rows + 7) / 8) bands = (rows + 7) / 8;
   if (bands < 1) bands = 1;
-  CK(launch_pdl(e, layernorm_bwd_cols_kernel, dim3(cbx, bands), dim3(256), st, dy, x, gather, stats, dx, rows, W, dgamma, dbeta, dxsum));
+  if (e->deterministic) {                              // band sums added in band order (train_kernels.cuh)
+    if (static_cast<size_t>(bands) * 3 * W > e->tw.det_ws_floats || static_cast<size_t>(cbx) > e->tw.det_cnt_ints)
+      return fail(LEAF_ERR_STATE, "deterministic workspace too small for the LayerNorm backward (%d bands)", bands);
+    CK(launch_pdl(e, layernorm_bwd_cols_kernel<true>, dim3(cbx, bands), dim3(256), st, dy, x, gather, stats, dx, rows, W, dgamma, dbeta,
+                  dxsum, e->tw.det_ws, e->tw.det_cnt));
+  } else {
+    CK(launch_pdl(e, layernorm_bwd_cols_kernel<false>, dim3(cbx, bands), dim3(256), st, dy, x, gather, stats, dx, rows, W, dgamma, dbeta,
+                  dxsum, nullptr, nullptr));
+  }
   e->launches += 2;
   CK(cudaGetLastError());
   return LEAF_OK;
@@ -935,6 +1008,7 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
                 "saved forward (run each encode_text's backward before the next encode_text with gradients enabled)",
                 (long long)t.generation, (long long)generation);
   if (dfeat_rows != t.N) return fail(LEAF_ERR_INVALID, "dfeat has %d rows, the saved forward has %d sequences", dfeat_rows, t.N);
+  if (e->deterministic && !t.det_ws) return fail(LEAF_ERR_STATE, "deterministic mode without its workspace (leaf_train_reserve)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int W = e->cfg.width, E = e->cfg.embed_dim, N = t.N, M = t.M;
   const long cap = t.rows_cap;
@@ -992,7 +1066,12 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
       float* bq = p.in_proj_w ? F(g.in_proj_b) : F(g.q_b);
       float* bk = p.in_proj_w ? (g.in_proj_b ? F(g.in_proj_b) + W : nullptr) : F(g.k_b);
       float* bv = p.in_proj_w ? (g.in_proj_b ? F(g.in_proj_b) + 2 * W : nullptr) : F(g.v_b);
-      attention_bwd_kernel<<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16, bq, bk, bv);
+      if (e->deterministic && (bq || bk || bv))         // bias column sums added in (sequence, warp) order
+        attention_bwd_kernel<true><<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16,
+                                                                                                      bq, bk, bv, t.det_ws, t.det_cnt);
+      else
+        attention_bwd_kernel<false><<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16,
+                                                                                                       bq, bk, bv);
     }
     e->launches++;
     CK(cudaGetLastError());
@@ -1013,8 +1092,18 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
     // a frozen table still needs a target for the atomics: reuse dtmp as a sink is not possible (49408 rows) -> require both
     if (!grads->token_embedding || !grads->positional_embedding)
       return fail(LEAF_ERR_INVALID, "token and positional embedding gradients must be given together");
-    embed_bwd_kernel<<<N, 256, 0, st>>>(t.tok, t.meta, N, W, t.dx, F(grads->token_embedding), F(grads->positional_embedding));
-    e->launches++;
+    if (e->deterministic) {                            // rows grouped by token id, one writer per table row (train_kernels.cuh)
+      int* row_tok = t.det_idx;
+      int* order = row_tok + t.rows_cap;
+      int* key = order + t.rows_cap;
+      embed_sort_kernel<<<1, 1024, LEAF_VOCAB * 4, st>>>(t.tok, t.meta, N, M, row_tok, order, key);
+      embed_bwd_det_kernel<<<dim3(M + LEAF_CTX, (W + 255) / 256), 256, 0, st>>>(order, key, t.meta, N, M, W, t.dx, F(grads->token_embedding),
+                                                                                F(grads->positional_embedding));
+      e->launches += 2;
+    } else {
+      embed_bwd_kernel<<<N, 256, 0, st>>>(t.tok, t.meta, N, W, t.dx, F(grads->token_embedding), F(grads->positional_embedding));
+      e->launches++;
+    }
   }
   CK(cudaGetLastError());
   t.have_forward = false;                              // consumed: dx / dtmp were overwritten, a second backward would be wrong
@@ -1028,6 +1117,24 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
 extern "C" int leaf_set_sm_budget(leaf_handle_t e, int32_t n_sms) {
   if (!e || n_sms < 0) return fail(LEAF_ERR_INVALID, "bad argument");
   e->gemm_sm_budget = n_sms >= 2 ? n_sms : 0;
+  return LEAF_OK;
+}
+
+extern "C" int leaf_set_deterministic(leaf_handle_t e, int32_t on) {
+  if (!e) return fail(LEAF_ERR_INVALID, "null handle");
+  if (on) {
+    if (!e->det_sum_ws) {
+      CK(cudaMalloc(&e->det_sum_ws, static_cast<size_t>(e->sm_count) * 16 * 4));
+      CK(cudaMalloc(&e->det_sum_cnt, 4));
+      CK(cudaMemset(e->det_sum_cnt, 0, 4));
+      CK(cudaDeviceSynchronize());
+    }
+    e->deterministic = true;
+    int rc = reserve_deterministic(e);
+    if (rc) { e->deterministic = false; return rc; }
+  } else {
+    e->deterministic = false;
+  }
   return LEAF_OK;
 }
 
@@ -1061,7 +1168,11 @@ extern "C" int leaf_adamw(leaf_handle_t e, float* params, const float* grads, fl
 // out[0] (device fp32, zeroed by the caller) += sum of squares of g[0, n)
 extern "C" int leaf_sumsq(leaf_handle_t e, const float* g, int64_t n, float* out, void* stream) {
   if (!e || !g || !out || n <= 0 || n % 4 != 0) return fail(LEAF_ERR_INVALID, "bad argument");
-  sumsq_kernel<<<launch_ew(e, static_cast<size_t>(n) / 4), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, static_cast<size_t>(n), out);
+  const int grid = launch_ew(e, static_cast<size_t>(n) / 4);       // <= 16 x SMs: leaf_set_deterministic sizes det_sum_ws for it
+  if (e->deterministic)
+    sumsq_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(g, static_cast<size_t>(n), out, e->det_sum_ws, e->det_sum_cnt);
+  else
+    sumsq_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(g, static_cast<size_t>(n), out);
   e->launches++;
   CK(cudaGetLastError());
   return LEAF_OK;

@@ -103,7 +103,7 @@ gemm2_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
   const int n_tiles = (p.N + GEMM_BN - 1) / GEMM_BN;
   const int k_blocks = (p.K + GEMM_BK - 1) / GEMM_BK;
   // split-K: the k-blocks of an output tile are divided over `split` consecutive work units (GemmParams::split_k)
-  const int split = (EPI == EPI_F32_SPLITK && p.split_k > 1) ? p.split_k : 1;
+  const int split = ((EPI == EPI_F32_SPLITK || EPI == EPI_F32_SPLITK_DET) && p.split_k > 1) ? p.split_k : 1;
   const int kpb = (k_blocks + split - 1) / split;
   const int total_tiles = m_tiles * n_tiles * split;
 
@@ -233,12 +233,80 @@ gemm2_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
                                static_cast<uint32_t>(acc * GEMM_BN + part * 64 + c);
         tmem_ld32(taddr, v);
         tmem_ld_wait();
-        if (row0 < M) epilogue_chunk<EPI>(p, v, res, stage_buf, lane, row0, col0, M);      // warp-uniform
+        if constexpr (EPI == EPI_F32_SPLITK_DET) {
+          // this work unit's partial sums, [column][lane] in the warp's region of the unit's tile (coalesced)
+          if (row0 < M) {
+            float* w = p.ws + static_cast<size_t>(tile) * (GEMM2_BM * GEMM_BN) + ((rank * EPI_WARPS + warp) * 2 + (c >> 5)) * 1024 + lane;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) w[j * 32] = __uint_as_float(v[j]);
+          }
+        } else {
+          if (row0 < M) epilogue_chunk<EPI>(p, v, res, stage_buf, lane, row0, col0, M);      // warp-uniform
+        }
       }
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_leader(tempty_bar(acc));
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+      if constexpr (EPI == EPI_F32_SPLITK_DET) {
+        // The last of the `split` units of this output tile to reach this warp's region adds the partials to C in split order.
+        int* ctr = p.cnt + mn * (2 * EPI_WARPS) + rank * EPI_WARPS + warp;
+        __threadfence();
+        __syncwarp();
+        int old = 0;
+        if (lane == 0) old = atomicAdd(ctr, 1);
+        old = __shfl_sync(0xffffffffu, old, 0);
+        if (old == split - 1) {
+          __threadfence();
+          if (row0 < M) {
+#pragma unroll 1
+            for (int c = 0; c < 64; c += 32) {
+              const int col0 = n_blk * GEMM_BN + part * 64 + c;
+              if (col0 >= p.N) break;
+              const float* w = p.ws + static_cast<size_t>(mn) * split * (GEMM2_BM * GEMM_BN) + ((rank * EPI_WARPS + warp) * 2 + (c >> 5)) * 1024 + lane;
+              float f[32];
+#pragma unroll
+              for (int j = 0; j < 32; ++j) f[j] = __ldcg(w + j * 32);
+#pragma unroll 1
+              for (int u = 1; u < split; ++u) {
+                w += GEMM2_BM * GEMM_BN;
+#pragma unroll
+                for (int j = 0; j < 32; ++j) f[j] += __ldcg(w + j * 32);
+              }
+              uint32_t v[32];
+#pragma unroll
+              for (int j = 0; j < 32; ++j) v[j] = __float_as_uint(f[j]);
+              ResidualRegs res;                                   // C = C + sum, through the staged fp32 store
+              epilogue_load_residual<EPI_F32_RESIDUAL>(p, res, lane, row0, col0, M);
+              epilogue_chunk<EPI_F32_RESIDUAL>(p, v, res, stage_buf, lane, row0, col0, M);
+            }
+          }
+          if (lane == 0) *ctr = 0;
+        }
+      }
+      if constexpr (EPI == EPI_BF16_ACTBWD_DET) {
+        // The last 32-row chunk to finish these 64 columns adds every chunk's column sums to C2 in row order.
+        if (p.C2 && row0 < M && n_blk * GEMM_BN + part * 64 < p.N) {
+          int* ctr = p.cnt + n_blk * 4 + part;
+          __threadfence();
+          __syncwarp();
+          int old = 0;
+          if (lane == 0) old = atomicAdd(ctr, 1);
+          old = __shfl_sync(0xffffffffu, old, 0);
+          const int chunks = (M + 31) >> 5;
+          if (old == chunks - 1) {
+            __threadfence();
+#pragma unroll 1
+            for (int c = 0; c < 64; c += 32) {
+              const int col = n_blk * GEMM_BN + part * 64 + c + lane;
+              if (col < p.N) {
+                reinterpret_cast<float*>(p.C2)[col] += ordered_sum<16>(p.ws + col, p.N, chunks);
+              }
+            }
+            if (lane == 0) *ctr = 0;
+          }
+        }
+      }
     }
   }
 

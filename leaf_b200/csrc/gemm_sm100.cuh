@@ -40,7 +40,11 @@ constexpr int GEMM_BK = 64;
 constexpr int GEMM_UMMA_K = 16;
 
 enum { EPI_BF16 = 0, EPI_BF16_ACT = 1, EPI_F32_RESIDUAL = 2, EPI_F32 = 3, EPI_F32_SPLITK = 4,   // 4: C += partial sums (red.global.add)
-       EPI_BF16_ACTBWD = 5 };   // 5: C = bf16(acc * act'(U)), U = GemmParams::delta (bf16 [M, ldc]); C2 (fp32 [N], may be null) += column sums
+       EPI_BF16_ACTBWD = 5,     // 5: C = bf16(acc * act'(U)), U = GemmParams::delta (bf16 [M, ldc]); C2 (fp32 [N], may be null) += column sums
+       // Deterministic variants of 4 and 5 (leaf_set_deterministic): the partial sums go to GemmParams::ws, and the epilogue warp
+       // that arrives last at a region (per-region counter in GemmParams::cnt) adds them to C / C2 in index order, so the result
+       // does not depend on which work unit finished first. Own template instances: 4 and 5 keep their code and registers.
+       EPI_F32_SPLITK_DET = 6, EPI_BF16_ACTBWD_DET = 7 };
 enum { ACT_GELU_ERF = 0, ACT_QUICK_GELU = 1 };
 
 struct GemmParams {
@@ -67,6 +71,11 @@ struct GemmParams {
   // epilogues ADD their partial sums into C with red.global.add.v4.f32 (C += A.B is what the weight-gradient products want
   // anyway). Its own template instance, so the hot fc2 epilogue (EPI_F32_RESIDUAL) keeps its register budget. 1 = off.
   int split_k;
+  // EPI_F32_SPLITK_DET: ws holds one 256 x 256 fp32 partial tile per work unit, cnt one arrival counter per (output tile, epilogue
+  // warp of the pair). EPI_BF16_ACTBWD_DET: ws holds the column sums of every 32-row chunk [ceil(M / 32), N], cnt one counter per
+  // 64 columns. Counters are zero before the launch and are left at zero.
+  float* ws;
+  int* cnt;
 };
 constexpr int GEMM_A_MN = 1, GEMM_B_MN = 2;
 // MN-major 128B-swizzled tile as TMA lays it down from a [K, MN] row-major tensor with a 64 (MN) x 64 (k) box: one 128-byte
@@ -174,6 +183,23 @@ __device__ __forceinline__ uint64_t make_smem_desc_mn_sw128(uint32_t saddr, uint
   d |= static_cast<uint64_t>(1) << 46;
   d |= static_cast<uint64_t>(2) << 61;
   return d;
+}
+
+// sum of p[0], p[stride], ..., p[(n - 1) stride], added one after another in index order (the fixed order of the deterministic
+// reductions' last step), with U loads in flight: these sums read L2-resident partials written by other SMs (hence .cg).
+template <int U>
+__device__ __forceinline__ float ordered_sum(const float* p, size_t stride, int n) {
+  float t = 0.f;
+  int i = 0;
+  for (; i + U <= n; i += U) {
+    float v[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) v[u] = __ldcg(p + static_cast<size_t>(i + u) * stride);
+#pragma unroll
+    for (int u = 0; u < U; ++u) t += v[u];
+  }
+  for (; i < n; ++i) t += __ldcg(p + static_cast<size_t>(i) * stride);
+  return t;
 }
 
 __device__ __forceinline__ float fast_ex2(float x) {
@@ -297,7 +323,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32
       for (int j = 0; j < 32; ++j) f[j] = gelu_erf(f[j]);
     }
   }
-  if (EPI == EPI_BF16_ACTBWD) {
+  if (EPI == EPI_BF16_ACTBWD || EPI == EPI_BF16_ACTBWD_DET) {
     // du = dg * act'(u) (the backward's dgrad through fc2, fused with what was a separate activation-backward pass). The u tile comes in through the
     // staging buffer (8 rows x 64 B per load instruction), each lane then reads its own row; rows past M are zeroed (their
     // accumulators are whatever lay behind the operand) so that the column sums below - the gradient of fc1's bias - see
@@ -340,7 +366,11 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32
           f[j] = keep + __shfl_xor_sync(0xffffffffu, send, off);
         }
       }
-      if (col0 + lane < p.N) atomicAdd(reinterpret_cast<float*>(p.C2) + col0 + lane, f[0]);
+      if (EPI == EPI_BF16_ACTBWD_DET) {
+        if (col0 + lane < p.N) p.ws[static_cast<size_t>(row0 >> 5) * p.N + col0 + lane] = f[0];
+      } else if (col0 + lane < p.N) {
+        atomicAdd(reinterpret_cast<float*>(p.C2) + col0 + lane, f[0]);
+      }
     }
   } else if (EPI == EPI_BF16 || EPI == EPI_BF16_ACT) {
     store_bf16(p.C);

@@ -113,11 +113,15 @@ __global__ void __launch_bounds__(256, VPL <= 10 ? 2 : 1) layernorm_bwd_rows_ker
 // dgamma[c] += sum_r dy[r,c] xhat[r,c], dbeta[c] += sum_r dy[r,c], dxsum[c] += sum_r dx[row(r),c] (dxsum may be null) over the
 // rows of this CTA's band. CTA = 64 column quads (256 columns) x 4 row phases; grid = (ceil(W / 256), bands).
 // Launched behind layernorm_bwd_rows_kernel with programmatic stream serialization: it reads that kernel's stats and dx.
+// DET (leaf_set_deterministic): each band writes its sums to ws [bands][3][W] instead of adding them, and the last band of a
+// column block to finish (counter cnt[blockIdx.x], zero before and after) adds them to the gradients in band order.
+template <bool DET>
 __global__ void __launch_bounds__(256) layernorm_bwd_cols_kernel(const float* __restrict__ dy, const float* __restrict__ x,
                                                                  const int* __restrict__ gather, const float2* __restrict__ stats,
                                                                  const float* __restrict__ dx, int rows, int W,
                                                                  float* __restrict__ dgamma, float* __restrict__ dbeta,
-                                                                 float* __restrict__ dxsum) {
+                                                                 float* __restrict__ dxsum, float* __restrict__ ws = nullptr,
+                                                                 int* __restrict__ cnt = nullptr) {
   pdl_wait();
   pdl_trigger();
   __shared__ float4 red[3][4][64];
@@ -149,9 +153,32 @@ __global__ void __launch_bounds__(256) layernorm_bwd_cols_kernel(const float* __
   __syncthreads();
   // 768 sums per CTA (3 arrays x 256 columns): thread t takes column t of each array
   const int col = blockIdx.x * 256 + threadIdx.x;
-  if (col < W && r1 > r0) {
-    const float* f = reinterpret_cast<const float*>(&red[0][0][0]);      // [array][phase][256 floats]
-    float* dst[3] = {dgamma, dbeta, dxsum};
+  const float* f = reinterpret_cast<const float*>(&red[0][0][0]);        // [array][phase][256 floats]
+  float* dst[3] = {dgamma, dbeta, dxsum};
+  if constexpr (DET) {
+    __shared__ bool last;
+    if (col < W) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        const float* a = f + (k * 4) * 256 + threadIdx.x;
+        ws[(static_cast<size_t>(blockIdx.y) * 3 + k) * W + col] = (a[0] + a[256]) + (a[512] + a[768]);
+      }
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) last = atomicAdd(cnt + blockIdx.x, 1) == static_cast<int>(gridDim.y) - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    if (col < W) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        if (!dst[k]) continue;
+        dst[k][col] += ordered_sum<8>(ws + static_cast<size_t>(k) * W + col, static_cast<size_t>(3) * W, gridDim.y);
+      }
+    }
+    if (threadIdx.x == 0) cnt[blockIdx.x] = 0;
+  } else if (col < W && r1 > r0) {
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       if (!dst[k]) continue;
@@ -306,12 +333,16 @@ __device__ __forceinline__ void attb_colsum(const float (&acc)[8][4], float (&su
 // the rows beyond a sequence's length are exactly zero in all three, so they do not disturb the sums)
 // Two warps per (sequence, head): they split the staging rows, the query tiles of pass 1 and the key tiles of pass 2 (round
 // robin; the shared-memory footprint - what limits the CTAs per SM - is per item, so the second warp doubles the warps in flight).
+// DET (leaf_set_deterministic): each warp writes its column sums to ws [sequence][warp][q|k|v][W] instead of adding them, and
+// the last CTA of a head to finish (counter cnt[head], zero before and after) adds them in (sequence, warp) order.
 constexpr int ATTB_WARPS = 2;
+template <bool DET>
 __global__ void __launch_bounds__(ATTB_WARPS * 32) attention_bwd_kernel(const __nv_bfloat16* __restrict__ qkv, const __nv_bfloat16* __restrict__ o,
                                                            const float* __restrict__ dout, const int4* __restrict__ meta,
                                                            int W, int T, __nv_bfloat16* __restrict__ dqkv,
                                                            float* __restrict__ db_q = nullptr, float* __restrict__ db_k = nullptr,
-                                                           float* __restrict__ db_v = nullptr) {
+                                                           float* __restrict__ db_v = nullptr, float* __restrict__ ws = nullptr,
+                                                           int* __restrict__ cnt = nullptr) {
   pdl_trigger();
   extern __shared__ __align__(16) uint8_t attb_sm[];
   const int T16 = (T + 15) / 16 * 16, PP = T16 + 8;
@@ -422,7 +453,33 @@ __global__ void __launch_bounds__(ATTB_WARPS * 32) attention_bwd_kernel(const __
       }
     }
   }
-  if (g == 0) {
+  if constexpr (DET) {
+    if (!db_q && !db_k && !db_v) return;                 // uniform over the grid
+    __shared__ bool last;
+    if (g == 0) {
+      float* w = ws + static_cast<size_t>(seq * ATTB_WARPS + warp) * 3 * W;
+#pragma unroll
+      for (int n8 = 0; n8 < 8; ++n8) {
+        const int col = head * 64 + 8 * n8 + 2 * c;
+        *reinterpret_cast<float2*>(w + col) = make_float2(sq[n8][0], sq[n8][1]);
+        *reinterpret_cast<float2*>(w + W + col) = make_float2(sk[n8][0], sk[n8][1]);
+        *reinterpret_cast<float2*>(w + 2 * W + col) = make_float2(sv[n8][0], sv[n8][1]);
+      }
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) last = atomicAdd(cnt + head, 1) == static_cast<int>(gridDim.x) - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    float* dst[3] = {db_q, db_k, db_v};
+    for (int j = threadIdx.x; j < 3 * 64; j += ATTB_WARPS * 32) {
+      const int k = j >> 6, col = head * 64 + (j & 63);
+      if (!dst[k]) continue;
+      dst[k][col] += ordered_sum<16>(ws + static_cast<size_t>(k) * W + col, static_cast<size_t>(3) * W, gridDim.x * ATTB_WARPS);
+    }
+    if (threadIdx.x == 0) cnt[head] = 0;
+  } else if (g == 0) {
 #pragma unroll
     for (int n8 = 0; n8 < 8; ++n8) {
       const int col = head * 64 + 8 * n8 + 2 * c;
@@ -450,6 +507,123 @@ __global__ void __launch_bounds__(256) embed_bwd_kernel(const int* __restrict__ 
       atomicAdd(dpos + static_cast<size_t>(pos) * W + c, v);
     }
   }
+}
+
+// ---- deterministic embedding backward (leaf_set_deterministic): one writer per table row, summing in packed-row order ---------
+// embed_sort_kernel (one CTA, LEAF_VOCAB ints of shared memory) groups the packed rows by token id with a stable counting sort:
+// row_tok[r] = token id of packed row r, order[] = the rows sorted by (id, row), key[i] = row_tok[order[i]].
+__global__ void __launch_bounds__(1024) embed_sort_kernel(const int* __restrict__ tok, const int4* __restrict__ meta, int N, int M,
+                                                          int* __restrict__ row_tok, int* __restrict__ order, int* __restrict__ key) {
+  extern __shared__ int cursor[];                          // [LEAF_VOCAB]: counts, then the next free slot of each id
+  __shared__ int wsum[32];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (int i = tid; i < LEAF_VOCAB; i += 1024) cursor[i] = 0;
+  __syncthreads();
+  for (int i = tid; i < N * LEAF_CTX; i += 1024) {
+    const int seq = i / LEAF_CTX, pos = i - seq * LEAF_CTX;
+    const int4 mt = meta[seq];
+    if (pos >= mt.z && pos < mt.y) {
+      const int id = tok[i];
+      row_tok[mt.x + pos - mt.z] = id;
+      atomicAdd(cursor + id, 1);
+    }
+  }
+  __syncthreads();
+  // exclusive scan of the counts: thread t owns ids [t * per, (t + 1) * per)
+  constexpr int per = (LEAF_VOCAB + 1023) / 1024;
+  const int lo = tid * per, hi = min(lo + per, static_cast<int>(LEAF_VOCAB));
+  int s = 0;
+  for (int i = lo; i < hi; ++i) s += cursor[i];
+  int incl = s;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  if (lane == 31) wsum[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    int w = wsum[lane];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int v = __shfl_up_sync(0xffffffffu, w, o);
+      if (lane >= o) w += v;
+    }
+    wsum[lane] = w;                                        // inclusive over warps
+  }
+  __syncthreads();
+  int run = incl - s + (warp ? wsum[warp - 1] : 0);
+  for (int i = lo; i < hi; ++i) { const int c = cursor[i]; cursor[i] = run; run += c; }
+  __syncthreads();
+  // stable scatter in row order by one warp, 32 rows per step (ids of 8 steps loaded ahead)
+  if (warp == 0) {
+    for (int b0 = 0; b0 < M; b0 += 256) {
+      int ids[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) ids[u] = (b0 + 32 * u + lane < M) ? row_tok[b0 + 32 * u + lane] : -1;
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        const int r = b0 + 32 * u + lane, id = ids[u];
+        const unsigned peers = __match_any_sync(0xffffffffu, id);
+        const int start = id >= 0 ? cursor[id] : 0;
+        __syncwarp();
+        if (id >= 0) {
+          const int at = start + __popc(peers & ((1u << lane) - 1u));
+          order[at] = r;
+          key[at] = id;
+          if (lane == 31 - __clz(peers)) cursor[id] = start + __popc(peers);
+        }
+        __syncwarp();
+      }
+    }
+  }
+}
+
+// grid (M + LEAF_CTX, ceil(W / 256)): block x < M that starts a run of equal keys adds dtok[id] += the run's dx rows in row
+// order; block x = M + pos adds dpos[pos] += the dx rows of position pos in sequence order.
+__global__ void __launch_bounds__(256) embed_bwd_det_kernel(const int* __restrict__ order, const int* __restrict__ key,
+                                                            const int4* __restrict__ meta, int N, int M, int W,
+                                                            const float* __restrict__ dx, float* __restrict__ dtok,
+                                                            float* __restrict__ dpos) {
+  const int c = blockIdx.y * 256 + threadIdx.x;
+  const int i = blockIdx.x;
+  if (i < M) {
+    const int id = key[i];
+    if ((i > 0 && key[i - 1] == id) || c >= W) return;
+    float t = 0.f;
+    for (int j = i; j < M; j += 8) {
+      int rows[8];
+      bool in[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        in[u] = j + u < M && key[j + u] == id;
+        rows[u] = in[u] ? order[j + u] : 0;
+      }
+      float v[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) v[u] = in[u] ? dx[static_cast<size_t>(rows[u]) * W + c] : 0.f;
+#pragma unroll
+      for (int u = 0; u < 8; ++u)
+        if (in[u]) t += v[u];
+      if (!in[7]) break;
+    }
+    dtok[static_cast<size_t>(id) * W + c] += t;
+    return;
+  }
+  const int pos = i - M;
+  if (c >= W) return;
+  float t = 0.f;
+  for (int s0 = 0; s0 < N; s0 += 8) {                      // 8 sequences' loads in flight, added in sequence order
+    float v[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      const int4 mt = s0 + u < N ? meta[s0 + u] : make_int4(0, 0, 0, 0);
+      v[u] = (pos >= mt.z && pos < mt.y) ? dx[static_cast<size_t>(mt.x + pos - mt.z) * W + c] : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u) t += v[u];
+  }
+  dpos[static_cast<size_t>(pos) * W + c] += t;
 }
 
 // ---- AdamW over the tower's flat parameter buffer (torch.optim.AdamW semantics, decoupled weight decay;
@@ -480,7 +654,11 @@ __global__ void __launch_bounds__(256) adamw_kernel(float* __restrict__ p, const
 }
 
 // sum of squares of a flat fp32 buffer (gradient-norm clipping, utils_AT.py:349-357): out[0] += sum(g^2)
-__global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, size_t n, float* __restrict__ out) {
+// DET (leaf_set_deterministic): every block writes its sum to ws[blockIdx.x]; the last block to finish (counter *cnt, zero before
+// and after) adds them up in a fixed order: thread t takes blocks t, t + 256, ..., then the block reduction below.
+template <bool DET>
+__global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, size_t n, float* __restrict__ out,
+                                                    float* __restrict__ ws = nullptr, int* __restrict__ cnt = nullptr) {
   __shared__ float part[8];
   float s = 0.f;
   const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x * 4;
@@ -495,7 +673,30 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g,
     float t = 0.f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) t += part[i];
-    atomicAdd(out, t);
+    if constexpr (DET) ws[blockIdx.x] = t;
+    else atomicAdd(out, t);
+  }
+  if constexpr (DET) {
+    __shared__ bool last;
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) last = atomicAdd(cnt, 1) == static_cast<int>(gridDim.x) - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    float u = 0.f;
+    for (int b = threadIdx.x; b < static_cast<int>(gridDim.x); b += 256) u += __ldcg(ws + b);
+    u = warp_sum(u);
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = u;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      float t = 0.f;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) t += part[i];
+      out[0] += t;
+      *cnt = 0;
+    }
   }
 }
 

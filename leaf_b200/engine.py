@@ -113,6 +113,7 @@ class LeafEngine:
             check(self._lib.leaf_load_bpe(self._h, pairs.ctypes.data_as(ctypes.c_void_p), len(pairs)))
             self._bind()
         self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self.deterministic = False
         self.has_words = False
         self.max_seqs = 0
         self._caption_limit = MAX_CAPTION_BYTES
@@ -255,6 +256,16 @@ class LeafEngine:
                                      (16, "constraint filter buffer overflow")) if st & bit]
             raise LeafError("tokenizer kernel: " + "; ".join(what))
 
+    def set_deterministic(self, on: bool):
+        """Bit-reproducible gradients (leaf_set_deterministic): backward() and the gradient-norm reduction sum in a fixed order
+        instead of with atomics. backward() and FareTrainer follow torch.use_deterministic_algorithms on their own, so a caller
+        never needs this; the forward is deterministic either way."""
+        on = bool(on)
+        if on != self.deterministic:
+            with torch.cuda.device(self.device):
+                check(self._lib.leaf_set_deterministic(self._h, 1 if on else 0))
+            self.deterministic = on
+
     def set_tokenizer_mode(self, hf: bool):
         """hf=True: token ids of transformers' CLIPTokenizer (the reference's HF evaluation path, utils_attacks.py:67-71)
         instead of open_clip's SimpleTokenizer: no html.unescape, <|startoftext|> / <|endoftext|> spellings."""
@@ -364,6 +375,7 @@ class LeafEngine:
                 raise LeafError("gradient buffers must be contiguous fp32 CUDA tensors")
         keep = self._make_ptrs(c)
         with torch.cuda.device(self.device):
+            self.set_deterministic(torch.are_deterministic_algorithms_enabled())
             check(self._lib.leaf_backward(self._h, int(generation), _ptr(dfeat.to(torch.float32).contiguous()), int(dfeat.shape[0]),
                                           ctypes.byref(keep[1]), _stream()))
 

@@ -143,6 +143,7 @@ class FareTrainer:
     def _clip_scale(self, grad_scale: float = 1.0) -> float:
         """torch.nn.utils.clip_grad_norm_(norm_type=2): the factor min(1, max_norm / (total_norm + 1e-6))."""
         eng, g = self.tower.leaf_engine, self.tower.flat_grads
+        eng.set_deterministic(torch.are_deterministic_algorithms_enabled())
         self._norm.zero_()
         check(eng._lib.leaf_sumsq(eng._h, _ptr(g), g.numel(), _ptr(self._norm), _stream()))
         total = math.sqrt(float(self._norm.item())) * grad_scale
