@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIB_DIR, "libleaf_b200.so")
 SOURCES = ["engine.cu"]
-HEADERS = ["gemm_sm100.cuh", "gemm2_sm100.cuh", "train_kernels.cuh", "tower_kernels.cuh", "attention2.cuh", "k1_core.cuh", "k1_tokenize.cuh", "constrain_core.cuh", "constrain_kernel.cuh", "k1_tables_host.h", "k1_tables.inc",
+HEADERS = ["gemm_sm100.cuh", "gemm2_sm100.cuh", "train_kernels.cuh", "tower_kernels.cuh", "k1_core.cuh", "k1_tokenize.cuh", "constrain_core.cuh", "constrain_kernel.cuh", "k1_tables_host.h", "k1_tables.inc",
            os.path.join("..", "..", "include", "leaf_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

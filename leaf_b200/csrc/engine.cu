@@ -22,7 +22,6 @@
 #include "constrain_kernel.cuh"
 #include "k1_tokenize.cuh"
 #include "tower_kernels.cuh"
-#include "attention2.cuh"
 #include "train_kernels.cuh"
 
 using namespace leaf;
@@ -126,7 +125,6 @@ struct leaf_engine {
   bool deterministic = false;         // leaf_set_deterministic: fixed-order reductions in leaf_backward / leaf_sumsq
   float* det_sum_ws = nullptr;        // leaf_sumsq's per-block sums and arrival counter in deterministic mode
   int* det_sum_cnt = nullptr;
-  int att_impl = 1;                   // 1 = register-fed attention_kernel (default: faster in situ), 2 = cp.async ring attention2_kernel (LEAF_ATTENTION_IMPL=2)
   int *cu = nullptr, *eos_row = nullptr, *total_rows = nullptr, *pfx = nullptr, *own_len = nullptr, *dup_of = nullptr, *need = nullptr;
   int4* meta = nullptr;
   // bookkeeping
@@ -336,9 +334,6 @@ extern "C" int leaf_create(const leaf_cfg_t* cfg, leaf_handle_t* out) {
   CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD_DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(embed_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LEAF_VOCAB * 4));
   CK(cudaFuncSetAttribute(topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  CK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AT2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  if (const char* ai = getenv("LEAF_ATTENTION_IMPL")) e->att_impl = atoi(ai) == 2 ? 2 : 1;
   if (const char* pd = getenv("LEAF_PDL")) e->pdl = atoi(pd) != 0;
   CK(cudaFuncSetAttribute(attention_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
   CK(cudaFuncSetAttribute(attention_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
@@ -444,10 +439,9 @@ extern "C" int leaf_refresh_weights(leaf_handle_t e, void* stream) {
       if ((rc = cast_to(e, p.q_w, w.qkv_w, W * W, st))) return rc;
       if ((rc = cast_to(e, p.k_w, w.qkv_w + W * W, W * W, st))) return rc;
       if ((rc = cast_to(e, p.v_w, w.qkv_w + 2 * W * W, W * W, st))) return rc;
-      copy_f32_kernel<<<8, 256, 0, st>>>(p.q_b, w.qkv_b_own, W);
-      copy_f32_kernel<<<8, 256, 0, st>>>(p.k_b, w.qkv_b_own + W, W);
-      copy_f32_kernel<<<8, 256, 0, st>>>(p.v_b, w.qkv_b_own + 2 * W, W);
-      e->launches += 3;
+      CK(cudaMemcpyAsync(w.qkv_b_own, p.q_b, W * sizeof(float), cudaMemcpyDeviceToDevice, st));
+      CK(cudaMemcpyAsync(w.qkv_b_own + W, p.k_b, W * sizeof(float), cudaMemcpyDeviceToDevice, st));
+      CK(cudaMemcpyAsync(w.qkv_b_own + 2 * W, p.v_b, W * sizeof(float), cudaMemcpyDeviceToDevice, st));
       w.qkv_b = w.qkv_b_own;
     }
     if ((rc = cast_to(e, p.out_w, w.out_w, W * W, st))) return rc;
@@ -588,17 +582,8 @@ static int launch_layernorm(leaf_engine* e, const float* x, const int* rows_dev,
 
 // causal attention over the packed rows (tower_kernels.cuh)
 static int launch_attention(leaf_engine* e, const __nv_bfloat16* qkv, const int4* meta, int N, __nv_bfloat16* out, int last_only,
-                            cudaStream_t st, long rows_cap_hint = 0) {
-  if (rows_cap_hint <= 0) rows_cap_hint = static_cast<long>(N) * LEAF_CTX;      // no sequence has more than 77 rows
+                            cudaStream_t st) {
   const int H = e->cfg.heads, W = e->cfg.width;
-  if (e->att_impl == 2 && static_cast<unsigned long long>(rows_cap_hint) * 3ull * W < (1ull << 32)) {
-    const long ctas = (static_cast<long>(N) * H + AT2_WARPS - 1) / AT2_WARPS;
-    const int grid2 = static_cast<int>(ctas < 2L * e->sm_count ? ctas : 2L * e->sm_count);     // persistent: 2 CTAs of 8 warps per SM
-    attention2_kernel<<<grid2, AT2_WARPS * 32, AT2_SMEM_BYTES, st>>>(qkv, meta, N, H, W, out, last_only);
-    e->launches++;
-    CK(cudaGetLastError());
-    return LEAF_OK;
-  }
   const int grid = (N * H + ATT_WARPS - 1) / ATT_WARPS;
   CK(launch_pdl(e, attention_kernel, dim3(grid), dim3(ATT_WARPS * 32), st, qkv, meta, N, H, W, out, last_only));
   e->launches++;
@@ -810,9 +795,10 @@ extern "C" double leaf_timing_ms(leaf_handle_t e, int32_t which, int32_t* launch
 
 // =====================================================================================================================
 // K4: forward in train mode (activations kept) and backward of the selected adversarial batch
-// (/root/reference/utils_AT.py:312-337). Every product is a TN GEMM on the tcgen05 kernel:
-//   dgrad  dX[M,in]   = dY[M,out] . W[out,in]            -> A = dY (bf16),        Bt = W^T copy [in,out]
-//   wgrad  dW[out,in] += dY^T[out,M] . X[M,in]           -> A = dY^T [out,Mp],    Bt = X^T [in,Mp]   (fp32 accumulate into .grad)
+// (/root/reference/utils_AT.py:312-337). Every product runs on the tcgen05 kernel and reads its operands as they lie:
+//   dgrad  dX[M,in]   = dY[M,out] . W[out,in]            -> A = dY (bf16, K-major), B = W [out,in] MN-major (GEMM_B_MN)
+//   wgrad  dW[out,in] += dY^T[out,M] . X[M,in]           -> A = dY [M,out], B = X [M,in], both MN-major (GEMM_A_MN | GEMM_B_MN;
+//                                                           fp32 accumulate into .grad)
 // =====================================================================================================================
 template <typename Tp>
 static int tw_alloc(TrainWs& t, Tp** p, size_t count) {

@@ -7,7 +7,7 @@
 // 4.2 MFLOP (131 FLOP/B); the ring holds 5 stages and 40 KB are left for the 16 epilogue warps' staging buffers.
 //
 // Protocol (per stage s; "leader" = CTA rank 0 of the pair):
-//   producers (warp 0 of BOTH CTAs) wait on their local empty[s], then TMA their A and B boxes into local smem with
+//   producers (warp WARP_TMA = 16 of BOTH CTAs) wait on their local empty[s], then TMA their A and B boxes into local smem with
 //     cp.async.bulk.tensor...cta_group::2, whose complete_tx lands on the LEADER's full[s]; the leader's producer
 //     arms full[s] with the bytes of both CTAs;
 //   the leader's MMA thread waits full[s], issues 4 MMAs, then tcgen05.commit...multicast::cluster arrives on empty[s]

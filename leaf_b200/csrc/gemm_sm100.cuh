@@ -37,7 +37,6 @@ __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.lau
 
 constexpr int GEMM_BN = 256;
 constexpr int GEMM_BK = 64;
-constexpr int GEMM_UMMA_K = 16;
 
 enum { EPI_BF16 = 0, EPI_BF16_ACT = 1, EPI_F32_RESIDUAL = 2, EPI_F32 = 3, EPI_F32_SPLITK = 4,   // 4: C += partial sums (red.global.add)
        EPI_BF16_ACTBWD = 5,     // 5: C = bf16(acc * act'(U)), U = GemmParams::delta (bf16 [M, ldc]); C2 (fp32 [N], may be null) += column sums
@@ -94,9 +93,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 // Bounded wait: a protocol bug must end in a trap (reported as a CUDA error), never in a hung GPU.
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   uint32_t done = 0;
@@ -114,35 +110,11 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     if (it > 1024 && (it & 1023) == 0 && clock64() - t0 > 4000000000LL) __trap();
   }
 }
-__device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap* tmap, uint32_t bar, int x, int y) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar), "r"(x), "r"(y)
-      : "memory");
-}
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* tmap) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tmap)) : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(cols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* v) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 "

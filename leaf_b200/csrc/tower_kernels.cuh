@@ -15,11 +15,6 @@ __device__ __forceinline__ float warp_sum(float v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 
 // ---------------------------------------------------------------------------------------------
 // exclusive scan of the (own) row lengths -> cu[N+1]; clamps to [0, 77]. Single CTA (N <= ~10^5).
@@ -610,25 +605,4 @@ __global__ void cast_bf16_transpose_kernel(const float* __restrict__ src /*[R,C]
     if (c < C && r < R) dst[static_cast<size_t>(c) * R + r] = __float2bfloat16_rn(tile[threadIdx.x][i]);
   }
 }
-// same with a destination row pitch (writes a [C,R] block into a wider matrix)
-__global__ void cast_bf16_transpose_ld_kernel(const float* __restrict__ src /*[R,C]*/, __nv_bfloat16* __restrict__ dst, int R, int C,
-                                              int ld_dst) {
-  __shared__ float tile[32][33];
-  const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int r = r0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (r < R && c < C) ? src[static_cast<size_t>(r) * C + c] : 0.f;
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int c = c0 + i, r = r0 + threadIdx.x;
-    if (c < C && r < R) dst[static_cast<size_t>(c) * ld_dst + r] = __float2bfloat16_rn(tile[threadIdx.x][i]);
-  }
-}
-__global__ void copy_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, size_t n) {
-  size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x;
-  for (; i < n; i += stride) dst[i] = src[i];
-}
-
 }  // namespace leaf

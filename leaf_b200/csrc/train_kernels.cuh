@@ -700,25 +700,4 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g,
   }
 }
 
-// dst[r, :] += src[r, :] (fp32), used to add the attention/MLP branch gradient into the running dx
-__global__ void add_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, size_t n) {
-  for (size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x)
-    dst[i] += src[i];
-}
-
-// dst[W,E] += src[E,W]^T (HF projection layout -> open_clip layout or back), fp32
-__global__ void add_transposed_f32_kernel(const float* __restrict__ src, float* __restrict__ dst, int R, int C) {
-  __shared__ float tile[32][33];
-  const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int r = r0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (r < R && c < C) ? src[static_cast<size_t>(r) * C + c] : 0.f;
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int c = c0 + i, r = r0 + threadIdx.x;
-    if (c < C && r < R) dst[static_cast<size_t>(c) * R + r] += tile[threadIdx.x][i];
-  }
-}
-
 }  // namespace leaf

@@ -132,39 +132,6 @@ def test_attention_varlen_causal(eng):
         assert torch.allclose(out[t0:], ref_attn(q[p:], k, v, p), atol=3e-2, rtol=2e-2), p
 
 
-def test_attention_ring_kernel_matches(eng, monkeypatch):
-    """The cp.async-ring form (csrc/attention2.cuh, LEAF_ATTENTION_IMPL=2: measured, not the default) on the same checks:
-    against torch on every length class and with shared prefixes, against the default kernel within the bf16 rounding of the
-    output, bit-identical with and without prefix sharing, and through a whole attack step."""
-    from leaf_b200 import synth
-    from leaf_b200.tower import LeafTextTower
-    monkeypatch.setenv("LEAF_ATTENTION_IMPL", "2")
-    tower2 = LeafTextTower(synth.random_tower_state_dict(synth.TOWERS["small"], seed=3, device="cuda"), heads=4)
-    monkeypatch.delenv("LEAF_ATTENTION_IMPL")
-    eng2 = tower2.leaf_engine
-    test_attention_varlen_causal(eng2)
-    g = torch.Generator(device="cuda").manual_seed(5)
-    W = eng.width
-    lens = [77, 1, 30, 18, 64, 2, 47]
-    cu = np.concatenate([[0], np.cumsum(lens)])
-    qkv = torch.randn((int(cu[-1]), 3 * W), generator=g, device="cuda").to(torch.bfloat16)
-    meta = torch.tensor([[cu[i], t, 0, cu[i]] for i, t in enumerate(lens)], dtype=torch.int32, device="cuda")
-    assert (eng2.test_attention(qkv, meta).float() - eng.test_attention(qkv, meta).float()).abs().max() <= 2e-2
-    B, n = 6, 20
-    caps = synth.make_captions(B, seed=4)
-    rng = np.random.RandomState(1)
-    pos = torch.from_numpy(np.stack([rng.randint(0, 2 * len(S) + 1, size=n) for S in caps]).astype(np.int32)).cuda()
-    chr_ = torch.from_numpy(np.array(synth.V_DEFAULT, dtype=np.int32)[rng.randint(0, 96, size=(B, n))]).cuda()
-    d, o = eng2.upload_captions(caps)
-    tok, ln, base = eng2.expand_tokenize(d, o, B, n, pos, chr_)
-    shared = eng2.encode_tokens(tok, ln, False, base, (B * n, n))
-    assert torch.equal(shared, eng2.encode_tokens(tok, ln, False, None))         # packing changes no bit
-    sd = {k: v.cpu() for k, v in tower2.open_clip_state_dict().items()}
-    ref_tower = LeafTextTower(sd, heads=4)
-    want = ref_tower.leaf_engine.encode_tokens(tok, ln, False, base, (B * n, n))
-    assert torch.nn.functional.cosine_similarity(shared, want, dim=-1).min() >= 0.9999
-
-
 def test_attention_backward_kernel(eng):
     """K4's tensor-core attention backward against torch autograd of an fp32 attention on the same bf16 inputs: every
     length class (1 row, tile boundaries 16 / 17 / 32 / 33, the full 77)."""

@@ -1,14 +1,10 @@
 """Timing of the attention kernel alone on the bench workload's real sequence shapes.
 
-    python tools/ab_attention.py [variants ...]
+    python tools/ab_attention.py
 
 Builds the packed-row metadata of both attack phases of the ViT-H bench workload on the host (same rule as
 prefix_kernel / meta_kernel, without duplicate elimination), fills qkv with random bf16 and times leaf_test_attention
-with CUDA events. While a kernel is being developed the engine reads LEAF_ATT_VARIANT at leaf_create and this script
-alternates the variants on one box (clock drift hits all alike) and compares every output with the first variant's:
-profiles/r34_attention_ab.log is the run that chose the shipped kernel (variant 0 = 128-bit loads, 1 = the same with a
-software-pipelined load ring, 3/4/5 = 256-bit loads at 4/3/5 CTAs per SM). The shipped engine has one kernel and
-ignores the variable, so the default is a single timing.
+with CUDA events. To compare two builds, run it once per build with LEAF_B200_LIB naming the library.
 """
 import os
 import sys
@@ -41,17 +37,12 @@ def host_meta(tok, ln, base):
 
 
 def main():
-    variants = [int(v) for v in sys.argv[1:]] or [0]
     dev = torch.device("cuda", 0)
     B, n = 128, 50
     caps = synth.make_captions(B, seed=100, kind="typical")
-    engines = {}
     H, W = 16, 1024
     cfg = synth.TowerCfg("ab", W, 1, H, 1024)               # the kernel only depends on heads and width
-    for v in variants:
-        os.environ["LEAF_ATTENTION_IMPL"] = str(v)
-        engines[v] = LeafTextTower.random(cfg, seed=0, device=dev).leaf_engine
-    eng = engines[variants[0]]
+    eng = LeafTextTower.random(cfg, seed=0, device=dev).leaf_engine
     assert eng.width == W and eng.heads == H, (eng.width, eng.heads)
     rs = np.random.RandomState(0)
     Vt = np.asarray(V_DEFAULT, dtype=np.int32)
@@ -68,34 +59,23 @@ def main():
     for ph, (meta, rows) in enumerate(phases):
         meta_d = torch.from_numpy(meta).to(dev)
         qkv = (torch.randn((rows, 3 * W), device=dev) * 0.5).to(torch.bfloat16)
-        ref = None
-        for v in variants:
-            out = engines[v].test_attention(qkv, meta_d)
-            if ref is None:
-                ref = out
-            else:
-                d = (out.float() - ref.float()).abs().max().item()
-                print(f"  variant {v} vs {variants[0]}: max |diff| = {d:.3g}" + ("" if d else " (bit-identical)"))
-                assert d < 2e-2, f"variant {v} differs from variant {variants[0]}"
-        times = {v: [] for v in variants}
-        out = torch.empty_like(ref)
+        out = eng.test_attention(qkv, meta_d)
+        times = []
         for rep in range(6):
-            for v in variants:
-                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a.record()
-                for _ in range(10):
-                    engines[v].test_attention(qkv, meta_d, out)
-                b.record()
-                torch.cuda.synchronize()
-                if rep:
-                    times[v].append(a.elapsed_time(b) / 10)
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            for _ in range(10):
+                eng.test_attention(qkv, meta_d, out)
+            b.record()
+            torch.cuda.synchronize()
+            if rep:
+                times.append(a.elapsed_time(b) / 10)
         nkt = ((np.minimum(meta[:, 1] - 1, 76)) >> 4) + 1
         print(f"phase {ph + 1}: rows={rows} seqs={len(meta)} mean t={meta[:, 1].mean():.1f} mean own={(meta[:, 1] - meta[:, 2]).mean():.1f} "
               f"nkt hist={np.bincount(nkt, minlength=6)[1:].tolist()}")
-        for v in variants:
-            ms = np.array(times[v])
-            gb = rows * W * 8 / 1e9
-            print(f"  variant {v}: {ms.mean() * 1e3:8.1f} us  (min {ms.min() * 1e3:.1f})  {gb / ms.mean() * 1e3 / 1e3:.2f} TB/s algorithmic")
+        ms = np.array(times)
+        gb = rows * W * 8 / 1e9
+        print(f"  {ms.mean() * 1e3:8.1f} us  (min {ms.min() * 1e3:.1f})  {gb / ms.mean() * 1e3 / 1e3:.2f} TB/s algorithmic")
 
 
 if __name__ == "__main__":
