@@ -13,6 +13,7 @@
 #include <map>
 #include <string>
 #include <tuple>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/leaf_b200.h"
@@ -48,6 +49,9 @@ static int fail(int code, const char* fmt, ...) {
 typedef CUresult (*encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// Classes of leaf_timing_ms, numbered as include/leaf_b200.h documents them (public ABI)
+enum TimingClass { TC_GEMM = 0, TC_LAYERNORM = 1, TC_ATTENTION = 2, TC_PACK = 3, TC_EPI = 4, TC_FC2 = 8, TC_OUT_PROJ = 9, TC_COUNT = 10 };
 
 struct LayerW {
   __nv_bfloat16 *qkv_w = nullptr, *out_w = nullptr, *fc1_w = nullptr, *fc2_w = nullptr;   // engine-owned bf16 copies
@@ -130,55 +134,34 @@ struct leaf_engine {
   // bookkeeping
   int64_t launches = 0;
   bool timing = false;
-  struct Span { cudaEvent_t a, b; int cat; };
-  std::vector<Span> spans;            // cat: 0 GEMM, 1 LayerNorm, 2 attention, 3 everything else of the encode
-  double span_ms[10] = {0};        // 4 + epi: the GEMM launches of one epilogue kind (also counted in class 0);
-  int span_n[10] = {0};            // 8: the residual GEMMs with K > N (fc2), counted in class 6 as well; 9: bf16 store, N == K (out-proj)
+  struct Span { cudaEvent_t a, b; int cat; };   // cat: a TimingClass
+  std::vector<Span> spans;
+  double span_ms[TC_COUNT] = {0};
+  int span_n[TC_COUNT] = {0};
   std::vector<cudaEvent_t> event_pool;
-  std::map<std::tuple<const void*, long, long, int>, CUtensorMap> tmaps;
+  std::map<std::tuple<const void*, long, long, long, int, int>, CUtensorMap> tmaps;   // make_tmap's arguments
 };
 
 extern "C" const char* leaf_last_error(void) { return g_err.c_str(); }
 extern "C" const char* leaf_version(void) { return "leaf_b200 0.1 (sm_100a)"; }
 
-static int make_tmap(leaf_engine* e, const void* ptr, long rows, long cols, int box_rows, CUtensorMap* out) {
-  auto key = std::make_tuple(ptr, rows, cols, box_rows);
+// TMA map of a bf16 matrix [outer, inner] with a row pitch of pitch_elems elements, read in 128-byte-swizzled boxes of
+// [box_outer, box_inner]; cached per argument tuple.
+static int make_tmap(leaf_engine* e, const void* ptr, long inner, long outer, long pitch_elems, int box_inner, int box_outer,
+                     CUtensorMap* out) {
+  auto key = std::make_tuple(ptr, inner, outer, pitch_elems, box_inner, box_outer);
   auto it = e->tmaps.find(key);
   if (it != e->tmaps.end()) { *out = it->second; return LEAF_OK; }
-  if (cols % 8 != 0) return fail(LEAF_ERR_INVALID, "GEMM K (%ld) must be a multiple of 8", cols);
   if (reinterpret_cast<uintptr_t>(ptr) & 15) return fail(LEAF_ERR_INVALID, "GEMM operand must be 16-byte aligned");
-  cuuint64_t dims[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
-  cuuint64_t strides[1] = {static_cast<cuuint64_t>(cols) * 2};
-  cuuint32_t box[2] = {static_cast<cuuint32_t>(GEMM_BK), static_cast<cuuint32_t>(box_rows)};
+  cuuint64_t dims[2] = {static_cast<cuuint64_t>(inner), static_cast<cuuint64_t>(outer)};
+  cuuint64_t strides[1] = {static_cast<cuuint64_t>(pitch_elems) * 2};
+  cuuint32_t box[2] = {static_cast<cuuint32_t>(box_inner), static_cast<cuuint32_t>(box_outer)};
   cuuint32_t estr[2] = {1, 1};
   CUtensorMap m;
   CUresult r = e->encode_tiled(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(LEAF_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) rows=%ld cols=%ld", (int)r, rows, cols);
-  if (e->tmaps.size() > 4096) e->tmaps.clear();
-  e->tmaps[key] = m;
-  *out = m;
-  return LEAF_OK;
-}
-
-// operand stored [k_rows, mn_cols] row-major (MN-major): boxes of 64 MN elements (one 128-byte swizzle row) x 64 k
-static int make_tmap_mn(leaf_engine* e, const void* ptr, long k_rows, long mn_cols, long pitch, CUtensorMap* out) {
-  if (pitch <= 0) pitch = mn_cols;
-  auto key = std::make_tuple(ptr, k_rows, mn_cols, -static_cast<int>(pitch));
-  auto it = e->tmaps.find(key);
-  if (it != e->tmaps.end()) { *out = it->second; return LEAF_OK; }
-  if (mn_cols % 8 != 0 || pitch % 8 != 0) return fail(LEAF_ERR_INVALID, "MN-major operand width (%ld) and pitch (%ld) must be multiples of 8", mn_cols, pitch);
-  if (reinterpret_cast<uintptr_t>(ptr) & 15) return fail(LEAF_ERR_INVALID, "GEMM operand must be 16-byte aligned");
-  cuuint64_t dims[2] = {static_cast<cuuint64_t>(mn_cols), static_cast<cuuint64_t>(k_rows)};
-  cuuint64_t strides[1] = {static_cast<cuuint64_t>(pitch) * 2};
-  cuuint32_t box[2] = {64, 64};
-  cuuint32_t estr[2] = {1, 1};
-  CUtensorMap m;
-  CUresult r = e->encode_tiled(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(LEAF_ERR_CUDA, "cuTensorMapEncodeTiled (MN-major) failed (%d) rows=%ld cols=%ld", (int)r, k_rows, mn_cols);
+  if (r != CUDA_SUCCESS) return fail(LEAF_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) rows=%ld cols=%ld", (int)r, outer, inner);
   if (e->tmaps.size() > 4096) e->tmaps.clear();
   e->tmaps[key] = m;
   *out = m;
@@ -203,41 +186,90 @@ struct TimedSpan {
   }
 };
 
-// C[M,N] = A[M,K] . Bt[N,K]^T with the fused epilogue `epi`
-static int launch_gemm(leaf_engine* e, const __nv_bfloat16* A, long a_rows, const __nv_bfloat16* Bt, const float* bias,
-                       void* C, int ldc, int M, int N, int K, int epi, int act, const int* m_dev, cudaStream_t st,
-                       const __nv_bfloat16* delta = nullptr, int mn_major = 0, long a_pitch = 0, const float* res = nullptr,
-                       void* C2 = nullptr, bool allow_split_k = false) {
+// Launch configuration with programmatic dependent launch when e->pdl is on (the kernel must call pdl_wait() before its
+// first global access, gemm_sm100.cuh) and, for cluster > 1, clusters of that many CTAs along x. attr holds 2 entries.
+static cudaLaunchConfig_t launch_config(const leaf_engine* e, dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                        cudaLaunchAttribute* attr, unsigned cluster = 1) {
+  cudaLaunchConfig_t cfg{.gridDim = grid, .blockDim = block, .dynamicSmemBytes = smem, .stream = st, .attrs = attr, .numAttrs = 0};
+  if (cluster > 1) {
+    attr[cfg.numAttrs].id = cudaLaunchAttributeClusterDimension;
+    attr[cfg.numAttrs++].val.clusterDim = {cluster, 1, 1};
+  }
+  if (e->pdl) {
+    attr[cfg.numAttrs].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[cfg.numAttrs++].val.programmaticStreamSerializationAllowed = 1;
+  }
+  return cfg;
+}
+
+// A launch that may start while the previous kernel of the stream drains (programmatic dependent launch)
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(const leaf_engine* e, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
+  cudaLaunchAttribute attr[2];
+  const cudaLaunchConfig_t cfg = launch_config(e, grid, block, 0, st, attr);
+  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
+// The GEMM's template instance per epilogue, in EPI_* order (gemm_sm100.cuh)
+static void (*const gemm_kernels[])(CUtensorMap, CUtensorMap, GemmParams) = {
+    gemm2_bf16_tn_kernel<EPI_BF16>, gemm2_bf16_tn_kernel<EPI_BF16_ACT>, gemm2_bf16_tn_kernel<EPI_F32_RESIDUAL>,
+    gemm2_bf16_tn_kernel<EPI_F32>, gemm2_bf16_tn_kernel<EPI_F32_SPLITK>, gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD>,
+    gemm2_bf16_tn_kernel<EPI_F32_SPLITK_DET>, gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD_DET>};
+
+// The class a GEMM launch is timed in besides TC_GEMM
+static int gemm_timing_class(int epi, int N, int K) {
+  if (epi == EPI_F32_SPLITK || epi == EPI_F32_SPLITK_DET) return TC_EPI + EPI_F32_RESIDUAL;
+  if (epi == EPI_BF16_ACTBWD || epi == EPI_BF16_ACTBWD_DET) return TC_EPI + EPI_F32;
+  if (epi == EPI_F32_RESIDUAL && K > N) return TC_FC2;
+  if (epi == EPI_BF16 && K == N) return TC_OUT_PROJ;
+  return TC_EPI + epi;
+}
+
+// One product C[M,N] = A . B with a fused epilogue (gemm_sm100.cuh). Null pointers are absent operands.
+struct GemmOp {
+  const __nv_bfloat16* A = nullptr;   // [M,K], or [K,M] with GEMM_A_MN
+  long a_rows = 0;                    // K-major A only: rows of the allocation the TMA map covers (may exceed M)
+  long a_pitch = 0;                   // MN-major A only: row pitch when A is a column block of a wider matrix (0 = M)
+  const __nv_bfloat16* B = nullptr;   // [N,K], or [K,N] with GEMM_B_MN
+  int mn_major = 0;                   // GEMM_A_MN | GEMM_B_MN
+  void* C = nullptr;                  // [M,N], row pitch N
+  int M = 0;
+  const int* m_dev = nullptr;         // device row count that overrides M at run time
+  int N = 0, K = 0, epi = EPI_BF16, act = 0;
+  const float* bias = nullptr;
+  const __nv_bfloat16* delta = nullptr;   // GemmParams::delta
+  const float* res = nullptr;
+  void* C2 = nullptr;
+  bool split_k_ok = false;            // EPI_F32_RESIDUAL with no other operand: the contraction may be split over work units
+};
+
+static int launch_gemm(leaf_engine* e, const GemmOp& op, cudaStream_t st) {
+  const int M = op.M, N = op.N, K = op.K;
+  int epi = op.epi;
   if (M <= 0 || N <= 0 || K <= 0) return fail(LEAF_ERR_INVALID, "GEMM shape %dx%dx%d", M, N, K);
   if (N % 8 != 0) return fail(LEAF_ERR_INVALID, "GEMM N (%d) must be a multiple of 8", N);
+  if (epi < 0 || epi >= static_cast<int>(std::size(gemm_kernels))) return fail(LEAF_ERR_INVALID, "unknown epilogue %d", epi);
+  const bool a_mn = op.mn_major & GEMM_A_MN, b_mn = op.mn_major & GEMM_B_MN;
+  const long a_pitch = op.a_pitch > 0 ? op.a_pitch : M;
+  if ((!a_mn || !b_mn) && K % 8 != 0) return fail(LEAF_ERR_INVALID, "GEMM K (%d) must be a multiple of 8", K);
+  if (a_mn && M % 8 != 0) return fail(LEAF_ERR_INVALID, "MN-major GEMM M (%d) must be a multiple of 8", M);
+  if (a_mn && a_pitch % 8 != 0) return fail(LEAF_ERR_INVALID, "MN-major operand width (%d) and pitch (%ld) must be multiples of 8", M, a_pitch);
+  // A K-major operand [rows, K] is read in boxes of GEMM_BK k x up to 128 rows, an MN-major one [K, mn] in boxes of 64 mn
+  // elements (one 128-byte swizzle row) x 64 k, two per 128 rows of the tile
+  const int a_box = a_mn ? 128 : static_cast<int>(std::min(op.a_rows, 128L)), b_box = b_mn ? 128 : std::min(N, 128);
   CUtensorMap ta, tb;
-  int a_box = a_rows < 128 ? static_cast<int>(a_rows) : 128;
-  int b_box = N < 128 ? N : 128;
   int rc;
-  if (mn_major & GEMM_A_MN) {                  // A is [K, M] row-major
-    if (M % 8 != 0) return fail(LEAF_ERR_INVALID, "MN-major GEMM M (%d) must be a multiple of 8", M);
-    if ((rc = make_tmap_mn(e, A, K, M, a_pitch, &ta))) return rc;      // a_pitch: row pitch when A is a column block of a wider matrix
-    a_box = 128;
-  } else if ((rc = make_tmap(e, A, a_rows, K, a_box, &ta))) return rc;
-  if (mn_major & GEMM_B_MN) {                  // Bt is [K, N] row-major
-    if ((rc = make_tmap_mn(e, Bt, K, N, 0, &tb))) return rc;
-    b_box = 128;
-  } else if ((rc = make_tmap(e, Bt, N, K, b_box, &tb))) return rc;
-  GemmParams p;
-  p.mn_major = mn_major;
-  p.res = res;
-  p.C2 = C2;
-  p.split_k = 1;
-  p.ws = nullptr;
-  p.cnt = nullptr;
-  p.tx_bytes = static_cast<uint32_t>(a_box + b_box) * GEMM_BK * 2 * 2;       // both CTAs of the pair
-  p.M = M; p.m_dev = m_dev; p.N = N; p.K = K; p.bias = bias; p.C = C; p.ldc = ldc; p.act = act; p.delta = delta;
+  if ((rc = a_mn ? make_tmap(e, op.A, M, K, a_pitch, 64, 64, &ta) : make_tmap(e, op.A, K, op.a_rows, K, GEMM_BK, a_box, &ta))) return rc;
+  if ((rc = b_mn ? make_tmap(e, op.B, N, K, N, 64, 64, &tb) : make_tmap(e, op.B, K, N, K, GEMM_BK, b_box, &tb))) return rc;
+  GemmParams p{.M = M, .m_dev = op.m_dev, .N = N, .K = K, .bias = op.bias, .C = op.C, .delta = op.delta, .res = op.res, .ldc = N,
+               .act = op.act, .tx_bytes = static_cast<uint32_t>(a_box + b_box) * GEMM_BK * 2 * 2,    // both CTAs of the pair
+               .mn_major = op.mn_major, .C2 = op.C2, .split_k = 1};                                   // ws, cnt: null
   const int m_tiles = (M + GEMM2_BM - 1) / GEMM2_BM, n_tiles = (N + GEMM_BN - 1) / GEMM_BN;
   long tiles = static_cast<long>(m_tiles) * n_tiles;
   const int pairs_cap = ((e->gemm_sm_budget > 0 && e->gemm_sm_budget < e->sm_count) ? e->gemm_sm_budget : e->sm_count) / 2;
   // Deterministic mode: fc1's bias gradient and the split-K partial sums are added in a fixed order (gemm_sm100.cuh,
   // EPI_*_DET), and the split factor is chosen for the whole device, so that an SM budget cannot change the summation order.
-  const bool det = e->deterministic && ((epi == EPI_BF16_ACTBWD && C2) || allow_split_k);
+  const bool det = e->deterministic && ((epi == EPI_BF16_ACTBWD && op.C2) || op.split_k_ok);
   const int split_pairs = det ? e->sm_count / 2 : pairs_cap;
   if (det) {
     if (!e->tw.det_ws) return fail(LEAF_ERR_STATE, "deterministic mode without its workspace (leaf_train_reserve)");
@@ -249,7 +281,7 @@ static int launch_gemm(leaf_engine* e, const __nv_bfloat16* A, long a_rows, cons
       epi = EPI_BF16_ACTBWD_DET;
     }
   }
-  if (allow_split_k && epi == EPI_F32_RESIDUAL && !bias && !delta && !res && !m_dev && tiles < split_pairs) {
+  if (op.split_k_ok && epi == EPI_F32_RESIDUAL && !op.bias && !op.delta && !op.res && !op.m_dev && tiles < split_pairs) {
     // C += A.B with few output tiles and a long contraction (the weight gradients: 16-64 tiles, K = packed rows): divide the
     // k-blocks over several work units so that the launch fills the 74 CTA pairs; cost model = waves x (k-blocks per part +
     // 3 for the epilogue and the pipeline ramp). Partial sums are added with red.global.add.v4.f32.
@@ -268,32 +300,11 @@ static int launch_gemm(leaf_engine* e, const __nv_bfloat16* A, long a_rows, cons
     tiles *= p.split_k;
     if (p.split_k > 1) epi = det ? EPI_F32_SPLITK_DET : EPI_F32_SPLITK;
   }
-  TimedSpan span(e, (epi == EPI_F32_SPLITK || epi == EPI_F32_SPLITK_DET) ? 4 + EPI_F32_RESIDUAL :
-                    (epi == EPI_BF16_ACTBWD || epi == EPI_BF16_ACTBWD_DET) ? 4 + EPI_F32 : (epi == EPI_F32_RESIDUAL && K > N) ? 8 : (epi == EPI_BF16 && K == N) ? 9 : 4 + epi, st);
+  TimedSpan span(e, gemm_timing_class(epi, N, K), st);
   const int pairs = static_cast<int>(tiles < pairs_cap ? tiles : pairs_cap);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3(GEMM_THREADS);
-  cfg.dynamicSmemBytes = GEMM2_SMEM_BYTES;
-  cfg.stream = st;
   cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;      // see pdl_wait() in gemm_sm100.cuh
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = e->pdl ? 2 : 1;
-  switch (epi) {
-    case EPI_BF16: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_BF16>, ta, tb, p)); break;
-    case EPI_BF16_ACT: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_BF16_ACT>, ta, tb, p)); break;
-    case EPI_F32_RESIDUAL: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32_RESIDUAL>, ta, tb, p)); break;
-    case EPI_F32: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32>, ta, tb, p)); break;
-    case EPI_F32_SPLITK: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32_SPLITK>, ta, tb, p)); break;
-    case EPI_BF16_ACTBWD: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD>, ta, tb, p)); break;
-    case EPI_F32_SPLITK_DET: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_F32_SPLITK_DET>, ta, tb, p)); break;
-    case EPI_BF16_ACTBWD_DET: CK(cudaLaunchKernelEx(&cfg, gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD_DET>, ta, tb, p)); break;
-    default: return fail(LEAF_ERR_INVALID, "unknown epilogue %d", epi);
-  }
+  const cudaLaunchConfig_t cfg = launch_config(e, dim3(2 * pairs), dim3(GEMM_THREADS), GEMM2_SMEM_BYTES, st, attr, 2);
+  CK(cudaLaunchKernelEx(&cfg, gemm_kernels[epi], ta, tb, p));
   e->launches++;
   CK(cudaGetLastError());
   return LEAF_OK;
@@ -324,14 +335,7 @@ extern "C" int leaf_create(const leaf_cfg_t* cfg, leaf_handle_t* out) {
     return fail(LEAF_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
   }
   e->encode_tiled = reinterpret_cast<encode_tiled_fn>(fn);
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16_ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32_RESIDUAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32_SPLITK>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_F32_SPLITK_DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
-  CK(cudaFuncSetAttribute(gemm2_bf16_tn_kernel<EPI_BF16_ACTBWD_DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
+  for (auto kernel : gemm_kernels) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(embed_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LEAF_VOCAB * 4));
   CK(cudaFuncSetAttribute(topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   if (const char* pd = getenv("LEAF_PDL")) e->pdl = atoi(pd) != 0;
@@ -541,43 +545,31 @@ extern "C" int leaf_expand_tokenize(leaf_handle_t e, const uint8_t* caps, const 
   return LEAF_OK;
 }
 
-// A launch that may start while the previous kernel of the stream drains (programmatic dependent launch): the kernel
-// must call pdl_wait() before its first global access (gemm_sm100.cuh).
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(const leaf_engine* e, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = e->pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+// The LayerNorm kernels hold W / 128 values per lane as a template parameter: calls f(std::integral_constant<int, V>())
+// for V = W / 128 in 1..16 and returns what f returns
+template <int V = 1, typename F>
+static int with_width(int W, F&& f) {
+  if constexpr (V > 16) return fail(LEAF_ERR_INVALID, "unsupported width %d", W);
+  else return W / 128 == V ? f(std::integral_constant<int, V>()) : with_width<V + 1>(W, f);
 }
 
 static int launch_layernorm(leaf_engine* e, const float* x, const int* rows_dev, int rows_max, const int* gather,
                             const float* g, const float* b, __nv_bfloat16* y, cudaStream_t st,
                             const __nv_bfloat16* delta = nullptr, __nv_bfloat16* y_lo = nullptr) {
   const int W = e->cfg.width;
-  const int vpl = W / 128;
-  TimedSpan span(e, 1, st);
+  TimedSpan span(e, TC_LAYERNORM, st);
   long warps = rows_max;
   int blocks = static_cast<int>((warps + 7) / 8);
   const int cap = e->sm_count * 8;
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
-#define LN_CASE(V) case V: CK(launch_pdl(e, layernorm_bf16_kernel<V>, dim3(blocks), dim3(256), st, x, rows_dev, rows_max, gather, W, g, b, e->cfg.ln_eps, y, delta, y_lo)); break;
-  switch (vpl) {
-    LN_CASE(1) LN_CASE(2) LN_CASE(3) LN_CASE(4) LN_CASE(5) LN_CASE(6) LN_CASE(7) LN_CASE(8)
-    LN_CASE(9) LN_CASE(10) LN_CASE(11) LN_CASE(12) LN_CASE(13) LN_CASE(14) LN_CASE(15) LN_CASE(16)
-    default: return fail(LEAF_ERR_INVALID, "unsupported width %d", W);
-  }
-#undef LN_CASE
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return with_width(W, [&](auto V) -> int {
+    CK(launch_pdl(e, layernorm_bf16_kernel<V>, dim3(blocks), dim3(256), st, x, rows_dev, rows_max, gather, W, g, b, e->cfg.ln_eps, y,
+                  delta, y_lo));
+    e->launches++;
+    CK(cudaGetLastError());
+    return LEAF_OK;
+  });
 }
 
 // causal attention over the packed rows (tower_kernels.cuh)
@@ -604,7 +596,7 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
   int rc;
   const int* dup = nullptr;
   {
-  TimedSpan span(e, 3, st);
+  TimedSpan span(e, TC_PACK, st);
   if (dedup_group > 1 && dedup_rows > 0) {
     if (dedup_rows > N || dedup_rows % dedup_group != 0) return fail(LEAF_ERR_INVALID, "dedup_rows=%d dedup_group=%d N=%d", dedup_rows, dedup_group, N);
     dedup_kernel<<<(N + 7) / 8, 256, 0, st>>>(tok, len, dedup_rows, dedup_group, N, e->dup_of);
@@ -628,14 +620,15 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
     const leaf_layer_ptrs_t& p = e->layer_ptrs[l];
     const LayerW& w = e->lw[l];
     if ((rc = launch_layernorm(e, e->x, e->total_rows, rows_max, nullptr, p.ln1_w, p.ln1_b, e->h, st))) return rc;
-    if ((rc = launch_gemm(e, e->h, e->rows_cap, w.qkv_w, w.qkv_b, e->big, 3 * W, rows_max, 3 * W, W, EPI_BF16, 0, e->total_rows, st))) return rc;
+    if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.qkv_w, .C = e->big, .M = rows_max, .m_dev = e->total_rows,
+                              .N = 3 * W, .K = W, .epi = EPI_BF16, .bias = w.qkv_b}, st))) return rc;
     // Final layer: only the pooled EOS position of a sequence is read after it (transformer.py:661), so everything past
     // the key/value projection runs on ONE row per sequence: attention writes the EOS query's output to h[seq], the
     // residual rows are compacted into xc, and out-proj / LayerNorm / MLP see N rows instead of the packed row count.
     const bool last = e->prune_last && l == e->cfg.layers - 1;
     const __nv_bfloat16* dl = e->dlt;
     {
-      TimedSpan span(e, 2, st);
+      TimedSpan span(e, TC_ATTENTION, st);
       if ((rc = launch_attention(e, e->big, e->meta, N, e->h, last ? 1 : 0, st))) return rc;
     }
     // The attention branch's out-proj result stays OUT of the fp32 residual stream for now: it is stored as a bf16
@@ -646,20 +639,26 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
     // own autocast path produces; the fp32 stream itself is untouched.
     if (last) {
       {
-        TimedSpan span(e, 3, st);
+        TimedSpan span(e, TC_PACK, st);
         gather_rows_f32_kernel<<<(N + 7) / 8, 256, 0, st>>>(e->x, e->eos_row, N, W, e->xc);
         e->launches++;
       }
-      if ((rc = launch_gemm(e, e->h, e->rows_cap, w.out_w, p.out_b, e->dlt, W, N, W, W, EPI_BF16, 0, nullptr, st))) return rc;
+      if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.out_w, .C = e->dlt, .M = N, .N = W, .K = W, .epi = EPI_BF16,
+                                .bias = p.out_b}, st))) return rc;
       if ((rc = launch_layernorm(e, e->xc, nullptr, N, nullptr, p.ln2_w, p.ln2_b, e->h, st, dl))) return rc;
-      if ((rc = launch_gemm(e, e->h, e->rows_cap, w.fc1_w, p.fc1_b, e->big, 4 * W, N, 4 * W, W, EPI_BF16_ACT, e->cfg.activation, nullptr, st))) return rc;
-      if ((rc = launch_gemm(e, e->big, e->rows_cap, w.fc2_w, p.fc2_b, e->xc, W, N, W, 4 * W, EPI_F32_RESIDUAL, 0, nullptr, st, dl))) return rc;
+      if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.fc1_w, .C = e->big, .M = N, .N = 4 * W, .K = W,
+                                .epi = EPI_BF16_ACT, .act = e->cfg.activation, .bias = p.fc1_b}, st))) return rc;
+      if ((rc = launch_gemm(e, {.A = e->big, .a_rows = e->rows_cap, .B = w.fc2_w, .C = e->xc, .M = N, .N = W, .K = 4 * W,
+                                .epi = EPI_F32_RESIDUAL, .bias = p.fc2_b, .delta = dl}, st))) return rc;
       break;
     }
-    if ((rc = launch_gemm(e, e->h, e->rows_cap, w.out_w, p.out_b, e->dlt, W, rows_max, W, W, EPI_BF16, 0, e->total_rows, st))) return rc;
+    if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.out_w, .C = e->dlt, .M = rows_max, .m_dev = e->total_rows,
+                              .N = W, .K = W, .epi = EPI_BF16, .bias = p.out_b}, st))) return rc;
     if ((rc = launch_layernorm(e, e->x, e->total_rows, rows_max, nullptr, p.ln2_w, p.ln2_b, e->h, st, dl))) return rc;
-    if ((rc = launch_gemm(e, e->h, e->rows_cap, w.fc1_w, p.fc1_b, e->big, 4 * W, rows_max, 4 * W, W, EPI_BF16_ACT, e->cfg.activation, e->total_rows, st))) return rc;
-    if ((rc = launch_gemm(e, e->big, e->rows_cap, w.fc2_w, p.fc2_b, e->x, W, rows_max, W, 4 * W, EPI_F32_RESIDUAL, 0, e->total_rows, st, dl))) return rc;
+    if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.fc1_w, .C = e->big, .M = rows_max, .m_dev = e->total_rows,
+                              .N = 4 * W, .K = W, .epi = EPI_BF16_ACT, .act = e->cfg.activation, .bias = p.fc1_b}, st))) return rc;
+    if ((rc = launch_gemm(e, {.A = e->big, .a_rows = e->rows_cap, .B = w.fc2_w, .C = e->x, .M = rows_max, .m_dev = e->total_rows,
+                              .N = W, .K = 4 * W, .epi = EPI_F32_RESIDUAL, .bias = p.fc2_b, .delta = dl}, st))) return rc;
   }
   // ln_final and the projection in split precision: both operands carry what their bf16 rounding dropped as a second bf16
   // matrix (pooled = hi + lo, P = hi + lo; feat = hi.hi + lo.hi + hi.lo, fp32 accumulate: error 2^-17 instead of 2^-9). One row
@@ -668,9 +667,10 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
   if (e->prune_last) rc = launch_layernorm(e, e->xc, nullptr, N, e->first_of, e->wp.lnf_w, e->wp.lnf_b, e->pooled, st, nullptr, e->pooled_lo);
   else rc = launch_layernorm(e, e->x, nullptr, N, e->eos_row, e->wp.lnf_w, e->wp.lnf_b, e->pooled, st, nullptr, e->pooled_lo);
   if (rc) return rc;
-  if ((rc = launch_gemm(e, e->pooled, e->max_seqs + 128, e->proj_w, nullptr, feat_out, E, N, E, W, EPI_F32, 0, nullptr, st))) return rc;
-  if ((rc = launch_gemm(e, e->pooled_lo, e->max_seqs + 128, e->proj_w, nullptr, feat_out, E, N, E, W, EPI_F32_RESIDUAL, 0, nullptr, st))) return rc;
-  if ((rc = launch_gemm(e, e->pooled, e->max_seqs + 128, e->proj_w_lo, nullptr, feat_out, E, N, E, W, EPI_F32_RESIDUAL, 0, nullptr, st))) return rc;
+  const long pooled_rows = e->max_seqs + 128;
+  if ((rc = launch_gemm(e, {.A = e->pooled, .a_rows = pooled_rows, .B = e->proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32}, st))) return rc;
+  if ((rc = launch_gemm(e, {.A = e->pooled_lo, .a_rows = pooled_rows, .B = e->proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32_RESIDUAL}, st))) return rc;
+  if ((rc = launch_gemm(e, {.A = e->pooled, .a_rows = pooled_rows, .B = e->proj_w_lo, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32_RESIDUAL}, st))) return rc;
   if (normalize) {
     l2_normalize_kernel<<<(N + 7) / 8, 256, 0, st>>>(feat_out, N, E);
     e->launches++;
@@ -707,15 +707,19 @@ extern "C" int leaf_topk(leaf_handle_t e, const float* score_a, const float* sco
 extern "C" int leaf_gemm_bf16(leaf_handle_t e, const void* A, const void* Bt, const float* bias, void* C, int32_t M, int32_t N,
                               int32_t K, int32_t epilogue, int32_t act, const int32_t* m_dev, void* stream) {
   if (!e || !A || !Bt || !C) return fail(LEAF_ERR_INVALID, "null argument");
-  return launch_gemm(e, static_cast<const __nv_bfloat16*>(A), M, static_cast<const __nv_bfloat16*>(Bt), bias, C, N, M, N, K,
-                     epilogue, act, m_dev, static_cast<cudaStream_t>(stream));
+  if (epilogue < EPI_BF16 || epilogue > EPI_F32) return fail(LEAF_ERR_INVALID, "epilogue %d (0-3)", epilogue);
+  if (act != ACT_GELU_ERF && act != ACT_QUICK_GELU) return fail(LEAF_ERR_INVALID, "activation %d (0 erf GELU, 1 QuickGELU)", act);
+  return launch_gemm(e, {.A = static_cast<const __nv_bfloat16*>(A), .a_rows = M, .B = static_cast<const __nv_bfloat16*>(Bt), .C = C,
+                         .M = M, .m_dev = m_dev, .N = N, .K = K, .epi = epilogue, .act = act, .bias = bias}, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int leaf_gemm_bf16_mn(leaf_handle_t e, const void* A, const void* B, const float* bias, void* C, int32_t M, int32_t N,
                                  int32_t K, int32_t epilogue, int32_t a_mn, void* stream) {
   if (!e || !A || !B || !C) return fail(LEAF_ERR_INVALID, "null argument");
-  return launch_gemm(e, static_cast<const __nv_bfloat16*>(A), a_mn ? K : M, static_cast<const __nv_bfloat16*>(B), bias, C, N, M, N, K,
-                     epilogue, 0, nullptr, static_cast<cudaStream_t>(stream), nullptr, GEMM_B_MN | (a_mn ? GEMM_A_MN : 0));
+  if (epilogue < EPI_BF16 || epilogue > EPI_F32) return fail(LEAF_ERR_INVALID, "epilogue %d (0-3)", epilogue);
+  return launch_gemm(e, {.A = static_cast<const __nv_bfloat16*>(A), .a_rows = M, .B = static_cast<const __nv_bfloat16*>(B),
+                         .mn_major = GEMM_B_MN | (a_mn ? GEMM_A_MN : 0), .C = C, .M = M, .N = N, .K = K, .epi = epilogue, .bias = bias},
+                     static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int leaf_test_layernorm(leaf_handle_t e, const float* x, int32_t rows, const float* gamma, const float* beta, void* y,
@@ -768,21 +772,21 @@ extern "C" int leaf_set_timing(leaf_handle_t e, int32_t on) {
   if (e->timing) {                               // a new measurement starts from zero
     int32_t dummy;
     leaf_timing_ms(e, 0, &dummy);
-    for (int i = 0; i < 10; ++i) { e->span_ms[i] = 0; e->span_n[i] = 0; }
+    for (int i = 0; i < TC_COUNT; ++i) { e->span_ms[i] = 0; e->span_n[i] = 0; }
   }
   return LEAF_OK;
 }
 
 extern "C" double leaf_timing_ms(leaf_handle_t e, int32_t which, int32_t* launches) {
-  if (!e || which < 0 || which > 9) return 0.0;
+  if (!e || which < 0 || which >= TC_COUNT) return 0.0;
   if (!e->spans.empty()) {                       // fold the recorded spans into the per-category totals
     for (auto& sp : e->spans) {
       cudaEventSynchronize(sp.b);
       float ms = 0.f;
       if (cudaEventElapsedTime(&ms, sp.a, sp.b) == cudaSuccess) {
         e->span_ms[sp.cat] += ms; e->span_n[sp.cat]++;
-        if (sp.cat >= 4) { e->span_ms[0] += ms; e->span_n[0]++; }
-        if (sp.cat == 8) { e->span_ms[4 + EPI_F32_RESIDUAL] += ms; e->span_n[4 + EPI_F32_RESIDUAL]++; }
+        if (sp.cat >= TC_EPI) { e->span_ms[TC_GEMM] += ms; e->span_n[TC_GEMM]++; }
+        if (sp.cat == TC_FC2) { e->span_ms[TC_EPI + EPI_F32_RESIDUAL] += ms; e->span_n[TC_EPI + EPI_F32_RESIDUAL]++; }
       }
       e->event_pool.push_back(sp.a);
       e->event_pool.push_back(sp.b);
@@ -929,17 +933,20 @@ extern "C" int leaf_forward_train(leaf_handle_t e, const int32_t* tok, const int
     TrainLayer& a = t.L[l];
     float* x_next = (l + 1 < e->cfg.layers) ? t.L[l + 1].x_in : t.x_out;
     if ((rc = launch_layernorm(e, a.x_in, nullptr, M, nullptr, p.ln1_w, p.ln1_b, a.h1, st))) return rc;
-    if ((rc = launch_gemm(e, a.h1, t.rows_cap, w.qkv_w, w.qkv_b, a.qkv, 3 * W, M, 3 * W, W, EPI_BF16, 0, nullptr, st))) return rc;
+    if ((rc = launch_gemm(e, {.A = a.h1, .a_rows = t.rows_cap, .B = w.qkv_w, .C = a.qkv, .M = M, .N = 3 * W, .K = W, .epi = EPI_BF16,
+                              .bias = w.qkv_b}, st))) return rc;
     if ((rc = launch_attention(e, a.qkv, t.meta, N, a.o, 0, st))) return rc;
-    if ((rc = launch_gemm(e, a.o, t.rows_cap, w.out_w, p.out_b, a.x_mid, W, M, W, W, EPI_F32_RESIDUAL, 0, nullptr, st, nullptr, 0, 0, a.x_in))) return rc;
+    if ((rc = launch_gemm(e, {.A = a.o, .a_rows = t.rows_cap, .B = w.out_w, .C = a.x_mid, .M = M, .N = W, .K = W, .epi = EPI_F32_RESIDUAL,
+                              .bias = p.out_b, .res = a.x_in}, st))) return rc;
     if ((rc = launch_layernorm(e, a.x_mid, nullptr, M, nullptr, p.ln2_w, p.ln2_b, a.h2, st))) return rc;
     // one epilogue stores fc1's output twice: the pre-activation u (kept for act'(u) in the backward) and act(u)
-    if ((rc = launch_gemm(e, a.h2, t.rows_cap, w.fc1_w, p.fc1_b, a.g, 4 * W, M, 4 * W, W, EPI_BF16_ACT, e->cfg.activation, nullptr, st,
-                          nullptr, 0, 0, nullptr, a.u))) return rc;
-    if ((rc = launch_gemm(e, a.g, t.rows_cap, w.fc2_w, p.fc2_b, x_next, W, M, W, 4 * W, EPI_F32_RESIDUAL, 0, nullptr, st, nullptr, 0, 0, a.x_mid))) return rc;
+    if ((rc = launch_gemm(e, {.A = a.h2, .a_rows = t.rows_cap, .B = w.fc1_w, .C = a.g, .M = M, .N = 4 * W, .K = W, .epi = EPI_BF16_ACT,
+                              .act = e->cfg.activation, .bias = p.fc1_b, .C2 = a.u}, st))) return rc;
+    if ((rc = launch_gemm(e, {.A = a.g, .a_rows = t.rows_cap, .B = w.fc2_w, .C = x_next, .M = M, .N = W, .K = 4 * W, .epi = EPI_F32_RESIDUAL,
+                              .bias = p.fc2_b, .res = a.x_mid}, st))) return rc;
   }
   if ((rc = launch_layernorm(e, t.x_out, nullptr, N, t.eos_row, e->wp.lnf_w, e->wp.lnf_b, t.pooled, st))) return rc;
-  if ((rc = launch_gemm(e, t.pooled, t.max_seqs + 128, e->proj_w, nullptr, feat_out, E, N, E, W, EPI_F32, 0, nullptr, st))) return rc;
+  if ((rc = launch_gemm(e, {.A = t.pooled, .a_rows = t.max_seqs + 128, .B = e->proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32}, st))) return rc;
   CK(cudaGetLastError());
   t.have_forward = true;
   if (generation_out) *generation_out = t.generation;
@@ -958,26 +965,20 @@ static int launch_layernorm_bwd(leaf_engine* e, const float* dy, const float* x,
   int blocks = (rows + 7) / 8;
   if (blocks > 2 * e->sm_count) blocks = 2 * e->sm_count;
   if (blocks < 1) blocks = 1;
-#define LNB_CASE(V) case V: layernorm_bwd_rows_kernel<V><<<blocks, 256, 0, st>>>(dy, x, gather, rows, W, gamma, e->cfg.ln_eps, dx, accumulate, dx16, stats); break;
-  switch (W / 128) {
-    LNB_CASE(1) LNB_CASE(2) LNB_CASE(3) LNB_CASE(4) LNB_CASE(5) LNB_CASE(6) LNB_CASE(7) LNB_CASE(8)
-    LNB_CASE(9) LNB_CASE(10) LNB_CASE(11) LNB_CASE(12) LNB_CASE(13) LNB_CASE(14) LNB_CASE(15) LNB_CASE(16)
-    default: return fail(LEAF_ERR_INVALID, "unsupported width %d", W);
-  }
-#undef LNB_CASE
+  int rc = with_width(W, [&](auto V) -> int {
+    layernorm_bwd_rows_kernel<V><<<blocks, 256, 0, st>>>(dy, x, gather, rows, W, gamma, e->cfg.ln_eps, dx, accumulate, dx16, stats);
+    return LEAF_OK;
+  });
+  if (rc) return rc;
   const int cbx = (W + 255) / 256;
   int bands = (2 * e->sm_count + cbx - 1) / cbx;
   if (bands > (rows + 7) / 8) bands = (rows + 7) / 8;
   if (bands < 1) bands = 1;
-  if (e->deterministic) {                              // band sums added in band order (train_kernels.cuh)
-    if (static_cast<size_t>(bands) * 3 * W > e->tw.det_ws_floats || static_cast<size_t>(cbx) > e->tw.det_cnt_ints)
-      return fail(LEAF_ERR_STATE, "deterministic workspace too small for the LayerNorm backward (%d bands)", bands);
-    CK(launch_pdl(e, layernorm_bwd_cols_kernel<true>, dim3(cbx, bands), dim3(256), st, dy, x, gather, stats, dx, rows, W, dgamma, dbeta,
-                  dxsum, e->tw.det_ws, e->tw.det_cnt));
-  } else {
-    CK(launch_pdl(e, layernorm_bwd_cols_kernel<false>, dim3(cbx, bands), dim3(256), st, dy, x, gather, stats, dx, rows, W, dgamma, dbeta,
-                  dxsum, nullptr, nullptr));
-  }
+  const bool det = e->deterministic;                  // band sums added in band order (train_kernels.cuh)
+  if (det && (static_cast<size_t>(bands) * 3 * W > e->tw.det_ws_floats || static_cast<size_t>(cbx) > e->tw.det_cnt_ints))
+    return fail(LEAF_ERR_STATE, "deterministic workspace too small for the LayerNorm backward (%d bands)", bands);
+  CK(launch_pdl(e, det ? layernorm_bwd_cols_kernel<true> : layernorm_bwd_cols_kernel<false>, dim3(cbx, bands), dim3(256), st, dy, x,
+                gather, stats, dx, rows, W, dgamma, dbeta, dxsum, det ? e->tw.det_ws : nullptr, det ? e->tw.det_cnt : nullptr));
   e->launches += 2;
   CK(cudaGetLastError());
   return LEAF_OK;
@@ -1005,23 +1006,22 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
   // forward's bf16 weight copy W[out,in] as B[k = out][n = in], the weight gradients take dY[rows,out] and X[rows,in] as
   // A[k = rows][m = out] and B[k = rows][n = in]. No transposed copies of weights or activations exist.
   auto dgrad = [&](const __nv_bfloat16* dy, long dy_rows, const __nv_bfloat16* w_oi, float* dx_out, int rows, int in, int out) {
-    return launch_gemm(e, dy, dy_rows, w_oi, nullptr, dx_out, in, rows, in, out, EPI_F32, 0, nullptr, st, nullptr, GEMM_B_MN);
+    return launch_gemm(e, {.A = dy, .a_rows = dy_rows, .B = w_oi, .mn_major = GEMM_B_MN, .C = dx_out, .M = rows, .N = in, .K = out, .epi = EPI_F32}, st);
   };
   auto wgrad = [&](const __nv_bfloat16* dy, long dy_pitch, const __nv_bfloat16* x, float* dw, int rows, int in, int out) {
-    return launch_gemm(e, dy, rows, x, nullptr, dw, in, out, in, rows, EPI_F32_RESIDUAL, 0, nullptr, st, nullptr,
-                       GEMM_A_MN | GEMM_B_MN, dy_pitch, nullptr, nullptr, /*allow_split_k=*/true);
+    return launch_gemm(e, {.A = dy, .a_pitch = dy_pitch, .B = x, .mn_major = GEMM_A_MN | GEMM_B_MN, .C = dw, .M = out, .N = in, .K = rows,
+                           .epi = EPI_F32_RESIDUAL, .split_k_ok = true}, st);
   };
   // ---- projection + ln_final on the pooled rows ----
   const size_t nfe = static_cast<size_t>(N) * E;
   cast_f32_bf16_kernel<<<launch_ew(e, nfe), 256, 0, st>>>(dfeat, t.d16, nfe);
   e->launches++;
   if ((rc = dgrad(t.d16, N, e->proj_w, t.dtmp, N, W, E))) return rc;                                        // dpooled [N,W] = dfeat . P[E,W]
-  if (grads->text_projection) {
-    if (grads->projection_is_ew) {
-      if ((rc = wgrad(t.d16, 0, t.pooled, F(grads->text_projection), N, W, E))) return rc;                 // dP[E,W] += dfeat^T . pooled
-    } else if ((rc = launch_gemm(e, t.pooled, N, t.d16, nullptr, F(grads->text_projection), E, W, E, N, EPI_F32_RESIDUAL, 0, nullptr, st,
-                                 nullptr, GEMM_A_MN | GEMM_B_MN))) return rc;                              // dP[W,E] += pooled^T . dfeat
-  }
+  const GemmOp dp_ew = {.A = t.d16, .B = t.pooled, .mn_major = GEMM_A_MN | GEMM_B_MN, .C = F(grads->text_projection), .M = E, .N = W,
+                        .K = N, .epi = EPI_F32_RESIDUAL, .split_k_ok = true};                               // dP[E,W] += dfeat^T . pooled
+  const GemmOp dp_we = {.A = t.pooled, .B = t.d16, .mn_major = GEMM_A_MN | GEMM_B_MN, .C = F(grads->text_projection), .M = W, .N = E,
+                        .K = N, .epi = EPI_F32_RESIDUAL};                                                    // dP[W,E] += pooled^T . dfeat
+  if (grads->text_projection && (rc = launch_gemm(e, grads->projection_is_ew ? dp_ew : dp_we, st))) return rc;
   // dx and its bf16 copy dx16 (the A operand of the next dgrad GEMM) are written together by the LayerNorm backward
   CK(cudaMemsetAsync(t.dx, 0, static_cast<size_t>(M) * W * 4, st));
   CK(cudaMemsetAsync(t.dx16, 0, static_cast<size_t>(M) * W * 2, st));
@@ -1039,8 +1039,8 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
     // ================= MLP branch: x_next = x_mid + fc2(act(fc1(ln_2(x_mid)))) =================
     // du [M,4W] = (dx . W2[W,4W]) * act'(u), bf16, with fc1's bias gradient (its column sums): one GEMM, the activation
     // backward is its epilogue (EPI_BF16_ACTBWD; a separate pass over an fp32 dg [M,4W] before)
-    if ((rc = launch_gemm(e, t.dx16, cap, w.fc2_w, nullptr, t.d16, 4 * W, M, 4 * W, W, EPI_BF16_ACTBWD, e->cfg.activation, nullptr, st,
-                          a.u, GEMM_B_MN, 0, nullptr, F(g.fc1_b)))) return rc;
+    if ((rc = launch_gemm(e, {.A = t.dx16, .a_rows = cap, .B = w.fc2_w, .mn_major = GEMM_B_MN, .C = t.d16, .M = M, .N = 4 * W, .K = W,
+                              .epi = EPI_BF16_ACTBWD, .act = e->cfg.activation, .delta = a.u, .C2 = F(g.fc1_b)}, st))) return rc;
     if (g.fc2_w && (rc = wgrad(t.dx16, 0, a.g, F(g.fc2_w), M, 4 * W, W))) return rc;
     if ((rc = dgrad(t.d16, cap, w.fc1_w, t.dtmp, M, W, 4 * W))) return rc;                                  // dh2 [M,W]
     if (g.fc1_w && (rc = wgrad(t.d16, 0, a.h2, F(g.fc1_w), M, W, 4 * W))) return rc;
@@ -1052,12 +1052,10 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
       float* bq = p.in_proj_w ? F(g.in_proj_b) : F(g.q_b);
       float* bk = p.in_proj_w ? (g.in_proj_b ? F(g.in_proj_b) + W : nullptr) : F(g.k_b);
       float* bv = p.in_proj_w ? (g.in_proj_b ? F(g.in_proj_b) + 2 * W : nullptr) : F(g.v_b);
-      if (e->deterministic && (bq || bk || bv))         // bias column sums added in (sequence, warp) order
-        attention_bwd_kernel<true><<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16,
-                                                                                                      bq, bk, bv, t.det_ws, t.det_cnt);
-      else
-        attention_bwd_kernel<false><<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16,
-                                                                                                       bq, bk, bv);
+      const bool det = e->deterministic && (bq || bk || bv);   // bias column sums added in (sequence, warp) order
+      auto attention_bwd = det ? attention_bwd_kernel<true> : attention_bwd_kernel<false>;
+      attention_bwd<<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16, bq, bk, bv,
+                                                                                            det ? t.det_ws : nullptr, det ? t.det_cnt : nullptr);
     }
     e->launches++;
     CK(cudaGetLastError());

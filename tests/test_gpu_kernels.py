@@ -87,6 +87,30 @@ def test_gemm_duplicate_rows_bitwise_equal(eng):
     assert torch.equal(C, C[0:1].expand_as(C))
 
 
+def test_gemm_hook_rejects_internal_epilogues(eng):
+    """The GEMM hooks take epilogues 0-3 and activations 0-1 (leaf_b200.h). The engine's internal epilogues 4-7 read operands
+    these entry points never set (the activation backward's U, the deterministic workspaces), so the hooks refuse them, and
+    unknown activation codes, before anything is launched."""
+    from leaf_b200 import LeafError
+    g = torch.Generator(device="cuda").manual_seed(11)
+    A = torch.randn((128, 256), generator=g, device="cuda").to(torch.bfloat16)
+    Bt = (torch.randn((256, 256), generator=g, device="cuda") / 16).to(torch.bfloat16)
+    C = torch.zeros((128, 256), device="cuda")
+    launches = eng.launch_count()
+    for epi in range(4, 8):
+        with pytest.raises(LeafError, match="epilogue"):
+            eng.gemm(A, Bt, None, epilogue=epi, C=C)
+    with pytest.raises(LeafError, match="epilogue"):
+        eng.gemm_mn(A, Bt[:128], None, epilogue=5, C=torch.zeros((256, 256), device="cuda"))
+    with pytest.raises(LeafError, match="activation"):
+        eng.gemm(A, Bt, None, epilogue=1, act=2)
+    assert eng.launch_count() == launches
+    assert torch.equal(C, torch.zeros_like(C))
+    ref = A.float() @ Bt.float().T                                            # the engine is still usable
+    eng.gemm(A, Bt, None, epilogue=3, C=C)
+    assert torch.allclose(C, ref, atol=2e-3, rtol=1e-3), (C - ref).abs().max().item()
+
+
 def test_layernorm(eng):
     g = torch.Generator(device="cuda").manual_seed(1)
     W = eng.width

@@ -1,10 +1,10 @@
 """Timing of the tower's tcgen05 GEMM alone at the bench workload's shapes, per epilogue (one box, interleaved A/B).
 
-    python tools/ab_gemm.py [--rows 130000] [--acts 0 2]
+    python tools/ab_gemm.py [--rows 130000] [--acts 0]
 
 Runs the four Linear layers of one ViT-H block (QKV, out-proj + residual, fc1 + activation, fc2 + residual) through
 leaf_gemm_bf16 on random bf16 operands with M packed rows, alternating the activation codes given in --acts for the fc1
-epilogue (0 = two-MUFU erf GELU, 2 = one-MUFU form, 1 = QuickGELU) so that clock drift hits all of them alike. Prints
+epilogue (0 = erf GELU, 1 = QuickGELU) so that clock drift hits all of them alike. Prints
 microseconds per launch and TFLOP/s; the operands (> 1 GB per launch) are far larger than L2, so no flush is needed.
 """
 import argparse
@@ -21,7 +21,7 @@ from leaf_b200.tower import LeafTextTower                    # noqa: E402
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rows", type=int, default=130000)
-    ap.add_argument("--acts", type=int, nargs="+", default=[0, 2])
+    ap.add_argument("--acts", type=int, nargs="+", default=[0])
     ap.add_argument("--reps", type=int, default=6)
     a = ap.parse_args()
     dev = torch.device("cuda", 0)
