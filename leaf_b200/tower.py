@@ -48,18 +48,21 @@ class _EncodeTextTrain(torch.autograd.Function):
         return (None, None) + (None,) * len(grads)
 
 
-_TEXT_KEYS = re.compile(r"^(text\.)?(token_embedding\.weight|positional_embedding|ln_final\.(weight|bias)|text_projection(\.weight)?|"
+_TEXT_KEYS = re.compile(r"^(?:module\.)?(?:text\.)?(?P<key>token_embedding\.weight|positional_embedding|ln_final\.(weight|bias)|"
+                        r"text_projection(\.weight)?|"
                         r"transformer\.resblocks\.\d+\.(ln_1|ln_2|attn\.out_proj|mlp\.c_fc|mlp\.c_proj)\.(weight|bias)|"
                         r"transformer\.resblocks\.\d+\.attn\.in_proj_(weight|bias))$")
 
 
 def text_tower_state_dict(state_dict: dict) -> dict:
     """The text-tower entries of an open_clip CLIP / CustomTextCLIP state dict (SURVEY.md appendix C): everything under
-    `visual.`, `logit_scale`, the attention-mask buffer etc. is dropped; a `text.` prefix is removed."""
+    `visual.`, `logit_scale`, the attention-mask buffer etc. is dropped; a `text.` prefix, and the `module.` prefix of a
+    state dict saved through DDP, are removed."""
     out = {}
     for k, v in state_dict.items():
-        if _TEXT_KEYS.match(k):
-            out[k[5:] if k.startswith("text.") else k] = v
+        m = _TEXT_KEYS.match(k)
+        if m:
+            out[m["key"]] = v
     return out
 
 
@@ -189,6 +192,34 @@ class LeafTextTower(torch.nn.Module):
 
     def open_clip_state_dict(self) -> dict:
         return {k: getattr(self, safe).data for k, safe in self._names.items()}
+
+    def load_open_clip_state_dict(self, state_dict: dict):
+        """The inverse of open_clip_state_dict(): copies the text-tower entries of `state_dict` (any key form
+        text_tower_state_dict accepts: a whole CLIP state dict, a `text.` or a DDP `module.` prefix) IN PLACE into the flat
+        buffer, so the .grad views and a FareTrainer's references stay valid, then re-casts the engine's operand copies.
+        Names and shapes are checked before anything is copied: ValueError lists the missing, unexpected and mis-shaped keys."""
+        sd = text_tower_state_dict(state_dict)
+        bad = [f"missing: {k}" for k in self._slices if k not in sd]
+        bad += [f"unexpected: {k}" for k in sd if k not in self._slices]
+        bad += [f"shape of {k}: {tuple(v.shape)}, this tower has {self._slices[k][2]}" for k, v in sd.items()
+                if k in self._slices and tuple(v.shape) != self._slices[k][2]]
+        if bad:
+            raise ValueError("state dict does not fit this LeafTextTower: " + "; ".join(bad))
+        with torch.no_grad():
+            for k, (off, n, shape) in self._slices.items():
+                self._flat[off:off + n].view(shape).copy_(sd[k])
+        self.refresh()
+
+    def load_state_dict(self, state_dict, strict: bool = True, assign: bool = False):
+        """nn.Module.load_state_dict (this module's own parameter names), followed by refresh(): without it the engine would
+        keep computing with its operand copies of the old weights. assign=True would replace the parameters, which are
+        views of the flat buffer the engine and the optimizer read, and is refused."""
+        if assign:
+            raise ValueError("LeafTextTower parameters are views of one flat buffer: load_state_dict(assign=True) would detach them")
+        try:
+            return super().load_state_dict(state_dict, strict=strict)
+        finally:                                  # torch copies every entry that fits before it raises on the others
+            self.refresh()
 
     @property
     def flat_params(self) -> torch.Tensor:
