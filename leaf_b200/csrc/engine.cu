@@ -11,9 +11,11 @@
 
 #include <algorithm>
 #include <map>
+#include <memory>
 #include <string>
 #include <tuple>
 #include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/leaf_b200.h"
@@ -53,10 +55,74 @@ typedef CUresult (*encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_
 // Classes of leaf_timing_ms, numbered as include/leaf_b200.h documents them (public ABI)
 enum TimingClass { TC_GEMM = 0, TC_LAYERNORM = 1, TC_ATTENTION = 2, TC_PACK = 3, TC_EPI = 4, TC_FC2 = 8, TC_OUT_PROJ = 9, TC_COUNT = 10 };
 
+// Owner of device allocations that share one lifetime. Assigning a fresh owner (or a struct that holds one) frees what the
+// old one allocated.
+class DevMem {
+ public:
+  DevMem() = default;
+  DevMem& operator=(DevMem&& o) noexcept { std::swap(ptrs_, o.ptrs_); return *this; }   // o, a temporary, frees ours
+  ~DevMem() { release(); }
+  template <typename Tp>
+  int alloc(Tp** p, size_t count) {
+    void* d = nullptr;
+    CK(cudaMalloc(&d, count * sizeof(Tp)));
+    ptrs_.push_back(d);
+    *p = static_cast<Tp*>(d);
+    return LEAF_OK;
+  }
+  void release() {
+    for (void* p : ptrs_) cudaFree(p);
+    ptrs_.clear();
+  }
+
+ private:
+  std::vector<void*> ptrs_;
+};
+
+// What prefix_kernel, scan_lengths_kernel and meta_kernel write for up to max_seqs sequences (tower_kernels.cuh):
+// total_rows = {packed rows, longest sequence}
+struct PackBufs {
+  int *cu = nullptr, *eos_row = nullptr, *total_rows = nullptr, *pfx = nullptr, *own_len = nullptr;
+  int4* meta = nullptr;
+};
+
+static int alloc_pack(DevMem& m, PackBufs& p, size_t max_seqs) {
+  int rc;
+  if ((rc = m.alloc(&p.cu, max_seqs + 1))) return rc;
+  if ((rc = m.alloc(&p.eos_row, max_seqs))) return rc;
+  if ((rc = m.alloc(&p.total_rows, 2))) return rc;
+  if ((rc = m.alloc(&p.pfx, max_seqs))) return rc;
+  if ((rc = m.alloc(&p.own_len, max_seqs))) return rc;
+  return m.alloc(&p.meta, max_seqs);
+}
+
 struct LayerW {
   __nv_bfloat16 *qkv_w = nullptr, *out_w = nullptr, *fc1_w = nullptr, *fc2_w = nullptr;   // engine-owned bf16 copies
   float* qkv_b_own = nullptr;                                                              // HF layout only
   const float* qkv_b = nullptr;
+};
+
+struct Weights {                      // bf16 operand copies of the bound parameters (leaf_bind_weights)
+  DevMem mem;
+  std::vector<LayerW> lw;
+  __nv_bfloat16* proj_w = nullptr;    // [E, W] bf16
+  __nv_bfloat16* proj_w_lo = nullptr; // [E, W] what proj_w's rounding dropped (split-precision final projection of leaf_encode)
+};
+
+struct Workspace {                    // of leaf_encode, sized by leaf_reserve
+  DevMem mem;
+  int max_seqs = 0;
+  long rows_cap = 0;
+  float* x = nullptr;                 // [rows_cap, W] fp32 residual stream
+  __nv_bfloat16* h = nullptr;         // [rows_cap, W]  LN output / attention output
+  __nv_bfloat16* big = nullptr;       // [rows_cap, 4W] qkv (3W) or MLP hidden (4W)
+  __nv_bfloat16* dlt = nullptr;       // [rows_cap, W]  out-proj result of the current layer (added to x by fc2's epilogue)
+  __nv_bfloat16* pooled = nullptr;    // [max_seqs, W]
+  __nv_bfloat16* pooled_lo = nullptr; // [max_seqs, W] what pooled's rounding dropped (split-precision final projection)
+  float* xc = nullptr;                // [max_seqs, W] fp32 residual rows of the pooled positions (final layer, compact)
+  int* first_of = nullptr;            // [max_seqs] sequence whose rows stand for sequence i
+  int *dup_of = nullptr, *need = nullptr;
+  PackBufs pack;
 };
 
 struct TrainLayer {        // activations one layer keeps for the backward pass (K4)
@@ -64,7 +130,8 @@ struct TrainLayer {        // activations one layer keeps for the backward pass 
   __nv_bfloat16 *h1 = nullptr, *qkv = nullptr, *o = nullptr, *h2 = nullptr, *u = nullptr, *g = nullptr;
 };
 
-struct TrainWs {
+struct TrainWs {                      // of leaf_forward_train / leaf_backward, sized by leaf_train_reserve
+  DevMem mem;
   int max_seqs = 0;
   long rows_cap = 0;
   int N = 0, M = 0, T = 0;            // sequences / packed rows / longest sequence of the saved forward
@@ -80,9 +147,8 @@ struct TrainWs {
   int* det_cnt = nullptr;
   int* det_idx = nullptr;
   size_t det_ws_floats = 0, det_cnt_ints = 0;
-  int *tok = nullptr, *cu = nullptr, *eos_row = nullptr, *total_rows = nullptr, *pfx = nullptr, *own_len = nullptr;
-  int4* meta = nullptr;
-  std::vector<void*> allocs;
+  int* tok = nullptr;
+  PackBufs pack;
 };
 
 struct leaf_engine {
@@ -94,43 +160,30 @@ struct leaf_engine {
   bool bpe_loaded = false;
   bool hf_tokenizer = false;          // leaf_set_tokenizer_mode
   int max_caption_bytes = LEAF_MAX_CAPTION_BYTES;   // leaf_set_max_caption_bytes
-  std::vector<void*> table_allocs;
+  DevMem mem;                         // for the engine's lifetime: the K1 and --constrain tables, det_sum_*
   K1Tables tables{};
   // --constrain filter: hash sets of the word list and of Punkt abbreviation types
   CnTables cn{};
   bool words_loaded = false;
+  DevMem cn_mem;                      // cn_count, grown by leaf_constrain_mask
   int32_t* cn_count = nullptr;
   int cn_count_cap = 0;
   // weights
   bool bound = false;
   leaf_weight_ptrs_t wp{};
   std::vector<leaf_layer_ptrs_t> layer_ptrs;
-  std::vector<LayerW> lw;
-  __nv_bfloat16* proj_w = nullptr;    // [E, W] bf16
-  __nv_bfloat16* proj_w_lo = nullptr; // [E, W] what proj_w's rounding dropped (split-precision final projection of leaf_encode)
-  __nv_bfloat16* pooled_lo = nullptr; // [max_seqs, W] likewise for the ln_final output
+  Weights wts;
   TrainWs tw;
   int64_t train_generation = 0;
   leaf_backward_hook_t bwd_hook = nullptr;   // host callback after each layer's gradients are enqueued (leaf_set_backward_hook)
   void* bwd_hook_user = nullptr;
-  // workspace
-  int max_seqs = 0;
-  long rows_cap = 0;
-  float* x = nullptr;                 // [rows_cap, W] fp32 residual stream
-  __nv_bfloat16* h = nullptr;         // [rows_cap, W]  LN output / attention output
-  __nv_bfloat16* big = nullptr;       // [rows_cap, 4W] qkv (3W) or MLP hidden (4W)
-  __nv_bfloat16* dlt = nullptr;       // [rows_cap, W]  out-proj result of the current layer (added to x by fc2's epilogue)
-  __nv_bfloat16* pooled = nullptr;    // [max_seqs, W]
-  float* xc = nullptr;                // [max_seqs, W] fp32 residual rows of the pooled positions (final layer, compact)
-  int* first_of = nullptr;            // [max_seqs] sequence whose rows stand for sequence i
+  Workspace ws;
   bool prune_last = true;             // final layer: out-proj + MLP on the pooled rows only
   int gemm_sm_budget = 0;             // > 0: the persistent GEMM grids use at most this many SMs (leaf_set_sm_budget)
   int pdl = 1;                        // launch the per-layer chain with programmatic dependent launch (LEAF_PDL=0 turns it off)
   bool deterministic = false;         // leaf_set_deterministic: fixed-order reductions in leaf_backward / leaf_sumsq
   float* det_sum_ws = nullptr;        // leaf_sumsq's per-block sums and arrival counter in deterministic mode
   int* det_sum_cnt = nullptr;
-  int *cu = nullptr, *eos_row = nullptr, *total_rows = nullptr, *pfx = nullptr, *own_len = nullptr, *dup_of = nullptr, *need = nullptr;
-  int4* meta = nullptr;
   // bookkeeping
   int64_t launches = 0;
   bool timing = false;
@@ -140,7 +193,19 @@ struct leaf_engine {
   int span_n[TC_COUNT] = {0};
   std::vector<cudaEvent_t> event_pool;
   std::map<std::tuple<const void*, long, long, long, int, int>, CUtensorMap> tmaps;   // make_tmap's arguments
+
+  ~leaf_engine() {                    // device memory goes with the DevMem members
+    for (auto& sp : spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
+    for (auto ev : event_pool) cudaEventDestroy(ev);
+  }
 };
+
+// Frees the weights or a workspace: assigns a fresh owner. Tensor maps are cached by address, so the cache goes with them.
+template <typename Owner>
+static void reset(leaf_engine* e, Owner& o) {
+  o = Owner();
+  e->tmaps.clear();
+}
 
 extern "C" const char* leaf_last_error(void) { return g_err.c_str(); }
 extern "C" const char* leaf_version(void) { return "leaf_b200 0.1 (sm_100a)"; }
@@ -186,28 +251,34 @@ struct TimedSpan {
   }
 };
 
-// Launch configuration with programmatic dependent launch when e->pdl is on (the kernel must call pdl_wait() before its
-// first global access, gemm_sm100.cuh) and, for cluster > 1, clusters of that many CTAs along x. attr holds 2 entries.
-static cudaLaunchConfig_t launch_config(const leaf_engine* e, dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                        cudaLaunchAttribute* attr, unsigned cluster = 1) {
+// How a kernel may start relative to the one before it on the stream. PDL: with programmatic dependent launch while e->pdl is
+// on, so it may start while that kernel drains; only for kernels that call pdl_wait() before their first global access
+// (gemm_sm100.cuh). PDL_PAIR: the same, in clusters of two CTAs along x (the GEMM's CTA pairs).
+enum LaunchDep { SERIAL, PDL, PDL_PAIR };
+
+// Every kernel launch of the engine: counted for leaf_launch_count, and a failure is returned before the caller enqueues more
+template <typename... KArgs, typename... Args>
+static int launch(leaf_engine* e, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, LaunchDep dep,
+                  Args&&... args) {
+  cudaLaunchAttribute attr[2];
   cudaLaunchConfig_t cfg{.gridDim = grid, .blockDim = block, .dynamicSmemBytes = smem, .stream = st, .attrs = attr, .numAttrs = 0};
-  if (cluster > 1) {
+  if (dep == PDL_PAIR) {
     attr[cfg.numAttrs].id = cudaLaunchAttributeClusterDimension;
-    attr[cfg.numAttrs++].val.clusterDim = {cluster, 1, 1};
+    attr[cfg.numAttrs++].val.clusterDim = {2, 1, 1};
   }
-  if (e->pdl) {
+  if (dep != SERIAL && e->pdl) {
     attr[cfg.numAttrs].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[cfg.numAttrs++].val.programmaticStreamSerializationAllowed = 1;
   }
-  return cfg;
-}
-
-// A launch that may start while the previous kernel of the stream drains (programmatic dependent launch)
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(const leaf_engine* e, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
-  cudaLaunchAttribute attr[2];
-  const cudaLaunchConfig_t cfg = launch_config(e, grid, block, 0, st, attr);
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+  const cudaError_t err = cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+  if (err != cudaSuccess) {
+    cudaGetLastError();               // a launch error is not sticky: clear it, or the next CUDA call of the process reports it
+    const char* name = "kernel";
+    cudaFuncGetName(&name, kernel);
+    return fail(LEAF_ERR_CUDA, "launching %s failed: %s", name, cudaGetErrorString(err));
+  }
+  e->launches++;
+  return LEAF_OK;
 }
 
 // The GEMM's template instance per epilogue, in EPI_* order (gemm_sm100.cuh)
@@ -302,12 +373,7 @@ static int launch_gemm(leaf_engine* e, const GemmOp& op, cudaStream_t st) {
   }
   TimedSpan span(e, gemm_timing_class(epi, N, K), st);
   const int pairs = static_cast<int>(tiles < pairs_cap ? tiles : pairs_cap);
-  cudaLaunchAttribute attr[2];
-  const cudaLaunchConfig_t cfg = launch_config(e, dim3(2 * pairs), dim3(GEMM_THREADS), GEMM2_SMEM_BYTES, st, attr, 2);
-  CK(cudaLaunchKernelEx(&cfg, gemm_kernels[epi], ta, tb, p));
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, gemm_kernels[epi], 2 * pairs, GEMM_THREADS, GEMM2_SMEM_BYTES, st, PDL_PAIR, ta, tb, p);
 }
 
 extern "C" int leaf_create(const leaf_cfg_t* cfg, leaf_handle_t* out) {
@@ -324,16 +390,14 @@ extern "C" int leaf_create(const leaf_cfg_t* cfg, leaf_handle_t* out) {
   cudaDeviceProp prop;
   CK(cudaGetDeviceProperties(&prop, dev));
   if (prop.major != 10) return fail(LEAF_ERR_CUDA, "device %s is sm_%d%d; leaf_b200 is built for sm_100a only", prop.name, prop.major, prop.minor);
-  leaf_engine* e = new leaf_engine();
+  std::unique_ptr<leaf_engine> e(new leaf_engine());
   e->cfg = *cfg;
   e->device = dev;
   e->sm_count = prop.multiProcessorCount;
   void* fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) {
-    delete e;
+  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn)
     return fail(LEAF_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
-  }
   e->encode_tiled = reinterpret_cast<encode_tiled_fn>(fn);
   for (auto kernel : gemm_kernels) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM2_SMEM_BYTES));
   CK(cudaFuncSetAttribute(embed_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LEAF_VOCAB * 4));
@@ -341,56 +405,24 @@ extern "C" int leaf_create(const leaf_cfg_t* cfg, leaf_handle_t* out) {
   if (const char* pd = getenv("LEAF_PDL")) e->pdl = atoi(pd) != 0;
   CK(cudaFuncSetAttribute(attention_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
   CK(cudaFuncSetAttribute(attention_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, attb_smem_bytes(LEAF_CTX)));
-  *out = e;
+  *out = e.release();
   return LEAF_OK;
-}
-
-static void free_workspace(leaf_engine* e) {
-  cudaFree(e->x); cudaFree(e->h); cudaFree(e->big); cudaFree(e->pooled); cudaFree(e->pooled_lo); e->pooled_lo = nullptr; cudaFree(e->xc); cudaFree(e->first_of); cudaFree(e->dlt);
-  e->xc = nullptr; e->first_of = nullptr; e->dlt = nullptr;
-  cudaFree(e->cu); cudaFree(e->eos_row); cudaFree(e->total_rows); cudaFree(e->pfx); cudaFree(e->own_len); cudaFree(e->dup_of); cudaFree(e->need); cudaFree(e->meta);
-  e->x = nullptr; e->h = nullptr; e->big = nullptr; e->pooled = nullptr;
-  e->cu = e->eos_row = e->total_rows = e->pfx = e->own_len = e->dup_of = e->need = nullptr;
-  e->meta = nullptr;
-  e->max_seqs = 0; e->rows_cap = 0;
-  e->tmaps.clear();
-}
-
-static void free_weights(leaf_engine* e) {
-  for (auto& l : e->lw) {
-    cudaFree(l.qkv_w); cudaFree(l.out_w); cudaFree(l.fc1_w); cudaFree(l.fc2_w); cudaFree(l.qkv_b_own);
-  }
-  e->lw.clear();
-  cudaFree(e->proj_w); cudaFree(e->proj_w_lo);
-  e->proj_w = e->proj_w_lo = nullptr;
-  e->bound = false;
-  e->tmaps.clear();
 }
 
 extern "C" int leaf_destroy(leaf_handle_t e) {
   if (!e) return LEAF_OK;
   cudaDeviceSynchronize();
-  free_workspace(e);
-  for (void* p : e->tw.allocs) cudaFree(p);
-  e->tw = TrainWs();
-  free_weights(e);
-  for (void* p : e->table_allocs) cudaFree(p);
-  cudaFree(e->cn_count);
-  cudaFree(e->det_sum_ws);
-  cudaFree(e->det_sum_cnt);
-  for (auto& sp : e->spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
-  for (auto ev : e->event_pool) cudaEventDestroy(ev);
   delete e;
   return LEAF_OK;
 }
 
 template <typename Tp>
 static int upload(leaf_engine* e, const Tp* host, size_t count, const Tp** dev_out) {
-  void* d = nullptr;
-  CK(cudaMalloc(&d, count * sizeof(Tp)));
-  e->table_allocs.push_back(d);
+  Tp* d = nullptr;
+  int rc;
+  if ((rc = e->mem.alloc(&d, count))) return rc;
   CK(cudaMemcpy(d, host, count * sizeof(Tp), cudaMemcpyHostToDevice));
-  *dev_out = static_cast<const Tp*>(d);
+  *dev_out = d;
   return LEAF_OK;
 }
 
@@ -422,10 +454,7 @@ static int cast_to(leaf_engine* e, const float* src, __nv_bfloat16* dst, size_t 
   if (n % 4 != 0) return fail(LEAF_ERR_INVALID, "weight size not a multiple of 4");
   size_t blocks = (n / 4 + 255) / 256;
   if (blocks > 4096) blocks = 4096;
-  cast_bf16_kernel<<<static_cast<int>(blocks), 256, 0, st>>>(src, dst, n, residual);
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, cast_bf16_kernel, static_cast<int>(blocks), 256, 0, st, SERIAL, src, dst, n, residual);
 }
 
 extern "C" int leaf_refresh_weights(leaf_handle_t e, void* stream) {
@@ -435,7 +464,7 @@ extern "C" int leaf_refresh_weights(leaf_handle_t e, void* stream) {
   int rc;
   for (int l = 0; l < e->cfg.layers; ++l) {
     const leaf_layer_ptrs_t& p = e->layer_ptrs[l];
-    LayerW& w = e->lw[l];
+    LayerW& w = e->wts.lw[l];
     if (p.in_proj_w) {
       if ((rc = cast_to(e, p.in_proj_w, w.qkv_w, 3 * W * W, st))) return rc;
       w.qkv_b = p.in_proj_b;
@@ -452,17 +481,16 @@ extern "C" int leaf_refresh_weights(leaf_handle_t e, void* stream) {
     if ((rc = cast_to(e, p.fc1_w, w.fc1_w, 4 * W * W, st))) return rc;
     if ((rc = cast_to(e, p.fc2_w, w.fc2_w, 4 * W * W, st))) return rc;
   }
+  Weights& wt = e->wts;
   if (e->wp.projection_is_ew) {
-    if ((rc = cast_to(e, e->wp.text_projection, e->proj_w, E * W, st))) return rc;
-    if ((rc = cast_to(e, e->wp.text_projection, e->proj_w_lo, E * W, st, 1))) return rc;
-  } else {
-    dim3 grid(static_cast<unsigned>((E + 31) / 32), static_cast<unsigned>((W + 31) / 32));
-    cast_bf16_transpose_kernel<<<grid, dim3(32, 8), 0, st>>>(e->wp.text_projection, e->proj_w, static_cast<int>(W), static_cast<int>(E));
-    cast_bf16_transpose_kernel<<<grid, dim3(32, 8), 0, st>>>(e->wp.text_projection, e->proj_w_lo, static_cast<int>(W), static_cast<int>(E), 1);
-    e->launches += 2;
+    if ((rc = cast_to(e, e->wp.text_projection, wt.proj_w, E * W, st))) return rc;
+    return cast_to(e, e->wp.text_projection, wt.proj_w_lo, E * W, st, 1);
   }
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  dim3 grid(static_cast<unsigned>((E + 31) / 32), static_cast<unsigned>((W + 31) / 32));
+  if ((rc = launch(e, cast_bf16_transpose_kernel, grid, dim3(32, 8), 0, st, SERIAL, e->wp.text_projection, wt.proj_w,
+                   static_cast<int>(W), static_cast<int>(E), 0))) return rc;
+  return launch(e, cast_bf16_transpose_kernel, grid, dim3(32, 8), 0, st, SERIAL, e->wp.text_projection, wt.proj_w_lo,
+                static_cast<int>(W), static_cast<int>(E), 1);
 }
 
 extern "C" int leaf_bind_weights(leaf_handle_t e, const leaf_weight_ptrs_t* w, void* stream) {
@@ -478,50 +506,50 @@ extern "C" int leaf_bind_weights(leaf_handle_t e, const leaf_weight_ptrs_t* w, v
         !p.fc2_w || !p.fc2_b)
       return fail(LEAF_ERR_INVALID, "missing parameter in layer %d", l);
   }
-  free_weights(e);
+  reset(e, e->wts);
+  e->bound = false;
   e->wp = *w;
   e->layer_ptrs.assign(w->layers, w->layers + e->cfg.layers);
   e->wp.layers = e->layer_ptrs.data();
-  e->lw.resize(e->cfg.layers);
-  for (auto& l : e->lw) {
-    CK(cudaMalloc(&l.qkv_w, 3 * W * W * 2));
-    CK(cudaMalloc(&l.out_w, W * W * 2));
-    CK(cudaMalloc(&l.fc1_w, 4 * W * W * 2));
-    CK(cudaMalloc(&l.fc2_w, 4 * W * W * 2));
-    CK(cudaMalloc(&l.qkv_b_own, 3 * W * 4));
+  Weights& wt = e->wts;
+  wt.lw.resize(e->cfg.layers);
+  int rc;
+  for (auto& l : wt.lw) {
+    if ((rc = wt.mem.alloc(&l.qkv_w, 3 * W * W))) return rc;
+    if ((rc = wt.mem.alloc(&l.out_w, W * W))) return rc;
+    if ((rc = wt.mem.alloc(&l.fc1_w, 4 * W * W))) return rc;
+    if ((rc = wt.mem.alloc(&l.fc2_w, 4 * W * W))) return rc;
+    if ((rc = wt.mem.alloc(&l.qkv_b_own, 3 * W))) return rc;
   }
-  CK(cudaMalloc(&e->proj_w, E * W * 2));
-  CK(cudaMalloc(&e->proj_w_lo, E * W * 2));
+  if ((rc = wt.mem.alloc(&wt.proj_w, E * W))) return rc;
+  if ((rc = wt.mem.alloc(&wt.proj_w_lo, E * W))) return rc;
   e->bound = true;
   return leaf_refresh_weights(e, stream);
 }
 
 extern "C" int leaf_reserve(leaf_handle_t e, int32_t max_seqs) {
   if (!e || max_seqs <= 0) return fail(LEAF_ERR_INVALID, "max_seqs");
-  if (max_seqs <= e->max_seqs) return LEAF_OK;
+  if (max_seqs <= e->ws.max_seqs) return LEAF_OK;
   cudaDeviceSynchronize();
-  free_workspace(e);
-  const size_t W = e->cfg.width;
-  const size_t rows = ((static_cast<size_t>(max_seqs) * LEAF_CTX + 127) / 128) * 128;
-  CK(cudaMalloc(&e->x, rows * W * 4));
-  CK(cudaMalloc(&e->h, rows * W * 2));
-  CK(cudaMalloc(&e->big, rows * 4 * W * 2));
-  CK(cudaMalloc(&e->dlt, rows * W * 2));
-  CK(cudaMalloc(&e->pooled, (static_cast<size_t>(max_seqs) + 128) * W * 2));
-  CK(cudaMalloc(&e->pooled_lo, (static_cast<size_t>(max_seqs) + 128) * W * 2));
-  CK(cudaMalloc(&e->xc, (static_cast<size_t>(max_seqs) + 128) * W * 4));
-  CK(cudaMalloc(&e->first_of, static_cast<size_t>(max_seqs) * 4));
-  CK(cudaMalloc(&e->cu, (static_cast<size_t>(max_seqs) + 1) * 4));
-  CK(cudaMalloc(&e->eos_row, static_cast<size_t>(max_seqs) * 4));
-  CK(cudaMalloc(&e->pfx, static_cast<size_t>(max_seqs) * 4));
-  CK(cudaMalloc(&e->own_len, static_cast<size_t>(max_seqs) * 4));
-  CK(cudaMalloc(&e->dup_of, static_cast<size_t>(max_seqs) * 4));
-  CK(cudaMalloc(&e->need, static_cast<size_t>(max_seqs) * 4));
-  CK(cudaMalloc(&e->meta, static_cast<size_t>(max_seqs) * 16));
-  CK(cudaMalloc(&e->total_rows, 4));
-  CK(cudaMemset(e->total_rows, 0, 4));
-  e->max_seqs = max_seqs;
-  e->rows_cap = static_cast<long>(rows);
+  reset(e, e->ws);
+  Workspace& ws = e->ws;
+  const size_t W = e->cfg.width, n = static_cast<size_t>(max_seqs);
+  const size_t rows = ((n * LEAF_CTX + 127) / 128) * 128;
+  int rc;
+  if ((rc = ws.mem.alloc(&ws.x, rows * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.h, rows * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.big, rows * 4 * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.dlt, rows * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.pooled, (n + 128) * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.pooled_lo, (n + 128) * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.xc, (n + 128) * W))) return rc;
+  if ((rc = ws.mem.alloc(&ws.first_of, n))) return rc;
+  if ((rc = ws.mem.alloc(&ws.dup_of, n))) return rc;
+  if ((rc = ws.mem.alloc(&ws.need, n))) return rc;
+  if ((rc = alloc_pack(ws.mem, ws.pack, n))) return rc;
+  CK(cudaMemset(ws.pack.total_rows, 0, 2 * sizeof(int)));
+  ws.max_seqs = max_seqs;
+  ws.rows_cap = static_cast<long>(rows);
   return LEAF_OK;
 }
 
@@ -534,15 +562,11 @@ extern "C" int leaf_expand_tokenize(leaf_handle_t e, const uint8_t* caps, const 
   if (n > 0 && (!pos || !chr)) return fail(LEAF_ERR_INVALID, "pos/chr required when n > 0");
   K1Args a{caps, cap_off, B, n, pos, chr, sel, valid, tok_out, len_out, base_out, status_out, e->hf_tokenizer ? 1 : 0};
   const long R = static_cast<long>(B) * (n > 0 ? n : 1) + (n > 0 ? B : 0);
-  if (e->max_caption_bytes > LEAF_MAX_CAPTION_BYTES) {        // long captions: one warp per CTA with 4 KB text buffers
-    k1_expand_tokenize_kernel<K1_LONG_TEXT, 1><<<static_cast<int>(R), 32, 0, static_cast<cudaStream_t>(stream)>>>(e->tables, a);
-  } else {
-    const int grid = static_cast<int>((R + K1_WARPS_PER_CTA - 1) / K1_WARPS_PER_CTA);
-    k1_expand_tokenize_kernel<K1_MAX_TEXT, K1_WARPS_PER_CTA><<<grid, K1_WARPS_PER_CTA * 32, 0, static_cast<cudaStream_t>(stream)>>>(e->tables, a);
-  }
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (e->max_caption_bytes > LEAF_MAX_CAPTION_BYTES)          // long captions: one warp per CTA with 4 KB text buffers
+    return launch(e, k1_expand_tokenize_kernel<K1_LONG_TEXT, 1>, static_cast<int>(R), 32, 0, st, SERIAL, e->tables, a);
+  const int grid = static_cast<int>((R + K1_WARPS_PER_CTA - 1) / K1_WARPS_PER_CTA);
+  return launch(e, k1_expand_tokenize_kernel<K1_MAX_TEXT, K1_WARPS_PER_CTA>, grid, K1_WARPS_PER_CTA * 32, 0, st, SERIAL, e->tables, a);
 }
 
 // The LayerNorm kernels hold W / 128 values per lane as a template parameter: calls f(std::integral_constant<int, V>())
@@ -564,11 +588,8 @@ static int launch_layernorm(leaf_engine* e, const float* x, const int* rows_dev,
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
   return with_width(W, [&](auto V) -> int {
-    CK(launch_pdl(e, layernorm_bf16_kernel<V>, dim3(blocks), dim3(256), st, x, rows_dev, rows_max, gather, W, g, b, e->cfg.ln_eps, y,
-                  delta, y_lo));
-    e->launches++;
-    CK(cudaGetLastError());
-    return LEAF_OK;
+    return launch(e, layernorm_bf16_kernel<V>, blocks, 256, 0, st, PDL, x, rows_dev, rows_max, gather, W, g, b, e->cfg.ln_eps, y,
+                  delta, y_lo);
   });
 }
 
@@ -577,10 +598,7 @@ static int launch_attention(leaf_engine* e, const __nv_bfloat16* qkv, const int4
                             cudaStream_t st) {
   const int H = e->cfg.heads, W = e->cfg.width;
   const int grid = (N * H + ATT_WARPS - 1) / ATT_WARPS;
-  CK(launch_pdl(e, attention_kernel, dim3(grid), dim3(ATT_WARPS * 32), st, qkv, meta, N, H, W, out, last_only));
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, attention_kernel, grid, ATT_WARPS * 32, 0, st, PDL, qkv, meta, N, H, W, out, last_only);
 }
 
 extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* len, const int32_t* base, int32_t N,
@@ -589,7 +607,9 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
   if (!e || !tok || !len || !feat_out) return fail(LEAF_ERR_INVALID, "null argument");
   if (!e->bound) return fail(LEAF_ERR_STATE, "weights not bound");
   if (N <= 0) return fail(LEAF_ERR_INVALID, "N=%d", N);
-  if (N > e->max_seqs) return fail(LEAF_ERR_STATE, "workspace reserved for %d rows, need %d (leaf_reserve)", e->max_seqs, N);
+  Workspace& ws = e->ws;
+  const PackBufs& pk = ws.pack;
+  if (N > ws.max_seqs) return fail(LEAF_ERR_STATE, "workspace reserved for %d rows, need %d (leaf_reserve)", ws.max_seqs, N);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int W = e->cfg.width, E = e->cfg.embed_dim;
   const int rows_max = static_cast<int>(static_cast<long>(N) * LEAF_CTX);
@@ -599,37 +619,35 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
   TimedSpan span(e, TC_PACK, st);
   if (dedup_group > 1 && dedup_rows > 0) {
     if (dedup_rows > N || dedup_rows % dedup_group != 0) return fail(LEAF_ERR_INVALID, "dedup_rows=%d dedup_group=%d N=%d", dedup_rows, dedup_group, N);
-    dedup_kernel<<<(N + 7) / 8, 256, 0, st>>>(tok, len, dedup_rows, dedup_group, N, e->dup_of);
-    e->launches++;
-    dup = e->dup_of;
+    if ((rc = launch(e, dedup_kernel, (N + 7) / 8, 256, 0, st, SERIAL, tok, len, dedup_rows, dedup_group, N, ws.dup_of))) return rc;
+    dup = ws.dup_of;
   }
   const bool trim = trim_providers && base && dedup_rows > 0 && dedup_rows < N;
-  if (trim) CK(cudaMemsetAsync(e->need, 0, static_cast<size_t>(N) * 4, st));
-  prefix_kernel<<<(N + 7) / 8, 256, 0, st>>>(tok, len, base, dup, N, e->pfx, e->own_len, trim ? e->need : nullptr);
-  if (trim) {
-    trim_providers_kernel<<<(N - dedup_rows + 255) / 256, 256, 0, st>>>(base, e->need, dedup_rows, N, e->own_len);
-    e->launches++;
+  if (trim) CK(cudaMemsetAsync(ws.need, 0, static_cast<size_t>(N) * 4, st));
+  if ((rc = launch(e, prefix_kernel, (N + 7) / 8, 256, 0, st, SERIAL, tok, len, base, dup, N, pk.pfx, pk.own_len,
+                   trim ? ws.need : nullptr))) return rc;
+  if (trim && (rc = launch(e, trim_providers_kernel, (N - dedup_rows + 255) / 256, 256, 0, st, SERIAL, base, ws.need, dedup_rows, N,
+                           pk.own_len))) return rc;
+  if ((rc = launch(e, scan_lengths_kernel, 1, 1024, 0, st, SERIAL, pk.own_len, N, pk.cu, pk.total_rows, nullptr))) return rc;
+  if ((rc = launch(e, meta_kernel, (N + 255) / 256, 256, 0, st, SERIAL, pk.cu, pk.pfx, base, dup, N, pk.meta, pk.eos_row,
+                   ws.first_of))) return rc;
+  if ((rc = launch(e, embed_kernel, N, 256, 0, st, SERIAL, tok, pk.meta, N, W, e->wp.token_embedding, e->wp.positional_embedding,
+                   ws.x))) return rc;
   }
-  scan_lengths_kernel<<<1, 1024, 0, st>>>(e->own_len, N, e->cu, e->total_rows);
-  meta_kernel<<<(N + 255) / 256, 256, 0, st>>>(e->cu, e->pfx, base, dup, N, e->meta, e->eos_row, e->first_of);
-  embed_kernel<<<N, 256, 0, st>>>(tok, e->meta, N, W, e->wp.token_embedding, e->wp.positional_embedding, e->x);
-  e->launches += 4;
-  }
-  CK(cudaGetLastError());
   for (int l = 0; l < e->cfg.layers; ++l) {
     const leaf_layer_ptrs_t& p = e->layer_ptrs[l];
-    const LayerW& w = e->lw[l];
-    if ((rc = launch_layernorm(e, e->x, e->total_rows, rows_max, nullptr, p.ln1_w, p.ln1_b, e->h, st))) return rc;
-    if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.qkv_w, .C = e->big, .M = rows_max, .m_dev = e->total_rows,
+    const LayerW& w = e->wts.lw[l];
+    if ((rc = launch_layernorm(e, ws.x, pk.total_rows, rows_max, nullptr, p.ln1_w, p.ln1_b, ws.h, st))) return rc;
+    if ((rc = launch_gemm(e, {.A = ws.h, .a_rows = ws.rows_cap, .B = w.qkv_w, .C = ws.big, .M = rows_max, .m_dev = pk.total_rows,
                               .N = 3 * W, .K = W, .epi = EPI_BF16, .bias = w.qkv_b}, st))) return rc;
     // Final layer: only the pooled EOS position of a sequence is read after it (transformer.py:661), so everything past
     // the key/value projection runs on ONE row per sequence: attention writes the EOS query's output to h[seq], the
     // residual rows are compacted into xc, and out-proj / LayerNorm / MLP see N rows instead of the packed row count.
     const bool last = e->prune_last && l == e->cfg.layers - 1;
-    const __nv_bfloat16* dl = e->dlt;
+    const __nv_bfloat16* dl = ws.dlt;
     {
       TimedSpan span(e, TC_ATTENTION, st);
-      if ((rc = launch_attention(e, e->big, e->meta, N, e->h, last ? 1 : 0, st))) return rc;
+      if ((rc = launch_attention(e, ws.big, pk.meta, N, ws.h, last ? 1 : 0, st))) return rc;
     }
     // The attention branch's out-proj result stays OUT of the fp32 residual stream for now: it is stored as a bf16
     // delta (2 B per element, no read), LayerNorm normalises x + delta on the fly, and fc2's epilogue writes
@@ -640,43 +658,38 @@ extern "C" int leaf_encode(leaf_handle_t e, const int32_t* tok, const int32_t* l
     if (last) {
       {
         TimedSpan span(e, TC_PACK, st);
-        gather_rows_f32_kernel<<<(N + 7) / 8, 256, 0, st>>>(e->x, e->eos_row, N, W, e->xc);
-        e->launches++;
+        if ((rc = launch(e, gather_rows_f32_kernel, (N + 7) / 8, 256, 0, st, SERIAL, ws.x, pk.eos_row, N, W, ws.xc))) return rc;
       }
-      if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.out_w, .C = e->dlt, .M = N, .N = W, .K = W, .epi = EPI_BF16,
+      if ((rc = launch_gemm(e, {.A = ws.h, .a_rows = ws.rows_cap, .B = w.out_w, .C = ws.dlt, .M = N, .N = W, .K = W, .epi = EPI_BF16,
                                 .bias = p.out_b}, st))) return rc;
-      if ((rc = launch_layernorm(e, e->xc, nullptr, N, nullptr, p.ln2_w, p.ln2_b, e->h, st, dl))) return rc;
-      if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.fc1_w, .C = e->big, .M = N, .N = 4 * W, .K = W,
+      if ((rc = launch_layernorm(e, ws.xc, nullptr, N, nullptr, p.ln2_w, p.ln2_b, ws.h, st, dl))) return rc;
+      if ((rc = launch_gemm(e, {.A = ws.h, .a_rows = ws.rows_cap, .B = w.fc1_w, .C = ws.big, .M = N, .N = 4 * W, .K = W,
                                 .epi = EPI_BF16_ACT, .act = e->cfg.activation, .bias = p.fc1_b}, st))) return rc;
-      if ((rc = launch_gemm(e, {.A = e->big, .a_rows = e->rows_cap, .B = w.fc2_w, .C = e->xc, .M = N, .N = W, .K = 4 * W,
+      if ((rc = launch_gemm(e, {.A = ws.big, .a_rows = ws.rows_cap, .B = w.fc2_w, .C = ws.xc, .M = N, .N = W, .K = 4 * W,
                                 .epi = EPI_F32_RESIDUAL, .bias = p.fc2_b, .delta = dl}, st))) return rc;
       break;
     }
-    if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.out_w, .C = e->dlt, .M = rows_max, .m_dev = e->total_rows,
+    if ((rc = launch_gemm(e, {.A = ws.h, .a_rows = ws.rows_cap, .B = w.out_w, .C = ws.dlt, .M = rows_max, .m_dev = pk.total_rows,
                               .N = W, .K = W, .epi = EPI_BF16, .bias = p.out_b}, st))) return rc;
-    if ((rc = launch_layernorm(e, e->x, e->total_rows, rows_max, nullptr, p.ln2_w, p.ln2_b, e->h, st, dl))) return rc;
-    if ((rc = launch_gemm(e, {.A = e->h, .a_rows = e->rows_cap, .B = w.fc1_w, .C = e->big, .M = rows_max, .m_dev = e->total_rows,
+    if ((rc = launch_layernorm(e, ws.x, pk.total_rows, rows_max, nullptr, p.ln2_w, p.ln2_b, ws.h, st, dl))) return rc;
+    if ((rc = launch_gemm(e, {.A = ws.h, .a_rows = ws.rows_cap, .B = w.fc1_w, .C = ws.big, .M = rows_max, .m_dev = pk.total_rows,
                               .N = 4 * W, .K = W, .epi = EPI_BF16_ACT, .act = e->cfg.activation, .bias = p.fc1_b}, st))) return rc;
-    if ((rc = launch_gemm(e, {.A = e->big, .a_rows = e->rows_cap, .B = w.fc2_w, .C = e->x, .M = rows_max, .m_dev = e->total_rows,
+    if ((rc = launch_gemm(e, {.A = ws.big, .a_rows = ws.rows_cap, .B = w.fc2_w, .C = ws.x, .M = rows_max, .m_dev = pk.total_rows,
                               .N = W, .K = 4 * W, .epi = EPI_F32_RESIDUAL, .bias = p.fc2_b, .delta = dl}, st))) return rc;
   }
   // ln_final and the projection in split precision: both operands carry what their bf16 rounding dropped as a second bf16
   // matrix (pooled = hi + lo, P = hi + lo; feat = hi.hi + lo.hi + hi.lo, fp32 accumulate: error 2^-17 instead of 2^-9). One row
   // per sequence and 2 W E FLOP each: 0.1 ms per step, and it removes ~15 % of the TextFARE-loss error against the fp32
   // reference (tests/tools/exp_final_stage_precision.py: the last stage's rounding alone is worth 1.2-1.9e-3 of loss rel. error).
-  if (e->prune_last) rc = launch_layernorm(e, e->xc, nullptr, N, e->first_of, e->wp.lnf_w, e->wp.lnf_b, e->pooled, st, nullptr, e->pooled_lo);
-  else rc = launch_layernorm(e, e->x, nullptr, N, e->eos_row, e->wp.lnf_w, e->wp.lnf_b, e->pooled, st, nullptr, e->pooled_lo);
+  if (e->prune_last) rc = launch_layernorm(e, ws.xc, nullptr, N, ws.first_of, e->wp.lnf_w, e->wp.lnf_b, ws.pooled, st, nullptr, ws.pooled_lo);
+  else rc = launch_layernorm(e, ws.x, nullptr, N, pk.eos_row, e->wp.lnf_w, e->wp.lnf_b, ws.pooled, st, nullptr, ws.pooled_lo);
   if (rc) return rc;
-  const long pooled_rows = e->max_seqs + 128;
-  if ((rc = launch_gemm(e, {.A = e->pooled, .a_rows = pooled_rows, .B = e->proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32}, st))) return rc;
-  if ((rc = launch_gemm(e, {.A = e->pooled_lo, .a_rows = pooled_rows, .B = e->proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32_RESIDUAL}, st))) return rc;
-  if ((rc = launch_gemm(e, {.A = e->pooled, .a_rows = pooled_rows, .B = e->proj_w_lo, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32_RESIDUAL}, st))) return rc;
-  if (normalize) {
-    l2_normalize_kernel<<<(N + 7) / 8, 256, 0, st>>>(feat_out, N, E);
-    e->launches++;
-  }
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  const long pooled_rows = ws.max_seqs + 128;
+  const __nv_bfloat16 *proj_w = e->wts.proj_w, *proj_w_lo = e->wts.proj_w_lo;
+  if ((rc = launch_gemm(e, {.A = ws.pooled, .a_rows = pooled_rows, .B = proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32}, st))) return rc;
+  if ((rc = launch_gemm(e, {.A = ws.pooled_lo, .a_rows = pooled_rows, .B = proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32_RESIDUAL}, st))) return rc;
+  if ((rc = launch_gemm(e, {.A = ws.pooled, .a_rows = pooled_rows, .B = proj_w_lo, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32_RESIDUAL}, st))) return rc;
+  return normalize ? launch(e, l2_normalize_kernel, (N + 7) / 8, 256, 0, st, SERIAL, feat_out, N, E) : LEAF_OK;
 }
 
 extern "C" int leaf_score(leaf_handle_t e, const float* feat, const float* anchor, int32_t B, int32_t n, int32_t objective,
@@ -685,11 +698,8 @@ extern "C" int leaf_score(leaf_handle_t e, const float* feat, const float* ancho
   if (B <= 0 || n <= 0 || objective < 0 || objective > 3) return fail(LEAF_ERR_INVALID, "B=%d n=%d objective=%d", B, n, objective);
   if (e->cfg.embed_dim % 4 != 0) return fail(LEAF_ERR_INVALID, "embed_dim");
   if (static_cast<size_t>(n) * 4 > 48 * 1024) return fail(LEAF_ERR_INVALID, "n=%d too large", n);
-  score_argmax_kernel<<<B, 256, static_cast<size_t>(n) * 4, static_cast<cudaStream_t>(stream)>>>(
-      feat, anchor, n, e->cfg.embed_dim, objective, loss_out, best_out, best_feat_out);
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, score_argmax_kernel, B, 256, static_cast<size_t>(n) * 4, static_cast<cudaStream_t>(stream), SERIAL, feat, anchor, n,
+                e->cfg.embed_dim, objective, loss_out, best_out, best_feat_out);
 }
 
 extern "C" int leaf_topk(leaf_handle_t e, const float* score_a, const float* score_b, int32_t m, int32_t k, int32_t* idx_out,
@@ -698,10 +708,7 @@ extern "C" int leaf_topk(leaf_handle_t e, const float* score_a, const float* sco
   if (m <= 0 || k <= 0 || k > m) return fail(LEAF_ERR_INVALID, "top-k of m=%d, k=%d", m, k);
   const size_t smem = static_cast<size_t>(m) * 4;
   if (smem > 200 * 1024) return fail(LEAF_ERR_INVALID, "m=%d too large (max %d)", m, 200 * 1024 / 4);
-  topk_kernel<<<1, 1024, smem, static_cast<cudaStream_t>(stream)>>>(score_a, score_b, m, k, idx_out, val_out);
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, topk_kernel, 1, 1024, smem, static_cast<cudaStream_t>(stream), SERIAL, score_a, score_b, m, k, idx_out, val_out);
 }
 
 extern "C" int leaf_gemm_bf16(leaf_handle_t e, const void* A, const void* Bt, const float* bias, void* C, int32_t M, int32_t N,
@@ -737,12 +744,9 @@ extern "C" int leaf_test_attention(leaf_handle_t e, const void* qkv, const int32
 extern "C" int leaf_test_attention_bwd(leaf_handle_t e, const void* qkv, const void* o, const float* dout, const int32_t* meta,
                                        int32_t N, int32_t T, void* dqkv, void* stream) {
   if (!e || !qkv || !o || !dout || !meta || !dqkv || N <= 0 || T <= 0 || T > LEAF_CTX) return fail(LEAF_ERR_INVALID, "bad argument");
-  attention_bwd_kernel<false><<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(T), static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(o), dout, reinterpret_cast<const int4*>(meta),
-      e->cfg.width, T, static_cast<__nv_bfloat16*>(dqkv));
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, attention_bwd_kernel<false>, dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(T), static_cast<cudaStream_t>(stream),
+                SERIAL, static_cast<const __nv_bfloat16*>(qkv), static_cast<const __nv_bfloat16*>(o), dout, reinterpret_cast<const int4*>(meta),
+                e->cfg.width, T, static_cast<__nv_bfloat16*>(dqkv), nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 extern "C" int leaf_set_prune_last(leaf_handle_t e, int32_t on) {
@@ -759,9 +763,9 @@ extern "C" int64_t leaf_launch_count(leaf_handle_t e, int32_t reset) {
 }
 
 extern "C" int64_t leaf_last_rows(leaf_handle_t e) {
-  if (!e || !e->total_rows) return 0;
+  if (!e || !e->ws.pack.total_rows) return 0;
   int v = 0;
-  if (cudaMemcpy(&v, e->total_rows, 4, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+  if (cudaMemcpy(&v, e->ws.pack.total_rows, 4, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
   return v;
 }
 
@@ -804,21 +808,6 @@ extern "C" double leaf_timing_ms(leaf_handle_t e, int32_t which, int32_t* launch
 //   wgrad  dW[out,in] += dY^T[out,M] . X[M,in]           -> A = dY [M,out], B = X [M,in], both MN-major (GEMM_A_MN | GEMM_B_MN;
 //                                                           fp32 accumulate into .grad)
 // =====================================================================================================================
-template <typename Tp>
-static int tw_alloc(TrainWs& t, Tp** p, size_t count) {
-  void* d = nullptr;
-  CK(cudaMalloc(&d, count * sizeof(Tp)));
-  t.allocs.push_back(d);
-  *p = static_cast<Tp*>(d);
-  return LEAF_OK;
-}
-
-static void free_train(leaf_engine* e) {
-  for (void* p : e->tw.allocs) cudaFree(p);
-  e->tw = TrainWs();
-  e->tmaps.clear();
-}
-
 // Workspace of the deterministic backward for the reserved training shape (a no-op when it exists or nothing is reserved).
 // Largest user of each buffer: the split-K partial tiles (two waves of work units at the device's pair count), fc1's bias
 // (one row of column sums per 32 packed rows), the LayerNorm bands (at most 2 x SMs / column blocks + 1), the attention
@@ -835,9 +824,9 @@ static int reserve_deterministic(leaf_engine* e) {
   size_t c = std::max(pairs * 2 * EPI_WARPS, (4 * W + GEMM_BN - 1) / GEMM_BN * 4);
   c = std::max(c, std::max(cbx, static_cast<size_t>(e->cfg.heads)));
   int rc;
-  if ((rc = tw_alloc(t, &t.det_ws, f))) return rc;
-  if ((rc = tw_alloc(t, &t.det_cnt, c))) return rc;
-  if ((rc = tw_alloc(t, &t.det_idx, 3 * rows))) return rc;
+  if ((rc = t.mem.alloc(&t.det_ws, f))) return rc;
+  if ((rc = t.mem.alloc(&t.det_cnt, c))) return rc;
+  if ((rc = t.mem.alloc(&t.det_idx, 3 * rows))) return rc;
   CK(cudaMemset(t.det_cnt, 0, c * 4));
   CK(cudaDeviceSynchronize());
   t.det_ws_floats = f;
@@ -852,36 +841,31 @@ extern "C" int leaf_train_reserve(leaf_handle_t e, int32_t max_seqs) {
   int rc;
   if (max_seqs <= e->tw.max_seqs) return LEAF_OK;
   cudaDeviceSynchronize();
-  free_train(e);
+  reset(e, e->tw);
   TrainWs& t = e->tw;
   const size_t rows = ((static_cast<size_t>(max_seqs) * LEAF_CTX + 127) / 128) * 128;
   const size_t wide = 4 * W > E ? 4 * W : E;
   t.L.resize(e->cfg.layers);
   for (auto& l : t.L) {
-    if ((rc = tw_alloc(t, &l.x_in, rows * W))) return rc;
-    if ((rc = tw_alloc(t, &l.x_mid, rows * W))) return rc;
-    if ((rc = tw_alloc(t, &l.h1, rows * W))) return rc;
-    if ((rc = tw_alloc(t, &l.qkv, rows * 3 * W))) return rc;
-    if ((rc = tw_alloc(t, &l.o, rows * W))) return rc;
-    if ((rc = tw_alloc(t, &l.h2, rows * W))) return rc;
-    if ((rc = tw_alloc(t, &l.u, rows * 4 * W))) return rc;
-    if ((rc = tw_alloc(t, &l.g, rows * 4 * W))) return rc;
+    if ((rc = t.mem.alloc(&l.x_in, rows * W))) return rc;
+    if ((rc = t.mem.alloc(&l.x_mid, rows * W))) return rc;
+    if ((rc = t.mem.alloc(&l.h1, rows * W))) return rc;
+    if ((rc = t.mem.alloc(&l.qkv, rows * 3 * W))) return rc;
+    if ((rc = t.mem.alloc(&l.o, rows * W))) return rc;
+    if ((rc = t.mem.alloc(&l.h2, rows * W))) return rc;
+    if ((rc = t.mem.alloc(&l.u, rows * 4 * W))) return rc;
+    if ((rc = t.mem.alloc(&l.g, rows * 4 * W))) return rc;
   }
-  if ((rc = tw_alloc(t, &t.x_out, rows * W))) return rc;
-  if ((rc = tw_alloc(t, &t.dx, rows * W))) return rc;
-  if ((rc = tw_alloc(t, &t.dtmp, rows * wide))) return rc;
-  if ((rc = tw_alloc(t, &t.scratch, 2 * W))) return rc;
-  if ((rc = tw_alloc(t, &t.pooled, (static_cast<size_t>(max_seqs) + 128) * W))) return rc;
-  if ((rc = tw_alloc(t, &t.d16, rows * wide))) return rc;
-  if ((rc = tw_alloc(t, &t.dx16, rows * W))) return rc;
-  if ((rc = tw_alloc(t, &t.ln_stats, rows * 2))) return rc;
-  if ((rc = tw_alloc(t, &t.tok, static_cast<size_t>(max_seqs) * LEAF_CTX))) return rc;
-  if ((rc = tw_alloc(t, &t.cu, static_cast<size_t>(max_seqs) + 1))) return rc;
-  if ((rc = tw_alloc(t, &t.eos_row, static_cast<size_t>(max_seqs)))) return rc;
-  if ((rc = tw_alloc(t, &t.total_rows, 2))) return rc;
-  if ((rc = tw_alloc(t, &t.pfx, static_cast<size_t>(max_seqs)))) return rc;
-  if ((rc = tw_alloc(t, &t.own_len, static_cast<size_t>(max_seqs)))) return rc;
-  if ((rc = tw_alloc(t, &t.meta, static_cast<size_t>(max_seqs)))) return rc;
+  if ((rc = t.mem.alloc(&t.x_out, rows * W))) return rc;
+  if ((rc = t.mem.alloc(&t.dx, rows * W))) return rc;
+  if ((rc = t.mem.alloc(&t.dtmp, rows * wide))) return rc;
+  if ((rc = t.mem.alloc(&t.scratch, 2 * W))) return rc;
+  if ((rc = t.mem.alloc(&t.pooled, (static_cast<size_t>(max_seqs) + 128) * W))) return rc;
+  if ((rc = t.mem.alloc(&t.d16, rows * wide))) return rc;
+  if ((rc = t.mem.alloc(&t.dx16, rows * W))) return rc;
+  if ((rc = t.mem.alloc(&t.ln_stats, rows * 2))) return rc;
+  if ((rc = t.mem.alloc(&t.tok, static_cast<size_t>(max_seqs) * LEAF_CTX))) return rc;
+  if ((rc = alloc_pack(t.mem, t.pack, static_cast<size_t>(max_seqs)))) return rc;
   t.max_seqs = max_seqs;
   t.rows_cap = static_cast<long>(rows);
   return e->deterministic ? reserve_deterministic(e) : LEAF_OK;
@@ -910,32 +894,32 @@ extern "C" int leaf_forward_train(leaf_handle_t e, const int32_t* tok, const int
   t.have_forward = false;
   t.generation = ++e->train_generation;
   CK(cudaMemcpyAsync(t.tok, tok, static_cast<size_t>(N) * LEAF_CTX * 4, cudaMemcpyDeviceToDevice, st));
-  prefix_kernel<<<(N + 7) / 8, 256, 0, st>>>(tok, len, nullptr, nullptr, N, t.pfx, t.own_len);
-  scan_lengths_kernel<<<1, 1024, 0, st>>>(t.own_len, N, t.cu, t.total_rows, t.total_rows + 1);
-  meta_kernel<<<(N + 255) / 256, 256, 0, st>>>(t.cu, t.pfx, nullptr, nullptr, N, t.meta, t.eos_row);
-  e->launches += 3;
+  const PackBufs& pk = t.pack;
+  if ((rc = launch(e, prefix_kernel, (N + 7) / 8, 256, 0, st, SERIAL, tok, len, nullptr, nullptr, N, pk.pfx, pk.own_len, nullptr))) return rc;
+  if ((rc = launch(e, scan_lengths_kernel, 1, 1024, 0, st, SERIAL, pk.own_len, N, pk.cu, pk.total_rows, pk.total_rows + 1))) return rc;
+  if ((rc = launch(e, meta_kernel, (N + 255) / 256, 256, 0, st, SERIAL, pk.cu, pk.pfx, nullptr, nullptr, N, pk.meta, pk.eos_row,
+                   nullptr))) return rc;
   int mt[2] = {rows_hint, max_len_hint};
   if (rows_hint > 0 && max_len_hint > 0) {             // the caller knows the lengths (e.g. from the tokenizer's status read): no sync
-    check_train_hints_kernel<<<1, 1, 0, st>>>(t.total_rows, rows_hint, max_len_hint);
-    e->launches++;
+    if ((rc = launch(e, check_train_hints_kernel, 1, 1, 0, st, SERIAL, pk.total_rows, rows_hint, max_len_hint))) return rc;
   } else {
-    CK(cudaMemcpyAsync(mt, t.total_rows, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(mt, pk.total_rows, 8, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));                     // packed row count (sizes the wgrad contractions) + longest sequence
   }
   const int M = mt[0];
   if (M <= 0 || M > t.rows_cap || mt[1] <= 0 || mt[1] > LEAF_CTX) return fail(LEAF_ERR_STATE, "bad packed row count %d / length %d", M, mt[1]);
   t.N = N; t.M = M; t.T = mt[1];
-  embed_kernel<<<N, 256, 0, st>>>(tok, t.meta, N, W, e->wp.token_embedding, e->wp.positional_embedding, t.L[0].x_in);
-  e->launches++;
+  if ((rc = launch(e, embed_kernel, N, 256, 0, st, SERIAL, tok, pk.meta, N, W, e->wp.token_embedding, e->wp.positional_embedding,
+                   t.L[0].x_in))) return rc;
   for (int l = 0; l < e->cfg.layers; ++l) {
     const leaf_layer_ptrs_t& p = e->layer_ptrs[l];
-    const LayerW& w = e->lw[l];
+    const LayerW& w = e->wts.lw[l];
     TrainLayer& a = t.L[l];
     float* x_next = (l + 1 < e->cfg.layers) ? t.L[l + 1].x_in : t.x_out;
     if ((rc = launch_layernorm(e, a.x_in, nullptr, M, nullptr, p.ln1_w, p.ln1_b, a.h1, st))) return rc;
     if ((rc = launch_gemm(e, {.A = a.h1, .a_rows = t.rows_cap, .B = w.qkv_w, .C = a.qkv, .M = M, .N = 3 * W, .K = W, .epi = EPI_BF16,
                               .bias = w.qkv_b}, st))) return rc;
-    if ((rc = launch_attention(e, a.qkv, t.meta, N, a.o, 0, st))) return rc;
+    if ((rc = launch_attention(e, a.qkv, pk.meta, N, a.o, 0, st))) return rc;
     if ((rc = launch_gemm(e, {.A = a.o, .a_rows = t.rows_cap, .B = w.out_w, .C = a.x_mid, .M = M, .N = W, .K = W, .epi = EPI_F32_RESIDUAL,
                               .bias = p.out_b, .res = a.x_in}, st))) return rc;
     if ((rc = launch_layernorm(e, a.x_mid, nullptr, M, nullptr, p.ln2_w, p.ln2_b, a.h2, st))) return rc;
@@ -945,9 +929,8 @@ extern "C" int leaf_forward_train(leaf_handle_t e, const int32_t* tok, const int
     if ((rc = launch_gemm(e, {.A = a.g, .a_rows = t.rows_cap, .B = w.fc2_w, .C = x_next, .M = M, .N = W, .K = 4 * W, .epi = EPI_F32_RESIDUAL,
                               .bias = p.fc2_b, .res = a.x_mid}, st))) return rc;
   }
-  if ((rc = launch_layernorm(e, t.x_out, nullptr, N, t.eos_row, e->wp.lnf_w, e->wp.lnf_b, t.pooled, st))) return rc;
-  if ((rc = launch_gemm(e, {.A = t.pooled, .a_rows = t.max_seqs + 128, .B = e->proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32}, st))) return rc;
-  CK(cudaGetLastError());
+  if ((rc = launch_layernorm(e, t.x_out, nullptr, N, pk.eos_row, e->wp.lnf_w, e->wp.lnf_b, t.pooled, st))) return rc;
+  if ((rc = launch_gemm(e, {.A = t.pooled, .a_rows = t.max_seqs + 128, .B = e->wts.proj_w, .C = feat_out, .M = N, .N = E, .K = W, .epi = EPI_F32}, st))) return rc;
   t.have_forward = true;
   if (generation_out) *generation_out = t.generation;
   return LEAF_OK;
@@ -966,8 +949,8 @@ static int launch_layernorm_bwd(leaf_engine* e, const float* dy, const float* x,
   if (blocks > 2 * e->sm_count) blocks = 2 * e->sm_count;
   if (blocks < 1) blocks = 1;
   int rc = with_width(W, [&](auto V) -> int {
-    layernorm_bwd_rows_kernel<V><<<blocks, 256, 0, st>>>(dy, x, gather, rows, W, gamma, e->cfg.ln_eps, dx, accumulate, dx16, stats);
-    return LEAF_OK;
+    return launch(e, layernorm_bwd_rows_kernel<V>, blocks, 256, 0, st, SERIAL, dy, x, gather, rows, W, gamma, e->cfg.ln_eps, dx,
+                  accumulate, dx16, stats);
   });
   if (rc) return rc;
   const int cbx = (W + 255) / 256;
@@ -977,11 +960,8 @@ static int launch_layernorm_bwd(leaf_engine* e, const float* dy, const float* x,
   const bool det = e->deterministic;                  // band sums added in band order (train_kernels.cuh)
   if (det && (static_cast<size_t>(bands) * 3 * W > e->tw.det_ws_floats || static_cast<size_t>(cbx) > e->tw.det_cnt_ints))
     return fail(LEAF_ERR_STATE, "deterministic workspace too small for the LayerNorm backward (%d bands)", bands);
-  CK(launch_pdl(e, det ? layernorm_bwd_cols_kernel<true> : layernorm_bwd_cols_kernel<false>, dim3(cbx, bands), dim3(256), st, dy, x,
-                gather, stats, dx, rows, W, dgamma, dbeta, dxsum, det ? e->tw.det_ws : nullptr, det ? e->tw.det_cnt : nullptr));
-  e->launches += 2;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, det ? layernorm_bwd_cols_kernel<true> : layernorm_bwd_cols_kernel<false>, dim3(cbx, bands), 256, 0, st, PDL, dy, x,
+                gather, stats, dx, rows, W, dgamma, dbeta, dxsum, det ? e->tw.det_ws : nullptr, det ? e->tw.det_cnt : nullptr);
 }
 
 // grads mirrors leaf_weight_ptrs_t: fp32 device buffers that are ACCUMULATED into (+=); NULL = parameter is frozen.
@@ -1014,9 +994,8 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
   };
   // ---- projection + ln_final on the pooled rows ----
   const size_t nfe = static_cast<size_t>(N) * E;
-  cast_f32_bf16_kernel<<<launch_ew(e, nfe), 256, 0, st>>>(dfeat, t.d16, nfe);
-  e->launches++;
-  if ((rc = dgrad(t.d16, N, e->proj_w, t.dtmp, N, W, E))) return rc;                                        // dpooled [N,W] = dfeat . P[E,W]
+  if ((rc = launch(e, cast_f32_bf16_kernel, launch_ew(e, nfe), 256, 0, st, SERIAL, dfeat, t.d16, nfe))) return rc;
+  if ((rc = dgrad(t.d16, N, e->wts.proj_w, t.dtmp, N, W, E))) return rc;                                        // dpooled [N,W] = dfeat . P[E,W]
   const GemmOp dp_ew = {.A = t.d16, .B = t.pooled, .mn_major = GEMM_A_MN | GEMM_B_MN, .C = F(grads->text_projection), .M = E, .N = W,
                         .K = N, .epi = EPI_F32_RESIDUAL, .split_k_ok = true};                               // dP[E,W] += dfeat^T . pooled
   const GemmOp dp_we = {.A = t.pooled, .B = t.d16, .mn_major = GEMM_A_MN | GEMM_B_MN, .C = F(grads->text_projection), .M = W, .N = E,
@@ -1028,13 +1007,13 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
   CK(cudaMemsetAsync(scratch, 0, 2 * W * 4, st));
   // the bias gradients that are column sums of dx (fc2's, out-proj's) are accumulated by the LayerNorm backward that writes
   // that dx: ln_final / the layer above's ln_1 for fc2, this layer's ln_2 for out-proj
-  if ((rc = launch_layernorm_bwd(e, t.dtmp, t.x_out, t.eos_row, N, e->wp.lnf_w, t.dx, 0, F(grads->lnf_w), F(grads->lnf_b), scratch, st, t.dx16,
+  if ((rc = launch_layernorm_bwd(e, t.dtmp, t.x_out, t.pack.eos_row, N, e->wp.lnf_w, t.dx, 0, F(grads->lnf_w), F(grads->lnf_b), scratch, st, t.dx16,
                                  F(grads->layers[e->cfg.layers - 1].fc2_b)))) return rc;
   if (e->bwd_hook) e->bwd_hook(e->cfg.layers, e->bwd_hook_user);          // projection + ln_final gradients are enqueued
   for (int l = e->cfg.layers - 1; l >= 0; --l) {
     const leaf_layer_ptrs_t& p = e->layer_ptrs[l];
     const leaf_layer_ptrs_t& g = grads->layers[l];
-    const LayerW& w = e->lw[l];
+    const LayerW& w = e->wts.lw[l];
     TrainLayer& a = t.L[l];
     // ================= MLP branch: x_next = x_mid + fc2(act(fc1(ln_2(x_mid)))) =================
     // du [M,4W] = (dx . W2[W,4W]) * act'(u), bf16, with fc1's bias gradient (its column sums): one GEMM, the activation
@@ -1054,11 +1033,9 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
       float* bv = p.in_proj_w ? (g.in_proj_b ? F(g.in_proj_b) + 2 * W : nullptr) : F(g.v_b);
       const bool det = e->deterministic && (bq || bk || bv);   // bias column sums added in (sequence, warp) order
       auto attention_bwd = det ? attention_bwd_kernel<true> : attention_bwd_kernel<false>;
-      attention_bwd<<<dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st>>>(a.qkv, a.o, t.dtmp, t.meta, W, t.T, t.d16, bq, bk, bv,
-                                                                                            det ? t.det_ws : nullptr, det ? t.det_cnt : nullptr);
+      if ((rc = launch(e, attention_bwd, dim3(N, e->cfg.heads), ATTB_WARPS * 32, attb_smem_bytes(t.T), st, SERIAL, a.qkv, a.o, t.dtmp,
+                       t.pack.meta, W, t.T, t.d16, bq, bk, bv, det ? t.det_ws : nullptr, det ? t.det_cnt : nullptr))) return rc;
     }
-    e->launches++;
-    CK(cudaGetLastError());
     if ((rc = dgrad(t.d16, cap, w.qkv_w, t.dtmp, M, W, 3 * W))) return rc;                                  // dh1 [M,W]
     if (p.in_proj_w) {                                                                                       // layout of the bound parameters
       if (g.in_proj_w && (rc = wgrad(t.d16, 0, a.h1, F(g.in_proj_w), M, W, 3 * W))) return rc;
@@ -1080,16 +1057,14 @@ extern "C" int leaf_backward(leaf_handle_t e, int64_t generation, const float* d
       int* row_tok = t.det_idx;
       int* order = row_tok + t.rows_cap;
       int* key = order + t.rows_cap;
-      embed_sort_kernel<<<1, 1024, LEAF_VOCAB * 4, st>>>(t.tok, t.meta, N, M, row_tok, order, key);
-      embed_bwd_det_kernel<<<dim3(M + LEAF_CTX, (W + 255) / 256), 256, 0, st>>>(order, key, t.meta, N, M, W, t.dx, F(grads->token_embedding),
-                                                                                F(grads->positional_embedding));
-      e->launches += 2;
+      if ((rc = launch(e, embed_sort_kernel, 1, 1024, LEAF_VOCAB * 4, st, SERIAL, t.tok, t.pack.meta, N, M, row_tok, order, key))) return rc;
+      if ((rc = launch(e, embed_bwd_det_kernel, dim3(M + LEAF_CTX, (W + 255) / 256), 256, 0, st, SERIAL, order, key, t.pack.meta, N, M, W,
+                       t.dx, F(grads->token_embedding), F(grads->positional_embedding)))) return rc;
     } else {
-      embed_bwd_kernel<<<N, 256, 0, st>>>(t.tok, t.meta, N, W, t.dx, F(grads->token_embedding), F(grads->positional_embedding));
-      e->launches++;
+      if ((rc = launch(e, embed_bwd_kernel, N, 256, 0, st, SERIAL, t.tok, t.pack.meta, N, W, t.dx, F(grads->token_embedding),
+                       F(grads->positional_embedding)))) return rc;
     }
   }
-  CK(cudaGetLastError());
   t.have_forward = false;                              // consumed: dx / dtmp were overwritten, a second backward would be wrong
   if (e->bwd_hook) e->bwd_hook(-1, e->bwd_hook_user);  // everything, embeddings included
   return LEAF_OK;
@@ -1108,8 +1083,9 @@ extern "C" int leaf_set_deterministic(leaf_handle_t e, int32_t on) {
   if (!e) return fail(LEAF_ERR_INVALID, "null handle");
   if (on) {
     if (!e->det_sum_ws) {
-      CK(cudaMalloc(&e->det_sum_ws, static_cast<size_t>(e->sm_count) * 16 * 4));
-      CK(cudaMalloc(&e->det_sum_cnt, 4));
+      int rc;
+      if ((rc = e->mem.alloc(&e->det_sum_ws, static_cast<size_t>(e->sm_count) * 16))) return rc;
+      if ((rc = e->mem.alloc(&e->det_sum_cnt, 1))) return rc;
       CK(cudaMemset(e->det_sum_cnt, 0, 4));
       CK(cudaDeviceSynchronize());
     }
@@ -1141,35 +1117,26 @@ extern "C" int leaf_adamw(leaf_handle_t e, float* params, const float* grads, fl
     return fail(LEAF_ERR_INVALID, "AdamW buffers must be 16-byte aligned");
   const float bc1 = 1.f - powf(beta1, static_cast<float>(step));
   const float bc2s = sqrtf(1.f - powf(beta2, static_cast<float>(step)));
-  adamw_kernel<<<launch_ew(e, static_cast<size_t>(n) / 4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      params, grads, exp_avg, exp_avg_sq, static_cast<size_t>(n), static_cast<size_t>(n_nodecay), lr, beta1, beta2, eps,
-      weight_decay, bc1, bc2s, grad_scale);
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, adamw_kernel, launch_ew(e, static_cast<size_t>(n) / 4), 256, 0, static_cast<cudaStream_t>(stream), SERIAL, params, grads,
+                exp_avg, exp_avg_sq, static_cast<size_t>(n), static_cast<size_t>(n_nodecay), lr, beta1, beta2, eps, weight_decay, bc1,
+                bc2s, grad_scale);
 }
 
 // out[0] (device fp32, zeroed by the caller) += sum of squares of g[0, n)
 extern "C" int leaf_sumsq(leaf_handle_t e, const float* g, int64_t n, float* out, void* stream) {
   if (!e || !g || !out || n <= 0 || n % 4 != 0) return fail(LEAF_ERR_INVALID, "bad argument");
   const int grid = launch_ew(e, static_cast<size_t>(n) / 4);       // <= 16 x SMs: leaf_set_deterministic sizes det_sum_ws for it
-  if (e->deterministic)
-    sumsq_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(g, static_cast<size_t>(n), out, e->det_sum_ws, e->det_sum_cnt);
-  else
-    sumsq_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(g, static_cast<size_t>(n), out);
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  const bool det = e->deterministic;
+  return launch(e, det ? sumsq_kernel<true> : sumsq_kernel<false>, grid, 256, 0, static_cast<cudaStream_t>(stream), SERIAL, g,
+                static_cast<size_t>(n), out, det ? e->det_sum_ws : nullptr, det ? e->det_sum_cnt : nullptr);
 }
 
 // g[0, n) *= s (in place): torch.nn.utils.clip_grad_norm_'s rescale of the accumulated gradients after a micro-batch that
 // is not followed by an optimizer step (utils_AT.py:356-357 runs it after EVERY micro-batch)
 extern "C" int leaf_scale(leaf_handle_t e, float* g, int64_t n, float s, void* stream) {
   if (!e || !g || n <= 0 || n % 4 != 0) return fail(LEAF_ERR_INVALID, "bad argument");
-  scale_f32_kernel<<<launch_ew(e, static_cast<size_t>(n) / 4), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, static_cast<size_t>(n), s);
-  e->launches++;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  return launch(e, scale_f32_kernel, launch_ew(e, static_cast<size_t>(n) / 4), 256, 0, static_cast<cudaStream_t>(stream), SERIAL, g,
+                static_cast<size_t>(n), s);
 }
 
 // ---- on-device --constrain filter (constrain_core.cuh) ---------------------------------------------------------------------
@@ -1198,23 +1165,21 @@ extern "C" int leaf_constrain_mask(leaf_handle_t e, const uint8_t* caps, const i
   if (B <= 0 || n <= 0) return fail(LEAF_ERR_INVALID, "B=%d n=%d", B, n);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int R = B * n + B;
+  int rc;
   int32_t* cnt = count_out;
   if (!cnt) {
     if (R > e->cn_count_cap) {
       CK(cudaStreamSynchronize(st));
-      cudaFree(e->cn_count);
-      e->cn_count = nullptr;
-      CK(cudaMalloc(&e->cn_count, static_cast<size_t>(R) * 4));
+      e->cn_mem = DevMem();
+      e->cn_count_cap = 0;
+      if ((rc = e->cn_mem.alloc(&e->cn_count, R))) return rc;
       e->cn_count_cap = R;
     }
     cnt = e->cn_count;
   }
   CnArgs a{caps, cap_off, B, n, pos, chr, sel, cnt, status_out};
-  constrain_count_kernel<<<(R + 63) / 64, 64, 0, st>>>(e->cn, a);
-  constrain_valid_kernel<<<(B * n + 255) / 256, 256, 0, st>>>(cnt, B, n, valid_out);
-  e->launches += 2;
-  CK(cudaGetLastError());
-  return LEAF_OK;
+  if ((rc = launch(e, constrain_count_kernel, (R + 63) / 64, 64, 0, st, SERIAL, e->cn, a))) return rc;
+  return launch(e, constrain_valid_kernel, (B * n + 255) / 256, 256, 0, st, SERIAL, cnt, B, n, valid_out);
 }
 
 // Captions longer than LEAF_MAX_CAPTION_BYTES (up to LEAF_MAX_CAPTION_BYTES_LONG) switch leaf_expand_tokenize to its

@@ -26,7 +26,7 @@
 namespace leaf {
 
 // Programmatic dependent launch. Every GEMM, LayerNorm and attention launch carries
-// cudaLaunchAttributeProgrammaticStreamSerialization (engine.cu: launch_gemm, launch_pdl), and the non-GEMM kernels call
+// cudaLaunchAttributeProgrammaticStreamSerialization (engine.cu: launch, PDL / PDL_PAIR), and the non-GEMM kernels call
 // pdl_trigger() on entry: the GEMM that follows becomes resident while they drain, runs its prologue (barrier init, TMEM
 // allocation, descriptor prefetch) and blocks in pdl_wait() until its predecessor has completed and its writes are visible.
 // Rule: nothing that a predecessor of the same per-layer chain writes may be read, and nothing may be written, before
