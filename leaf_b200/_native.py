@@ -26,6 +26,42 @@ class LeafWeightPtrs(ctypes.Structure):
                 ("layers", ctypes.POINTER(LeafLayerPtrs))]
 
 
+# The text tower's parameters in the two namings the engine binds, keyed by the LeafWeightPtrs / LeafLayerPtrs field that
+# carries each: (open_clip suffix, HF suffix), None where a naming has no such tensor (open_clip fuses q / k / v into
+# in_proj, HF splits them). HF names sit under `text_model.` and the layers under LAYER_PREFIX, except the projection,
+# which sits beside `text_model.`. open_clip also spells the projection as nn.Linear's `text_projection.weight`, and the
+# two namings store it transposed to each other ([W, E] against [E, W]); engine._canon_state handles both. The order is
+# the key order of the converters in tower.py.
+TOWER_PARAMS = {
+    "token_embedding": ("token_embedding.weight", "embeddings.token_embedding.weight"),
+    "positional_embedding": ("positional_embedding", "embeddings.position_embedding.weight"),
+    "lnf_w": ("ln_final.weight", "final_layer_norm.weight"),
+    "lnf_b": ("ln_final.bias", "final_layer_norm.bias"),
+    "text_projection": ("text_projection", "text_projection.weight"),
+}
+LAYER_PREFIX = ("transformer.resblocks.{}.", "encoder.layers.{}.")
+LAYER_PARAMS = {
+    "in_proj_w": ("attn.in_proj_weight", None),
+    "in_proj_b": ("attn.in_proj_bias", None),
+    "q_w": (None, "self_attn.q_proj.weight"),
+    "q_b": (None, "self_attn.q_proj.bias"),
+    "k_w": (None, "self_attn.k_proj.weight"),
+    "k_b": (None, "self_attn.k_proj.bias"),
+    "v_w": (None, "self_attn.v_proj.weight"),
+    "v_b": (None, "self_attn.v_proj.bias"),
+    "out_w": ("attn.out_proj.weight", "self_attn.out_proj.weight"),
+    "out_b": ("attn.out_proj.bias", "self_attn.out_proj.bias"),
+    "ln1_w": ("ln_1.weight", "layer_norm1.weight"),
+    "ln1_b": ("ln_1.bias", "layer_norm1.bias"),
+    "ln2_w": ("ln_2.weight", "layer_norm2.weight"),
+    "ln2_b": ("ln_2.bias", "layer_norm2.bias"),
+    "fc1_w": ("mlp.c_fc.weight", "mlp.fc1.weight"),
+    "fc1_b": ("mlp.c_fc.bias", "mlp.fc1.bias"),
+    "fc2_w": ("mlp.c_proj.weight", "mlp.fc2.weight"),
+    "fc2_b": ("mlp.c_proj.bias", "mlp.fc2.bias"),
+}
+
+
 # name -> (restype, argtypes); also the list tests check against the header
 SIGNATURES = {
     "leaf_create": (c_int, [ctypes.POINTER(LeafCfg), ctypes.POINTER(c_void_p)]),

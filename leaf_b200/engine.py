@@ -10,14 +10,16 @@ leaf_b200/lib/libleaf_b200.so, and nothing here runs without it and a B200.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import os
+from dataclasses import dataclass
 
 import numpy as np
 import torch
 
 from . import _native
-from ._native import LeafCfg, LeafLayerPtrs, LeafWeightPtrs, LeafError, check
+from ._native import BACKWARD_HOOK, LAYER_PARAMS, LAYER_PREFIX, TOWER_PARAMS, LeafCfg, LeafError, LeafLayerPtrs, LeafWeightPtrs, check
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 MERGES_BIN = os.path.join(HERE, "data", "clip_bpe_merges.bin")
@@ -38,53 +40,47 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
-def _canon_state(params: dict):
-    """Map a parameter dict in open_clip CLIP / CustomTextCLIP ('text.' prefix) / HF CLIPTextModel(WithProjection)
-    naming to canonical per-tensor entries (SURVEY.md appendix C; conversion/convert_2.py:37-99)."""
-    keys = params.keys()
-    if any(k.endswith("embeddings.token_embedding.weight") for k in keys):       # HF layout
-        pre = next(k for k in keys if k.endswith("embeddings.token_embedding.weight"))
-        pre = pre[: -len("embeddings.token_embedding.weight")]                    # "text_model." or "...text_model."
-        root = pre[: -len("text_model.")] if pre.endswith("text_model.") else pre
-        out = {"layout": "hf", "tok": params[pre + "embeddings.token_embedding.weight"],
-               "pos": params[pre + "embeddings.position_embedding.weight"],
-               "lnf_w": params[pre + "final_layer_norm.weight"], "lnf_b": params[pre + "final_layer_norm.bias"],
-               "proj": params.get(root + "text_projection.weight"), "proj_is_ew": 1, "layers": []}
-        if out["proj"] is None:        # CLIPTextModel: the reference reads .pooler_output (utils_attacks.py:49-53) = identity head
-            out["proj"] = torch.eye(out["tok"].shape[1], dtype=torch.float32, device=out["tok"].device)
-            out["proj_synth"] = True
-        i = 0
-        while (pre + f"encoder.layers.{i}.layer_norm1.weight") in params:
-            p = pre + f"encoder.layers.{i}."
-            g = lambda s: params[p + s]
-            out["layers"].append(dict(
-                ln1_w=g("layer_norm1.weight"), ln1_b=g("layer_norm1.bias"),
-                q_w=g("self_attn.q_proj.weight"), k_w=g("self_attn.k_proj.weight"), v_w=g("self_attn.v_proj.weight"),
-                q_b=g("self_attn.q_proj.bias"), k_b=g("self_attn.k_proj.bias"), v_b=g("self_attn.v_proj.bias"),
-                out_w=g("self_attn.out_proj.weight"), out_b=g("self_attn.out_proj.bias"),
-                ln2_w=g("layer_norm2.weight"), ln2_b=g("layer_norm2.bias"),
-                fc1_w=g("mlp.fc1.weight"), fc1_b=g("mlp.fc1.bias"), fc2_w=g("mlp.fc2.weight"), fc2_b=g("mlp.fc2.bias")))
-            i += 1
-        return out
-    pre = "text." if "text.token_embedding.weight" in params else ""
-    if (pre + "token_embedding.weight") not in params:
-        raise LeafError("unrecognised parameter naming: expected open_clip (token_embedding.weight / "
-                        "text.token_embedding.weight) or HF CLIPTextModel keys")
-    out = {"layout": "open_clip", "tok": params[pre + "token_embedding.weight"], "pos": params[pre + "positional_embedding"],
-           "lnf_w": params[pre + "ln_final.weight"], "lnf_b": params[pre + "ln_final.bias"],
-           "proj": params[pre + "text_projection"], "proj_is_ew": 0, "layers": []}
-    if out["proj"].dim() == 2 and (pre + "text_projection.weight") in params:     # nn.Linear projection variant
-        out["proj"], out["proj_is_ew"] = params[pre + "text_projection.weight"], 1
-    i = 0
-    while (pre + f"transformer.resblocks.{i}.ln_1.weight") in params:
-        p = pre + f"transformer.resblocks.{i}."
-        g = lambda s: params[p + s]
-        out["layers"].append(dict(
-            ln1_w=g("ln_1.weight"), ln1_b=g("ln_1.bias"), in_proj_w=g("attn.in_proj_weight"), in_proj_b=g("attn.in_proj_bias"),
-            out_w=g("attn.out_proj.weight"), out_b=g("attn.out_proj.bias"), ln2_w=g("ln_2.weight"), ln2_b=g("ln_2.bias"),
-            fc1_w=g("mlp.c_fc.weight"), fc1_b=g("mlp.c_fc.bias"), fc2_w=g("mlp.c_proj.weight"), fc2_b=g("mlp.c_proj.bias")))
-        i += 1
-    return out
+@dataclass
+class TowerParams:
+    """A text tower's tensors (the parameter dict's own objects) keyed by the ABI field that carries each (TOWER_PARAMS / LAYER_PARAMS)."""
+    layout: str                        # "open_clip" or "hf"
+    top: dict
+    layers: list                       # per layer, the fields its naming has
+    projection_is_ew: int              # 1: text_projection is [E, W] (HF, open_clip's nn.Linear); 0: open_clip's [W, E]
+    projection_synthesised: bool = False
+
+    def tensors(self) -> list:
+        """The tensors of the dict the view was read from: every field but a synthesised projection, None entries left out."""
+        top = [t for f, t in self.top.items() if f != "text_projection" or not self.projection_synthesised]
+        return [t for t in top + [t for l in self.layers for t in l.values()] if t is not None]
+
+
+def _canon_state(params: dict) -> TowerParams:
+    """The TowerParams of a dict in open_clip (bare or `text.`-prefixed) or HF (CLIPTextModel(WithProjection), CLIPModel) naming."""
+    hf_tok = TOWER_PARAMS["token_embedding"][1]
+    pre = next((k[: -len(hf_tok)] for k in params if k.endswith(hf_tok)), None)      # "text_model." or "...text_model."
+    col = int(pre is not None)
+    if col:
+        root = pre.removesuffix("text_model.")                         # HF keeps the projection beside text_model
+    else:
+        pre = root = "text." if "text.token_embedding.weight" in params else ""
+        if (pre + "token_embedding.weight") not in params:
+            raise LeafError("unrecognised parameter naming: expected open_clip (token_embedding.weight / "
+                            "text.token_embedding.weight) or HF CLIPTextModel keys")
+    top = {f: params[pre + n[col]] for f, n in TOWER_PARAMS.items() if f != "text_projection"}
+    v = TowerParams(("open_clip", "hf")[col], top, [], projection_is_ew=col)
+    proj = root + TOWER_PARAMS["text_projection"][col]
+    if proj in params:
+        top["text_projection"] = params[proj]
+    elif col:                          # CLIPTextModel: the reference reads .pooler_output (utils_attacks.py:49-53) = identity head
+        top["text_projection"] = torch.eye(top["token_embedding"].shape[1], dtype=torch.float32, device=top["token_embedding"].device)
+        v.projection_synthesised = True
+    else:                              # open_clip's nn.Linear projection: an [E, W] weight, like HF's
+        top["text_projection"], v.projection_is_ew = params[proj + ".weight"], 1
+    layer, names = pre + LAYER_PREFIX[col], {f: n[col] for f, n in LAYER_PARAMS.items() if n[col]}
+    while (p := layer.format(len(v.layers))) + names["ln1_w"] in params:
+        v.layers.append({f: params[p + n] for f, n in names.items()})
+    return v
 
 
 class LeafEngine:
@@ -96,14 +92,13 @@ class LeafEngine:
         if not torch.cuda.is_available():
             raise LeafError("leaf_b200 needs a CUDA device (sm_100a); there is no CPU path")
         self._lib = _native.lib()
-        c = _canon_state(params)
-        self._canon = c
-        self.width = int(c["tok"].shape[1])
-        self.layers = len(c["layers"])
+        self._params = v = _canon_state(params)
+        self.width = int(v.top["token_embedding"].shape[1])
+        self.layers = len(v.layers)
         self.heads = int(heads)
         self.quick_gelu, self.ln_eps = bool(quick_gelu), float(ln_eps)
-        self.embed_dim = int(c["proj"].shape[0] if c["proj_is_ew"] else c["proj"].shape[1])
-        self.device = c["tok"].device
+        self.embed_dim = int(v.top["text_projection"].shape[0 if v.projection_is_ew else 1])
+        self.device = v.top["token_embedding"].device
         self._check_tensors()
         cfg = LeafCfg(self.width, self.layers, self.heads, self.embed_dim, 1 if quick_gelu else 0, ln_eps)
         self._h = ctypes.c_void_p()
@@ -133,11 +128,9 @@ class LeafEngine:
             pass
 
     def _check_tensors(self):
-        c = self._canon
-        flat = [c["tok"], c["pos"], c["lnf_w"], c["lnf_b"], c["proj"]] + [t for l in c["layers"] for t in l.values()]
-        if not c["layers"]:
+        if not self._params.layers:
             raise LeafError("no transformer layers found in the parameter dict")
-        for t in flat:
+        for t in self._params.tensors():
             if not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
                 raise LeafError("tower parameters must be contiguous fp32 CUDA tensors")
             if t.data_ptr() % 16:
@@ -145,18 +138,15 @@ class LeafEngine:
         if self.width != self.heads * 64:
             raise LeafError(f"head_dim must be 64 (width {self.width}, heads {self.heads})")
 
-    def _make_ptrs(self, c):
-        """leaf_weight_ptrs_t over a canonical dict of tensors (None entries become NULL)."""
-        dp = lambda t: None if t is None else t.data_ptr()
-        arr = (LeafLayerPtrs * self.layers)()
-        for i, l in enumerate(c["layers"]):
-            for k, _ in LeafLayerPtrs._fields_:
-                setattr(arr[i], k, dp(l.get(k)))
-        wp = LeafWeightPtrs(dp(c["tok"]), dp(c["pos"]), dp(c["lnf_w"]), dp(c["lnf_b"]), dp(c["proj"]), c["proj_is_ew"], arr)
+    def _make_ptrs(self, v: TowerParams):
+        """leaf_weight_ptrs_t over a TowerParams (fields it does not hold, and None entries, become NULL)."""
+        ptrs = lambda d: {f: None if t is None else t.data_ptr() for f, t in d.items()}
+        arr = (LeafLayerPtrs * self.layers)(*(LeafLayerPtrs(**ptrs(l)) for l in v.layers))
+        wp = LeafWeightPtrs(**ptrs(v.top), projection_is_ew=v.projection_is_ew, layers=arr)
         return arr, wp
 
     def _bind(self):
-        self._keep = self._make_ptrs(self._canon)
+        self._keep = self._make_ptrs(self._params)
         check(self._lib.leaf_bind_weights(self._h, ctypes.byref(self._keep[1]), _stream()))
 
     def refresh_weights(self):
@@ -369,15 +359,46 @@ class LeafEngine:
         (forward_train's self.last_generation) makes the engine refuse to differentiate a forward it no longer holds."""
         if dfeat.dim() != 2 or dfeat.shape[1] != self.embed_dim:
             raise LeafError(f"dfeat must be [N, {self.embed_dim}], got {tuple(dfeat.shape)}")
-        c = _canon_state(grads)
-        for t in [c["tok"], c["pos"], c["lnf_w"], c["lnf_b"], c["proj"]] + [t for l in c["layers"] for t in l.values()]:
-            if t is not None and not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
+        g = _canon_state(grads)
+        for t in g.tensors():
+            if not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
                 raise LeafError("gradient buffers must be contiguous fp32 CUDA tensors")
-        keep = self._make_ptrs(c)
+        keep = self._make_ptrs(g)
         with torch.cuda.device(self.device):
             self.set_deterministic(torch.are_deterministic_algorithms_enabled())
             check(self._lib.leaf_backward(self._h, int(generation), _ptr(dfeat.to(torch.float32).contiguous()), int(dfeat.shape[0]),
                                           ctypes.byref(keep[1]), _stream()))
+
+    def set_backward_hook(self, fn):
+        """fn(layer, user) runs on the host once backward() has enqueued a layer's gradients, and with layer -1 after the
+        rest (leaf_set_backward_hook). The engine keeps the ctypes thunk alive for as long as it may call it."""
+        self._backward_hook = BACKWARD_HOOK(fn)
+        check(self._lib.leaf_set_backward_hook(self._h, ctypes.cast(self._backward_hook, ctypes.c_void_p), None))
+
+    @contextlib.contextmanager
+    def sm_budget(self, n_sms: int):
+        """The persistent GEMM grids take at most n_sms SMs inside the block (leaf_set_sm_budget), all of them again after it."""
+        check(self._lib.leaf_set_sm_budget(self._h, n_sms))
+        try:
+            yield
+        finally:
+            check(self._lib.leaf_set_sm_budget(self._h, 0))
+
+    def adamw(self, params, grads, exp_avg, exp_avg_sq, *, n_nodecay, lr, beta1, beta2, eps, weight_decay, step, grad_scale=1.0):
+        """One AdamW step (leaf_adamw) over flat fp32 buffers: grads are scaled by grad_scale, [0, n_nodecay) takes no weight decay."""
+        with torch.cuda.device(self.device):
+            check(self._lib.leaf_adamw(self._h, _ptr(params), _ptr(grads), _ptr(exp_avg), _ptr(exp_avg_sq), grads.numel(), n_nodecay,
+                                       lr, beta1, beta2, eps, weight_decay, step, grad_scale, _stream()))
+
+    def sumsq(self, g, out):
+        """Adds the sum of squares of the flat fp32 buffer g into out[0] (leaf_sumsq; fixed-order in deterministic mode)."""
+        with torch.cuda.device(self.device):
+            check(self._lib.leaf_sumsq(self._h, _ptr(g), g.numel(), _ptr(out), _stream()))
+
+    def scale(self, g, s: float):
+        """g *= s in place, for a flat fp32 buffer (leaf_scale)."""
+        with torch.cuda.device(self.device):
+            check(self._lib.leaf_scale(self._h, _ptr(g), g.numel(), s, _stream()))
 
     # ---- K3 ----------------------------------------------------------------------------------------------
     def score(self, feats: torch.Tensor, anchor: torch.Tensor, B: int, n: int, objective: str = "l2", want_loss=False):
@@ -531,9 +552,8 @@ def bind_module(model) -> LeafEngine:
     if isinstance(eng, LeafEngine) and getattr(module, "_leaf_self_managed", False):
         return eng                                                           # LeafTextTower refreshes its own engine
     live = module.state_dict(keep_vars=True)
-    c = _canon_state({k: v for k, v in live.items() if torch.is_tensor(v)})
-    flat = [c["tok"], c["pos"], c["lnf_w"], c["lnf_b"]] + ([] if c.get("proj_synth") else [c["proj"]]) + \
-           [t for l in c["layers"] for t in l.values()]
+    v = _canon_state({k: t for k, t in live.items() if torch.is_tensor(t)})
+    flat = v.tensors()
     ptrs = tuple(t.data_ptr() for t in flat)
     version = sum(t._version for t in flat)
     if isinstance(eng, LeafEngine) and getattr(eng, "_bound_ptrs", None) == ptrs:
@@ -543,7 +563,7 @@ def bind_module(model) -> LeafEngine:
         return eng
     heads, quick, eps = _text_config(module) or _open_clip_config(module)
     eng = LeafEngine({k: v.detach() for k, v in live.items() if torch.is_tensor(v)}, heads=heads, quick_gelu=quick, ln_eps=eps)
-    if c["layout"] == "hf":
+    if v.layout == "hf":
         eng.set_tokenizer_mode(True)
     eng._bound_ptrs, eng._bound_version = ptrs, version
     object.__setattr__(module, "leaf_engine", eng)                           # a plain attribute, not a registered submodule

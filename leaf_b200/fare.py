@@ -11,7 +11,7 @@ format (FareTrainer.reference_checkpoint / load_reference_checkpoint, train_AT_t
 """
 from __future__ import annotations
 
-import ctypes
+import contextlib
 import math
 import os
 import weakref
@@ -20,9 +20,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from ._native import BACKWARD_HOOK, check
 from .attack import V_DEFAULT, attack_text_leaf
-from .engine import _ptr, _stream
 from .eval_attacks import attack_text_charmer_inference
 from .tower import LeafTextTower, no_weight_decay, text_tower_state_dict
 
@@ -69,9 +67,7 @@ class FareTrainer:
                 if tr is not None:
                     tr._on_backward_layer(layer, user)
 
-            eng = tower.leaf_engine
-            eng._backward_hook = BACKWARD_HOOK(thunk)         # the ctypes thunk lives as long as the engine that calls it
-            check(eng._lib.leaf_set_backward_hook(eng._h, ctypes.cast(eng._backward_hook, ctypes.c_void_p), None))
+            tower.leaf_engine.set_backward_hook(thunk)
 
     def _gradient_ranges(self):
         """Contiguous [lo, hi) element ranges of the flat gradient buffer: one list per layer holding that layer's weight
@@ -150,7 +146,7 @@ class FareTrainer:
         eng, g = self.tower.leaf_engine, self.tower.flat_grads
         eng.set_deterministic(torch.are_deterministic_algorithms_enabled())
         self._norm.zero_()
-        check(eng._lib.leaf_sumsq(eng._h, _ptr(g), g.numel(), _ptr(self._norm), _stream()))
+        eng.sumsq(g, self._norm)
         total = math.sqrt(float(self._norm.item())) * grad_scale
         return min(1.0, self.grad_clip_norm / (total + 1e-6))
 
@@ -158,16 +154,14 @@ class FareTrainer:
         """utils_AT.py:338-362 with scaler = None: all-reduce (DDP's job in the reference), clip, AdamW, zero_grad; then the
         engine re-casts its bf16 operand copies from the updated fp32 parameters."""
         t = self.tower
-        g, eng = t.flat_grads, t.leaf_engine
         self._exchange()
         scale = grad_scale
         if self.grad_clip_norm is not None:                       # the clip is folded into AdamW's gradient scale
             scale *= self._clip_scale(grad_scale)
         self.opt_step += 1
-        f = ctypes.c_float
-        check(eng._lib.leaf_adamw(eng._h, _ptr(t.flat_params), _ptr(g), _ptr(self.exp_avg), _ptr(self.exp_avg_sq), g.numel(),
-                                  t.n_nodecay, f(self.lr_at(self.opt_step)), f(self.beta1), f(self.beta2), f(self.eps), f(self.wd),
-                                  self.opt_step, f(scale), _stream()))
+        t.leaf_engine.adamw(t.flat_params, t.flat_grads, self.exp_avg, self.exp_avg_sq, n_nodecay=t.n_nodecay,
+                            lr=self.lr_at(self.opt_step), beta1=self.beta1, beta2=self.beta2, eps=self.eps, weight_decay=self.wd,
+                            step=self.opt_step, grad_scale=scale)
         t.zero_grad()
         t.refresh()
 
@@ -187,11 +181,8 @@ class FareTrainer:
         budget = self.overlap_allreduce and (last or clip_now) and self.backward_sm_budget > 0
         if self.overlap_allreduce:
             self._hook_armed = last or clip_now
-        if budget:
-            check(t.leaf_engine._lib.leaf_set_sm_budget(t.leaf_engine._h, self.backward_sm_budget))
-        (loss / self.accum_freq).backward()                                                # :329-337
-        if budget:
-            check(t.leaf_engine._lib.leaf_set_sm_budget(t.leaf_engine._h, 0))
+        with t.leaf_engine.sm_budget(self.backward_sm_budget) if budget else contextlib.nullcontext():
+            (loss / self.accum_freq).backward()                                            # :329-337
         if self.overlap_allreduce:
             self._hook_armed = False
         self.micro += 1
@@ -201,8 +192,7 @@ class FareTrainer:
             self._exchange()                                  # averaging identical accumulated values again changes nothing
             s = self._clip_scale()
             if s < 1.0:
-                eng, g = t.leaf_engine, t.flat_grads
-                check(eng._lib.leaf_scale(eng._h, _ptr(g), g.numel(), ctypes.c_float(s), _stream()))
+                t.leaf_engine.scale(t.flat_grads, s)
         return loss.detach(), adv_texts
 
     # ---- checkpoints -----------------------------------------------------------------------------------------------------

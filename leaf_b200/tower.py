@@ -17,7 +17,8 @@ import re
 import torch
 
 from . import synth
-from .engine import LeafEngine
+from ._native import LAYER_PARAMS, LAYER_PREFIX, TOWER_PARAMS
+from .engine import LeafEngine, TowerParams, _canon_state
 
 
 def no_weight_decay(name: str, ndim: int) -> bool:
@@ -48,10 +49,8 @@ class _EncodeTextTrain(torch.autograd.Function):
         return (None, None) + (None,) * len(grads)
 
 
-_TEXT_KEYS = re.compile(r"^(?:module\.)?(?:text\.)?(?P<key>token_embedding\.weight|positional_embedding|ln_final\.(weight|bias)|"
-                        r"text_projection(\.weight)?|"
-                        r"transformer\.resblocks\.\d+\.(ln_1|ln_2|attn\.out_proj|mlp\.c_fc|mlp\.c_proj)\.(weight|bias)|"
-                        r"transformer\.resblocks\.\d+\.attn\.in_proj_(weight|bias))$")
+_TOP_KEYS = {oc for oc, _ in TOWER_PARAMS.values()} | {"text_projection.weight"}     # nn.Linear's projection too
+_LAYER_KEY = re.compile(r"transformer\.resblocks\.\d+\.(?:%s)" % "|".join(re.escape(oc) for oc, _ in LAYER_PARAMS.values() if oc))
 
 
 def text_tower_state_dict(state_dict: dict) -> dict:
@@ -60,9 +59,28 @@ def text_tower_state_dict(state_dict: dict) -> dict:
     state dict saved through DDP, are removed."""
     out = {}
     for k, v in state_dict.items():
-        m = _TEXT_KEYS.match(k)
-        if m:
-            out[m["key"]] = v
+        k = k.removeprefix("module.").removeprefix("text.")
+        if k in _TOP_KEYS or _LAYER_KEY.fullmatch(k):
+            out[k] = v
+    return out
+
+
+def _renamed(v: TowerParams, hf: bool) -> dict:
+    """New tensors of `v` under CLIPTextModelWithProjection's keys (hf) or bare open_clip keys, in TOWER_PARAMS / LAYER_PARAMS
+    order: q / k / v are in_proj's three row blocks, and the projection is transposed where the two orientations differ."""
+    col, pre = (1, "text_model.") if hf else (0, "")
+    out = {pre + TOWER_PARAMS[f][col]: t.clone() for f, t in v.top.items() if f != "text_projection"}
+    proj = v.top["text_projection"]
+    out[TOWER_PARAMS["text_projection"][col]] = proj.clone() if v.projection_is_ew == hf else proj.t().contiguous()
+    for i, l in enumerate(v.layers):
+        l = dict(l)
+        if hf:
+            for nm, w, b in zip("qkv", l["in_proj_w"].chunk(3, dim=0), l["in_proj_b"].chunk(3, dim=0)):
+                l[nm + "_w"], l[nm + "_b"] = w.contiguous(), b.contiguous()
+        else:
+            l["in_proj_w"], l["in_proj_b"] = (torch.cat([l[nm + s] for nm in "qkv"], dim=0) for s in ("_w", "_b"))
+        p = pre + LAYER_PREFIX[col].format(i)
+        out.update((p + n[col], l[f].clone()) for f, n in LAYER_PARAMS.items() if n[col])
     return out
 
 
@@ -70,47 +88,18 @@ def open_clip_to_hf(sd: dict) -> dict:
     """The reference's export mapping (conversion/convert_2.py:37-99, copy_text_model_and_projection): an open_clip text-tower
     state dict -> the keys of transformers' CLIPTextModelWithProjection (equally the text half of a CLIPModel): fused
     in_proj split into q / k / v (`chunk(3, dim=0)`, :39-40), c_fc / c_proj -> fc1 / fc2, ln_1 / ln_2 -> layer_norm1 / 2,
-    positional_embedding -> position_embedding.weight, text_projection [W,E] -> text_projection.weight = P^T [E,W] (:85).
-    Tensors are new (contiguous copies), on the source's device."""
-    sd = text_tower_state_dict(sd)
-    out = {"text_model.embeddings.token_embedding.weight": sd["token_embedding.weight"].clone(),
-           "text_model.embeddings.position_embedding.weight": sd["positional_embedding"].clone(),
-           "text_model.final_layer_norm.weight": sd["ln_final.weight"].clone(),
-           "text_model.final_layer_norm.bias": sd["ln_final.bias"].clone(),
-           "text_projection.weight": sd["text_projection"].t().contiguous()}
-    i = 0
-    while f"transformer.resblocks.{i}.ln_1.weight" in sd:
-        p, q = f"transformer.resblocks.{i}.", f"text_model.encoder.layers.{i}."
-        for nm, w, b in zip("qkv", sd[p + "attn.in_proj_weight"].chunk(3, dim=0), sd[p + "attn.in_proj_bias"].chunk(3, dim=0)):
-            out[q + f"self_attn.{nm}_proj.weight"], out[q + f"self_attn.{nm}_proj.bias"] = w.contiguous().clone(), b.contiguous().clone()
-        for a, b in (("attn.out_proj", "self_attn.out_proj"), ("ln_1", "layer_norm1"), ("ln_2", "layer_norm2"),
-                     ("mlp.c_fc", "mlp.fc1"), ("mlp.c_proj", "mlp.fc2")):
-            out[q + b + ".weight"], out[q + b + ".bias"] = sd[p + a + ".weight"].clone(), sd[p + a + ".bias"].clone()
-        i += 1
-    return out
+    positional_embedding -> position_embedding.weight, text_projection [W,E] -> text_projection.weight = P^T [E,W] (:85), or
+    nn.Linear's text_projection.weight [E,W] as it is. Tensors are new (contiguous copies), on the source's device."""
+    return _renamed(_canon_state(text_tower_state_dict(sd)), hf=True)
 
 
 def hf_to_open_clip(sd: dict) -> dict:
-    """The inverse mapping (the direction of the reference's convert_to_openclip.py): HF CLIPTextModel(WithProjection) /
+    """The inverse mapping (the direction of the reference's convert_to_openclip.py): HF CLIPTextModelWithProjection /
     CLIPModel keys -> an open_clip text-tower state dict LeafTextTower accepts."""
-    pre = next((k[: -len("embeddings.token_embedding.weight")] for k in sd if k.endswith("embeddings.token_embedding.weight")), None)
-    if pre is None:
-        raise ValueError("not an HF CLIP text state dict (no embeddings.token_embedding.weight)")
-    root = pre[: -len("text_model.")] if pre.endswith("text_model.") else pre
-    out = {"token_embedding.weight": sd[pre + "embeddings.token_embedding.weight"].clone(),
-           "positional_embedding": sd[pre + "embeddings.position_embedding.weight"].clone(),
-           "ln_final.weight": sd[pre + "final_layer_norm.weight"].clone(), "ln_final.bias": sd[pre + "final_layer_norm.bias"].clone(),
-           "text_projection": sd[root + "text_projection.weight"].t().contiguous()}
-    i = 0
-    while (pre + f"encoder.layers.{i}.layer_norm1.weight") in sd:
-        q, p = pre + f"encoder.layers.{i}.", f"transformer.resblocks.{i}."
-        out[p + "attn.in_proj_weight"] = torch.cat([sd[q + f"self_attn.{nm}_proj.weight"] for nm in "qkv"], dim=0)
-        out[p + "attn.in_proj_bias"] = torch.cat([sd[q + f"self_attn.{nm}_proj.bias"] for nm in "qkv"], dim=0)
-        for a, b in (("attn.out_proj", "self_attn.out_proj"), ("ln_1", "layer_norm1"), ("ln_2", "layer_norm2"),
-                     ("mlp.c_fc", "mlp.fc1"), ("mlp.c_proj", "mlp.fc2")):
-            out[p + a + ".weight"], out[p + a + ".bias"] = sd[q + b + ".weight"].clone(), sd[q + b + ".bias"].clone()
-        i += 1
-    return out
+    v = _canon_state(sd)
+    if v.layout != "hf" or v.projection_synthesised:
+        raise ValueError("not an HF CLIP text state dict with a projection (embeddings.token_embedding.weight, text_projection.weight)")
+    return _renamed(v, hf=False)
 
 
 class LeafTextTower(torch.nn.Module):

@@ -25,9 +25,10 @@ def lib():
     if _lib is None:
         if not os.path.exists(LIB) or os.path.getmtime(LIB) < _deps_mtime():
             subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-o", LIB, SRC])
-        _lib = ctypes.CDLL(LIB)
+        L = ctypes.CDLL(LIB)
         pairs = np.fromfile(MERGES, dtype="<u4")
-        _lib.k1h_load(pairs.ctypes.data_as(ctypes.c_void_p), ctypes.c_int(len(pairs)))
+        L.k1h_load(pairs.ctypes.data_as(ctypes.c_void_p), ctypes.c_int(len(pairs)))
+        _lib = L
     return _lib
 
 

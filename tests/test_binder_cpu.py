@@ -21,8 +21,8 @@ def test_hf_config_detection():
             if not isinstance(m, CLIPModel):      # (a CLIPModel's VISION tower has its own activation: scanning all modules would be wrong)
                 assert any(type(x).__name__ == "QuickGELUActivation" for x in m.modules()) == quick     # the class round 1 missed
             c = _canon_state({k: v for k, v in m.state_dict(keep_vars=True).items()})
-            assert c["layout"] == "hf" and len(c["layers"]) == 1 and c["tok"].shape == (49408, 128)
-            assert ("proj_synth" in c) == isinstance(m, CLIPTextModel)                              # pooler_output: identity head
+            assert c.layout == "hf" and len(c.layers) == 1 and c.top["token_embedding"].shape == (49408, 128)
+            assert c.projection_synthesised == isinstance(m, CLIPTextModel)                            # pooler_output: identity head
     bad = _hf_text_config(False, layers=1, W=128, heads=2, E=64)
     bad.hidden_act = "gelu_new"
     with pytest.raises(LeafError, match="activation"):
@@ -39,7 +39,7 @@ def test_open_clip_module_detection():
         holder.text = tower                                                       # CustomTextCLIP keeps its tower under `.text`
         assert _open_clip_config(holder) == (cfg.heads, quick, 1e-5)
         c = _canon_state({k: v for k, v in holder.state_dict(keep_vars=True).items()})
-        assert c["layout"] == "open_clip" and len(c["layers"]) == cfg.layers and c["proj_is_ew"] == 0
+        assert c.layout == "open_clip" and len(c.layers) == cfg.layers and c.projection_is_ew == 0
     with pytest.raises(LeafError):
         _open_clip_config(torch.nn.Linear(2, 2))
     with pytest.raises(LeafError, match="naming"):
@@ -67,7 +67,7 @@ for name, quick, heads, layers, width in (("ViT-B-32", False, 8, 12, 512), ("ViT
     assert _open_clip_config(m) == (heads, quick, 1e-5), (name, _open_clip_config(m))
     holder = torch.nn.Module(); holder.module = m
     c = _canon_state({k: v for k, v in m.state_dict(keep_vars=True).items()})
-    assert c["layout"] == "open_clip" and len(c["layers"]) == layers and c["tok"].shape[1] == width and c["proj_is_ew"] == 0
+    assert c.layout == "open_clip" and len(c.layers) == layers and c.top["token_embedding"].shape[1] == width and c.projection_is_ew == 0
 print("OK")
 '''.replace("ROOT", repr(root)).replace("REF", repr(ref))
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)

@@ -193,9 +193,6 @@ def test_backward_hf_layout():
 def test_adamw_kernel_matches_torch():
     """leaf_adamw over a flat buffer (no-decay group first) against torch.optim.AdamW with the reference's two parameter
     groups (train_AT_text_only.py:326-341), several steps, with a gradient scale."""
-    import ctypes
-    from leaf_b200._native import check
-    from leaf_b200.engine import _ptr, _stream
     from leaf_b200.tower import LeafTextTower
     eng = LeafTextTower.random("tiny", seed=0).leaf_engine
     g = torch.Generator(device="cuda").manual_seed(1)
@@ -206,13 +203,11 @@ def test_adamw_kernel_matches_torch():
     opt = torch.optim.AdamW([{"params": [ref_a], "weight_decay": 0.0}, {"params": [ref_b], "weight_decay": wd}], lr=lr,
                             betas=(b1, b2), eps=eps)
     m, v = torch.zeros_like(p), torch.zeros_like(p)
-    f = ctypes.c_float
     for step in range(1, 6):
         grad = torch.randn(n, generator=g, device="cuda") * (0.1 if step % 2 else 10.0)
         ref_a.grad, ref_b.grad = grad[:nd] * scale, grad[nd:] * scale
         opt.step()
-        check(eng._lib.leaf_adamw(eng._h, _ptr(p), _ptr(grad), _ptr(m), _ptr(v), n, nd, f(lr), f(b1), f(b2), f(eps), f(wd), step,
-                                  f(scale), _stream()))
+        eng.adamw(p, grad, m, v, n_nodecay=nd, lr=lr, beta1=b1, beta2=b2, eps=eps, weight_decay=wd, step=step, grad_scale=scale)
         want = torch.cat([ref_a.detach(), ref_b.detach()])
         assert torch.allclose(p, want, rtol=1e-5, atol=1e-7), (step, (p - want).abs().max().item())
 

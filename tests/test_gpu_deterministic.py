@@ -93,9 +93,8 @@ def test_sm_budget_and_dependent_launch_change_no_bit(name, monkeypatch):
     want = _grads_of(plain, tok, w)
     eng = chained.leaf_engine
     for budget in (0, 64, 32, 0):
-        eng._lib.leaf_set_sm_budget(eng._h, budget)
-        assert _bit_equal(want, _grads_of(chained, tok, w)), budget
-    eng._lib.leaf_set_sm_budget(eng._h, 0)
+        with eng.sm_budget(budget):
+            assert _bit_equal(want, _grads_of(chained, tok, w)), budget
 
 
 def _frozen(grads):
@@ -174,8 +173,6 @@ def test_deterministic_gradients_meet_the_autograd_bars(name, quick):
 
 
 def test_sumsq_is_reproducible_and_accurate():
-    from leaf_b200._native import check
-    from leaf_b200.engine import _ptr, _stream
     from leaf_b200.tower import LeafTextTower
     eng = LeafTextTower.random("tiny", seed=0).leaf_engine
     eng.set_deterministic(True)
@@ -184,7 +181,7 @@ def test_sumsq_is_reproducible_and_accurate():
     outs = []
     for _ in range(4):
         out = torch.zeros(1, device="cuda")
-        check(eng._lib.leaf_sumsq(eng._h, _ptr(g), g.numel(), _ptr(out), _stream()))
+        eng.sumsq(g, out)
         outs.append(out)
     assert all(_bit_equal(outs[0], o) for o in outs[1:])
     want = (g.double() ** 2).sum().item()
@@ -205,22 +202,20 @@ def test_fare_trainer_steps_are_bit_reproducible(budget):
     hp = dict(rho=12, k_adv=1, accum_freq=2, grad_clip_norm=0.5, lr=1e-3, wd=0.05)
     trs = [FareTrainer(LeafTextTower(sd, heads=cfg.heads), frozen, **hp),
            FareTrainer(LeafTextTower(sd, heads=cfg.heads), frozen, backward_sm_budget=budget, **hp)]
-    if budget:
-        eng = trs[1].tower.leaf_engine
-        eng._lib.leaf_set_sm_budget(eng._h, budget)
-    for i in range(6):
-        texts = synth.make_captions(6, seed=40 + i)
-        adv = []
-        for tr in trs:
-            np.random.seed(100 + i)
-            adv.append(tr.step(texts)[1])
-        assert adv[0] == adv[1], i
-        if i % 2 == 1:
-            a, b = trs
-            assert a.opt_step == b.opt_step == (i + 1) // 2
-            assert _bit_equal(a.tower.flat_params, b.tower.flat_params), i
-            assert _bit_equal(a.exp_avg, b.exp_avg), i
-            assert _bit_equal(a.exp_avg_sq, b.exp_avg_sq), i
+    with trs[1].tower.leaf_engine.sm_budget(budget or 0):
+        for i in range(6):
+            texts = synth.make_captions(6, seed=40 + i)
+            adv = []
+            for tr in trs:
+                np.random.seed(100 + i)
+                adv.append(tr.step(texts)[1])
+            assert adv[0] == adv[1], i
+            if i % 2 == 1:
+                a, b = trs
+                assert a.opt_step == b.opt_step == (i + 1) // 2
+                assert _bit_equal(a.tower.flat_params, b.tower.flat_params), i
+                assert _bit_equal(a.exp_avg, b.exp_avg), i
+                assert _bit_equal(a.exp_avg_sq, b.exp_avg_sq), i
     assert not torch.equal(trs[0].tower.flat_params, LeafTextTower(sd, heads=cfg.heads).flat_params)
 
 

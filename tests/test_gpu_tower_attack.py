@@ -81,6 +81,31 @@ def test_tower_hf_layout_binds_identically():
     assert torch.equal(e1.encode_tokens(tok), e2.encode_tokens(tok))
 
 
+def test_tower_linear_projection_binds_identically():
+    """open_clip's nn.Linear projection (text_projection.weight = P^T, [E, W]) and its parameter form (text_projection = P,
+    [W, E]) of the same weights encode to the bit: the engine casts the one, and casts and transposes the other, into the
+    same bf16 [E, W] operand. Training binds the .weight form too, and its projection gradient is the transposed one."""
+    from leaf_b200 import synth
+    from leaf_b200.tower import LeafTextTower
+    cfg = synth.TOWERS["small"]
+    sd = synth.random_tower_state_dict(cfg, seed=4, exact_numpy=True)
+    lin = dict(sd)
+    lin["text_projection.weight"] = lin.pop("text_projection").t().contiguous()
+    a, b = LeafTextTower(sd, heads=cfg.heads), LeafTextTower(lin, heads=cfg.heads)
+    assert b.leaf_engine.embed_dim == cfg.embed_dim
+    tok = a.tokenizer(synth.make_captions(16, seed=1))
+    for normalize in (False, True):
+        assert torch.equal(a.encode_text(tok, normalize=normalize), b.encode_text(tok, normalize=normalize)), normalize
+    fa, fb = a.trainable().encode_text(tok), b.trainable().encode_text(tok)
+    assert torch.equal(fa, fb)
+    d = torch.randn_like(fa)
+    (fa * d).sum().backward()
+    (fb * d).sum().backward()
+    ga, gb = dict(a.named_tower_parameters()), dict(b.named_tower_parameters())
+    assert torch.allclose(gb["text_projection.weight"].grad, ga["text_projection"].grad.T, rtol=1e-3, atol=1e-6)
+    assert torch.allclose(gb["token_embedding.weight"].grad, ga["token_embedding.weight"].grad, rtol=1e-3, atol=1e-6)
+
+
 @pytest.mark.parametrize("name", ["ViT-L-14"])
 def test_tower_full_width_vs_oracle(name):
     """A full-width tower against the fp32 oracle on a handful of rows (the oracle runs on the host in seconds)."""
